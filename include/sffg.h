@@ -251,7 +251,8 @@ SFFG_API int sffg_radius(sffg_index *idx, const float *queries, int64_t nq, floa
  * end call has returned: sffg_index_end(idx) for sffg_radius_begin, sffg_index_end(idx[0]) for sffg_knn_multi_begin and
  * sffg_index_add_multi_begin, sffg_env_end(env) for sffg_check_edges_begin / sffg_check_moves_begin.  Between begin
  * and end, calls on OTHER objects run concurrently on the GPU (every index and every environment has its own stream);
- * a second host-pointer call on an object with a pending call is refused with SFFG_ERR_ARG; *_device launches on an
+ * a second host-pointer call on an object with a pending call is refused with SFFG_ERR_ARG (of the indices of a multi
+ * call only idx[0] holds the pending call; the others stay usable without an end call); *_device launches on an
  * environment with a pending call are ordered behind it by the library (like all launches of one environment), *_device
  * calls on an index with a pending call share that index's scratch buffers and are the caller's to order.  Appends are ordered before
  * every later search on the indices they went to without any host synchronisation.  Batches too large for the pinned

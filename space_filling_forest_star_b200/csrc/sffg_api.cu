@@ -9,7 +9,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "bvh_device.cuh"
@@ -29,8 +31,94 @@ int fail(int code, const std::string &msg) {
 
 namespace {
 
-constexpr size_t kSmallBytes = 1 << 20;        // staging for small calls: inputs in the first 3/4, outputs in the last 1/4
-constexpr size_t kSmallIn = 768 << 10;
+constexpr size_t kSmallBytes = 1 << 20;   // pinned, device-mapped staging area of each object for planner-sized calls
+
+// The environment's staging area: inputs in the first 3/4, outputs in the last 1/4.  The outputs of a pose call are its
+// verdicts; those of an edge call are first hits [m] then free flags [m]; those of a move call are free flags [m] then
+// pose hits [m].
+struct EnvStaging {
+  static constexpr size_t kInBytes = 768 << 10;
+  static constexpr size_t kOutBytes = kSmallBytes - kInBytes;
+  unsigned char *base;
+  unsigned char *in() const { return base; }
+  uint8_t *out() const { return base + kInBytes; }
+  int32_t *edge_first_hit() const { return reinterpret_cast<int32_t *>(out()); }
+  uint8_t *edge_free(int64_t m) const { return out() + (size_t)m * 4; }
+  uint8_t *move_free() const { return out(); }
+  uint8_t *move_hit(int64_t m) const { return out() + (size_t)m; }
+};
+
+// The index's staging area.  The first 64 KiB hold the queries; the one-kernel radius search keeps its fallback flag in
+// their last 16 bytes.  After them:
+//   k-NN:    ids [nq * k], then d2 [nq * k]
+//   radius:  counts [nq] (64 KiB), then from 128 KiB the rows part: a head, ids [cap], d2 [cap].  The head is the row
+//            offsets [nq] (one-kernel form) or the total (one-sync form); the two-sync form has no head and stages the
+//            row offsets in the query part instead.
+// sffg_index_add_multi_begin uses the whole area for the rows to append.
+struct IndexStaging {
+  static constexpr size_t kQueryBytes = 64 << 10;
+  static constexpr size_t kCountBytes = 64 << 10;
+  static constexpr size_t kRowsAt = 128 << 10;
+  static constexpr size_t kRowsBytes = kSmallBytes - kRowsAt;
+  static constexpr size_t kKnnOutBytes = kSmallBytes - kQueryBytes;
+  static constexpr size_t kFlagAt = kQueryBytes - 16;
+  // entries of ids and of d2 that fit behind a head of `head_bytes`
+  static int64_t rows_cap(size_t head_bytes) { return (int64_t)((kRowsBytes - head_bytes) / 8); }
+  unsigned char *base;
+  unsigned char *queries() const { return base; }
+  int *fused_flag() const { return reinterpret_cast<int *>(base + kFlagAt); }
+  int32_t *knn_ids() const { return reinterpret_cast<int32_t *>(base + kQueryBytes); }
+  float *knn_d2(size_t obytes) const { return reinterpret_cast<float *>(base + kQueryBytes + obytes); }
+  int32_t *counts() const { return reinterpret_cast<int32_t *>(base + kQueryBytes); }
+  int64_t *rows_head() const { return reinterpret_cast<int64_t *>(base + kRowsAt); }
+  int32_t *rows_ids(size_t head_bytes) const { return reinterpret_cast<int32_t *>(base + kRowsAt + head_bytes); }
+  float *rows_d2(size_t head_bytes, int64_t cap) const {
+    return reinterpret_cast<float *>(base + kRowsAt + head_bytes + (size_t)cap * 4);
+  }
+};
+
+// enqueues an upload of host data on `st`, through `staging` (pinned) unless it is null
+cudaError_t upload_async(void *dst, const void *src, size_t bytes, unsigned char *staging, cudaStream_t st) {
+  if (staging) src = std::memcpy(staging, src, bytes);
+  return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+}
+
+// owners of CUDA resources: released when the owning object goes away
+struct CudaFree { void operator()(void *p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void *p) const { cudaFreeHost(p); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <class T> using PinnedPtr = std::unique_ptr<T, CudaFreeHost>;   // cudaHostAllocMapped
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+// hands the handle that `create` writes to the owner, once the call has succeeded
+template <class Owner, class Create> cudaError_t make(Owner &o, Create create) {
+  typename Owner::pointer h = nullptr;
+  const cudaError_t e = create(&h);
+  if (e == cudaSuccess) o.reset(h);
+  return e;
+}
+template <class T> cudaError_t dev_alloc(DevPtr<T> &o, size_t bytes) {
+  return make(o, [&](T **p) { return cudaMalloc(p, bytes); });
+}
+template <class T> cudaError_t host_alloc(PinnedPtr<T> &o, size_t bytes) {
+  return make(o, [&](T **p) { return cudaHostAlloc(p, bytes, cudaHostAllocMapped); });
+}
+cudaError_t make_stream(Stream &o) {
+  return make(o, [](cudaStream_t *s) { return cudaStreamCreateWithFlags(s, cudaStreamNonBlocking); });
+}
+cudaError_t make_event(Event &o) {
+  return make(o, [](cudaEvent_t *e) { return cudaEventCreateWithFlags(e, cudaEventDisableTiming); });
+}
+// a device copy of `n` bytes of host data (at least 16 bytes allocated); adds `n` to *counted
+template <class T> cudaError_t upload(DevPtr<T> &dst, const void *src, size_t n, size_t *counted) {
+  cudaError_t e = dev_alloc(dst, std::max<size_t>(n, 16));
+  if (e != cudaSuccess) return e;
+  *counted += n;
+  return n ? cudaMemcpy(dst.get(), src, n, cudaMemcpyHostToDevice) : cudaSuccess;
+}
 
 struct Runtime {
   bool ready = false;
@@ -56,6 +144,10 @@ int ensure_runtime() {
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  ~DevBuf() { release(); }
   int reserve(size_t bytes) {
     if (bytes <= cap) return SFFG_OK;
     if (p) cudaFree(p);
@@ -73,15 +165,6 @@ struct DevBuf {
   }
 };
 
-bool is_device_accessible_host(const void *p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-    cudaGetLastError();
-    return false;
-  }
-  return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
-}
-
 }  // namespace
 }  // namespace sffg
 
@@ -90,21 +173,26 @@ using namespace sffg;
 // ---------------------------------------------------------------------------------------------------------------
 struct sffg_env {
   EnvDev dev{};
-  void *d_slots = nullptr, *d_top = nullptr, *d_clear = nullptr, *d_tris32 = nullptr, *d_tris64 = nullptr, *d_robot = nullptr, *d_robot64 = nullptr;
-  void *d_order = nullptr;                       // leaf position -> caller's triangle index (refit)
+  DevPtr<ChildSlot> d_slots, d_top;
+  DevPtr<unsigned> d_clear;
+  DevPtr<float4> d_tris32;
+  DevPtr<double> d_tris64, d_robot64;
+  DevPtr<RobotTri> d_robot;
+  DevPtr<int> d_order;                           // leaf position -> caller's triangle index (refit)
   std::vector<int> level_base, level_count;      // breadth-first level table of the hierarchy (refit)
   int64_t obst_bytes = 0;
-  unsigned long long *d_counters = nullptr;
-  int *h_status = nullptr;      // pinned + device-mapped: the kernels raise it, the host reads it without a copy
-  unsigned *d_work = nullptr;   // ring of 8 work counters (never reset; see launch_collide_poses)
+  DevPtr<unsigned long long> d_counters;
+  PinnedPtr<int> h_status;      // the kernels raise it, the host reads it without a copy
+  DevPtr<unsigned> d_work;      // ring of 8 work counters (never reset; see launch_collide_poses)
   unsigned work_base[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   int work_next = 0;
-  unsigned char *h_small = nullptr;   // pinned + device-mapped staging for small calls (planner-sized batches)
-  cudaStream_t streams[2] = {nullptr, nullptr};
+  PinnedPtr<unsigned char> h_small;   // staging for small calls (planner-sized batches), see EnvStaging
+  EnvStaging staging() const { return {h_small.get()}; }
+  Stream streams[2];
   // launches of one environment share state (the ring of work counters, the first-hit scratch `fh`), so they are kept in
   // order across whatever streams the caller uses: every *_device launch records order_ev, and a launch on another
   // stream (or an internal stream of the host-pointer calls) first waits for it
-  cudaEvent_t order_ev = nullptr;
+  Event order_ev;
   cudaStream_t last_stream = nullptr;
   bool order_pending = false;
   DevBuf in[2], out[2], aux[2], fh;   // fh: per-edge first-hit scratch of small edge batches
@@ -127,13 +215,14 @@ static int env_busy(const sffg_env *env, const char *who) {
 
 struct sffg_index {
   int dim = 0;
-  float *d_coords = nullptr;
-  unsigned *d_amax = nullptr;   // float bits of the largest |angle| stored (dim 6): selects the kernels' exact wide wrap
+  DevPtr<float> d_coords;
+  DevPtr<unsigned> d_amax;   // float bits of the largest |angle| stored (dim 6): selects the kernels' exact wide wrap
   int64_t cap = 0, n = 0;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t ev = nullptr;   // fork / join of multi-index calls
+  Stream stream;
+  Event ev;   // fork / join of multi-index calls
   DevBuf q, ids, d2, scratch, counts, offsets, cursor, keys, stage;
-  unsigned char *h_small = nullptr;   // pinned + device-mapped staging for planner-sized queries
+  PinnedPtr<unsigned char> h_small;   // staging for planner-sized queries, see IndexStaging
+  IndexStaging staging() const { return {h_small.get()}; }
   // spatially sorted view (knn_pruned.cu): covers nodes [0, n_sorted); rebuilt when the unsorted tail grows too long
   DevBuf s_coords, s_ids, s_bb, s_keys, s_vals, s_temp, s_bounds;
   int64_t n_sorted = 0, s_cap = 0, s_nblk_cap = 0;
@@ -153,8 +242,8 @@ struct sffg_index {
     bool small = false, one_sync = false, pruned = false, fused = false;
     const float *queries = nullptr;
   } pend;
-  cudaEvent_t add_ev = nullptr;   // appends enqueued by sffg_index_add_multi_begin have run
-  unsigned long long *d_total = nullptr;   // row allocator of the one-kernel radius search
+  Event add_ev;   // appends enqueued by sffg_index_add_multi_begin have run
+  DevPtr<unsigned long long> d_total;   // row allocator of the one-kernel radius search
 };
 static int index_busy(const sffg_index *idx, const char *who) {
   if (idx->pend.kind != 0) return fail(SFFG_ERR_ARG, std::string(who) + ": an asynchronous call on this index is pending (sffg_index_end first)");
@@ -274,29 +363,8 @@ static void make_robot_tri(const double *t, RobotTri *o) {
 
 int sffg_env_destroy(sffg_env *env) {
   if (!env) return SFFG_OK;
-  for (int s = 0; s < 2; ++s) {
-    if (env->streams[s]) cudaStreamSynchronize(env->streams[s]);
-  }
-  cudaFree(env->d_slots);
-  cudaFree(env->d_order);
-  cudaFree(env->d_top);
-  cudaFree(env->d_clear);
-  cudaFree(env->d_tris32);
-  cudaFree(env->d_tris64);
-  cudaFree(env->d_robot);
-  cudaFree(env->d_robot64);
-  cudaFree(env->d_counters);
-  if (env->order_ev) cudaEventDestroy(env->order_ev);
-  if (env->h_status) cudaFreeHost(env->h_status);
-  if (env->h_small) cudaFreeHost(env->h_small);
-  cudaFree(env->d_work);
-  for (int s = 0; s < 2; ++s) {
-    env->in[s].release();
-    env->out[s].release();
-    env->aux[s].release();
-    env->fh.release();
-    if (env->streams[s]) cudaStreamDestroy(env->streams[s]);
-  }
+  for (const Stream &s : env->streams)
+    if (s) cudaStreamSynchronize(s.get());
   delete env;
   return SFFG_OK;
 }
@@ -309,18 +377,9 @@ constexpr int64_t kDeviceBuildMin = 1 << 18;   // SFFG_BUILD_AUTO: triangle coun
 static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, const double root_lo[3], const double root_hi[3],
                             int64_t n_obst, int64_t n_nodes, int depth, bool on_device, size_t bytes) {
   EnvDev &d = env->dev;
-  cudaFree(env->d_top);
-  env->d_top = nullptr;
-  cudaFree(env->d_clear);
-  env->d_clear = nullptr;
-  auto upload = [&](void **dst, const void *src, size_t n) -> cudaError_t {
-    cudaError_t e = cudaMalloc(dst, std::max<size_t>(n, 16));
-    if (e != cudaSuccess) return e;
-    bytes += n;
-    if (n) e = cudaMemcpy(*dst, src, n, cudaMemcpyHostToDevice);
-    return e;
-  };
-  SFFG_CUDA(upload(&env->d_top, top.data(), top.size() * sizeof(ChildSlot)));
+  env->d_top.reset();
+  env->d_clear.reset();
+  SFFG_CUDA(upload(env->d_top, top.data(), top.size() * sizeof(ChildSlot), &bytes));
   d.n_obst = (int)n_obst;
   for (int k = 0; k < 3; ++k) {
     const double oc = 0.5 * (root_lo[k] + root_hi[k]);
@@ -354,13 +413,13 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
     // reach = bounding radius + half cell diagonal + margins for float rounding of vertices, cell lookup and distances
     const double reach = (rho + 0.8661 * h) * 1.002 + 1e-3 * h + maxc * 3.9e-6;
     const size_t words = ((size_t)gn[0] * gn[1] * gn[2] + 31) / 32;
-    SFFG_CUDA(cudaMalloc(&env->d_clear, words * sizeof(unsigned)));
-    SFFG_CUDA(cudaMemset(env->d_clear, 0, words * sizeof(unsigned)));
-    SFFG_CUDA(launch_build_clearance(reinterpret_cast<const float4 *>(env->d_tris32), (int)n_obst, go, (float)h, gn, (float)reach,
-                                         (unsigned *)env->d_clear, env->streams[0]));
-    SFFG_CUDA(cudaStreamSynchronize(env->streams[0]));
+    SFFG_CUDA(dev_alloc(env->d_clear, words * sizeof(unsigned)));
+    SFFG_CUDA(cudaMemset(env->d_clear.get(), 0, words * sizeof(unsigned)));
+    SFFG_CUDA(launch_build_clearance(env->d_tris32.get(), (int)n_obst, go, (float)h, gn, (float)reach, env->d_clear.get(),
+                                     env->streams[0].get()));
+    SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
     bytes += words * sizeof(unsigned);
-    d.clear_bits = reinterpret_cast<const unsigned *>(env->d_clear);
+    d.clear_bits = env->d_clear.get();
     for (int k = 0; k < 3; ++k) {
       d.grid_o[k] = go[k];
       d.grid_n[k] = gn[k];
@@ -369,16 +428,16 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
     env->info.grid_cells = (int64_t)gn[0] * gn[1] * gn[2];
     env->info.grid_cell_size = h;
   }
-  d.slots = reinterpret_cast<const float4 *>(env->d_slots);
-  d.top = reinterpret_cast<const float4 *>(env->d_top);
+  d.slots = reinterpret_cast<const float4 *>(env->d_slots.get());
+  d.top = reinterpret_cast<const float4 *>(env->d_top.get());
   d.n_top = (int)top.size();
   {
     // leading (breadth-first) nodes a CTA stages in shared memory: what fits next to the robot and the warp scratch
     const int64_t room = ((int64_t)g_rt.smem_optin - 1024 - (int64_t)collide_smem_bytes(d.n_robot, 0)) / (int64_t)(kWide * sizeof(ChildSlot));
     d.n_stage_max = (int)std::max<int64_t>(0, std::min<int64_t>({n_nodes, (int64_t)kStageNodesCap, room}));
   }
-  d.tris32 = reinterpret_cast<const float4 *>(env->d_tris32);
-  d.tris64 = reinterpret_cast<const double *>(env->d_tris64);
+  d.tris32 = env->d_tris32.get();
+  d.tris64 = env->d_tris64.get();
   env->info.n_obst_tris = n_obst;
   env->info.n_nodes = n_nodes;
   env->info.depth = depth;
@@ -387,24 +446,32 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   return SFFG_OK;
 }
 
+// the caller's soup (9 doubles per triangle) in a temporary device block, copied on the environment's first stream
+static cudaError_t upload_soup(sffg_env *env, DevPtr<double> &d_soup, const double *tris, int64_t n) {
+  const size_t bytes = 9 * (size_t)n * sizeof(double);
+  const cudaError_t e = dev_alloc(d_soup, bytes);
+  return e == cudaSuccess ? cudaMemcpyAsync(d_soup.get(), tris, bytes, cudaMemcpyHostToDevice, env->streams[0].get()) : e;
+}
+
+// the cut through the top of the device-resident hierarchy, chosen on the host from its first levels (nodes are stored
+// level by level)
+static int read_top_cut(const sffg_env *env, int64_t n_nodes, std::vector<ChildSlot> *top) {
+  HostBvh head;
+  head.slots.resize((size_t)std::min<int64_t>(n_nodes, 1 + 8 + 64) * kWide);
+  SFFG_CUDA(cudaMemcpy(head.slots.data(), env->d_slots.get(), head.slots.size() * sizeof(ChildSlot), cudaMemcpyDeviceToHost));
+  top_cut(head, top);
+  return SFFG_OK;
+}
+
 static int set_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obst, int build_mode) {
   const bool on_device = n_obst > 0 && (build_mode == SFFG_BUILD_DEVICE || (build_mode == SFFG_BUILD_AUTO && n_obst >= kDeviceBuildMin));
-  void **olds[] = {&env->d_slots, &env->d_tris32, &env->d_tris64, &env->d_order};
   env->level_base.clear();
   env->level_count.clear();
-  for (void **p : olds) {
-    cudaFree(*p);
-    *p = nullptr;
-  }
-  EnvDev &d = env->dev;
+  env->d_slots.reset();
+  env->d_tris32.reset();
+  env->d_tris64.reset();
+  env->d_order.reset();
   size_t bytes = 0;
-  auto upload = [&](void **dst, const void *src, size_t n) -> cudaError_t {
-    cudaError_t e = cudaMalloc(dst, std::max<size_t>(n, 16));
-    if (e != cudaSuccess) return e;
-    bytes += n;
-    if (n) e = cudaMemcpy(*dst, src, n, cudaMemcpyHostToDevice);
-    return e;
-  };
   double root_lo[3] = {0, 0, 0}, root_hi[3] = {0, 0, 0};
   std::vector<ChildSlot> top;
   int64_t n_nodes = 0;
@@ -429,10 +496,10 @@ static int set_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obst,
       }
       t32[(size_t)i].p[0][3] = round_up_f32(err * 1.0000001);
     }
-    SFFG_CUDA(upload(&env->d_slots, bvh.slots.data(), bvh.slots.size() * sizeof(ChildSlot)));
-    SFFG_CUDA(upload(&env->d_tris32, t32.data(), t32.size() * sizeof(TriF32)));
-    SFFG_CUDA(upload(&env->d_tris64, t64.data(), t64.size() * sizeof(double)));
-    SFFG_CUDA(upload(&env->d_order, bvh.tri_order.data(), bvh.tri_order.size() * sizeof(int32_t)));
+    SFFG_CUDA(upload(env->d_slots, bvh.slots.data(), bvh.slots.size() * sizeof(ChildSlot), &bytes));
+    SFFG_CUDA(upload(env->d_tris32, t32.data(), t32.size() * sizeof(TriF32), &bytes));
+    SFFG_CUDA(upload(env->d_tris64, t64.data(), t64.size() * sizeof(double), &bytes));
+    SFFG_CUDA(upload(env->d_order, bvh.tri_order.data(), bvh.tri_order.size() * sizeof(int32_t), &bytes));
     env->level_base = bvh.level_base;
     env->level_count = bvh.level_count;
     top_cut(bvh, &top);
@@ -444,30 +511,24 @@ static int set_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obst,
     }
   } else {
     // ---- device: Morton-ordered 8-wide hierarchy built by bvh_device.cu from the uploaded soup
-    void *d_soup = nullptr;
-    size_t dummy = 0;
-    (void)dummy;
-    SFFG_CUDA(cudaMalloc(&d_soup, 9 * (size_t)n_obst * sizeof(double)));
-    cudaError_t e = cudaMemcpyAsync(d_soup, obst_tris, 9 * (size_t)n_obst * sizeof(double), cudaMemcpyHostToDevice, env->streams[0]);
+    DevPtr<double> d_soup;
+    cudaError_t e = upload_soup(env, d_soup, obst_tris, n_obst);
     DeviceBvh db;
-    if (e == cudaSuccess) e = build_bvh_device((const double *)d_soup, (int)n_obst, env->streams[0], &db);
-    cudaFree(d_soup);
+    if (e == cudaSuccess) e = build_bvh_device(d_soup.get(), (int)n_obst, env->streams[0].get(), &db);
+    d_soup.reset();
+    env->d_slots.reset(db.d_slots);
+    env->d_tris32.reset(db.d_tris32);
+    env->d_tris64.reset(db.d_tris64);
+    env->d_order.reset(db.d_order);
     if (e != cudaSuccess) {
       cudaGetLastError();
       return fail(SFFG_ERR_CUDA, std::string("device BVH build: ") + cudaGetErrorString(e));
     }
-    env->d_slots = db.d_slots;
-    env->d_tris32 = db.d_tris32;
-    env->d_tris64 = db.d_tris64;
-    env->d_order = db.d_order;
     env->level_base = db.level_base;
     env->level_count = db.level_count;
     bytes += (size_t)db.n_nodes * kWide * sizeof(ChildSlot) + (size_t)n_obst * (sizeof(TriF32) + 9 * sizeof(double));
-    // the cut through the top of the hierarchy is chosen on the host from the first levels (nodes are stored level by level)
-    HostBvh head;
-    head.slots.resize((size_t)std::min<int64_t>(db.n_nodes, 1 + 8 + 64) * kWide);
-    SFFG_CUDA(cudaMemcpy(head.slots.data(), env->d_slots, head.slots.size() * sizeof(ChildSlot), cudaMemcpyDeviceToHost));
-    top_cut(head, &top);
+    const int rc = read_top_cut(env, db.n_nodes, &top);
+    if (rc != SFFG_OK) return rc;
     n_nodes = db.n_nodes;
     depth = db.depth;
     for (int k = 0; k < 3; ++k) {
@@ -495,16 +556,7 @@ int sffg_env_create_ex(const double *obst_tris, int64_t n_obst, const double *ro
   }
   const auto t0 = std::chrono::steady_clock::now();
 
-  sffg_env *env = new sffg_env();
-  auto bail = [&](int code) {
-    sffg_env_destroy(env);
-    return code;
-  };
-#define SFFG_ENV_CUDA(expr)                                                                                       \
-  do {                                                                                                            \
-    cudaError_t e_ = (expr);                                                                                      \
-    if (e_ != cudaSuccess) return bail(fail(SFFG_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e_)));   \
-  } while (0)
+  std::unique_ptr<sffg_env, int (*)(sffg_env *)> env(new sffg_env(), sffg_env_destroy);   // released on every error return
 
   // ---- robot
   std::vector<RobotTri> rob((size_t)n_robot);
@@ -531,40 +583,32 @@ int sffg_env_create_ex(const double *obst_tris, int64_t n_obst, const double *ro
   d.rob_radius = round_up_f32(std::sqrt(rad2) * 1.000001);
 
   size_t bytes = 0;
-  auto upload = [&](void **dst, const void *src, size_t n) -> cudaError_t {
-    cudaError_t e = cudaMalloc(dst, std::max<size_t>(n, 16));
-    if (e != cudaSuccess) return e;
-    bytes += n;
-    if (n) e = cudaMemcpy(*dst, src, n, cudaMemcpyHostToDevice);
-    return e;
-  };
-  SFFG_ENV_CUDA(upload(&env->d_robot, rob.data(), rob.size() * sizeof(RobotTri)));
-  SFFG_ENV_CUDA(upload(&env->d_robot64, robot_tris, 9 * (size_t)n_robot * sizeof(double)));
-  SFFG_ENV_CUDA(cudaMalloc((void **)&env->d_counters, 10 * sizeof(unsigned long long)));
-  SFFG_ENV_CUDA(cudaMemset(env->d_counters, 0, 10 * sizeof(unsigned long long)));
-  SFFG_ENV_CUDA(cudaHostAlloc((void **)&env->h_status, sizeof(int), cudaHostAllocMapped));
+  SFFG_CUDA(upload(env->d_robot, rob.data(), rob.size() * sizeof(RobotTri), &bytes));
+  SFFG_CUDA(upload(env->d_robot64, robot_tris, 9 * (size_t)n_robot * sizeof(double), &bytes));
+  SFFG_CUDA(dev_alloc(env->d_counters, 10 * sizeof(unsigned long long)));
+  SFFG_CUDA(cudaMemset(env->d_counters.get(), 0, 10 * sizeof(unsigned long long)));
+  SFFG_CUDA(host_alloc(env->h_status, sizeof(int)));
   *env->h_status = 0;
-  SFFG_ENV_CUDA(cudaHostAlloc((void **)&env->h_small, kSmallBytes, cudaHostAllocMapped));
-  SFFG_ENV_CUDA(cudaMalloc((void **)&env->d_work, 8 * sizeof(unsigned)));
-  SFFG_ENV_CUDA(cudaMemset(env->d_work, 0, 8 * sizeof(unsigned)));
-  for (int s = 0; s < 2; ++s) SFFG_ENV_CUDA(cudaStreamCreateWithFlags(&env->streams[s], cudaStreamNonBlocking));
-  SFFG_ENV_CUDA(cudaEventCreateWithFlags(&env->order_ev, cudaEventDisableTiming));
-  d.robot = reinterpret_cast<const RobotTri *>(env->d_robot);
-  d.robot64 = reinterpret_cast<const double *>(env->d_robot64);
+  SFFG_CUDA(host_alloc(env->h_small, kSmallBytes));
+  SFFG_CUDA(dev_alloc(env->d_work, 8 * sizeof(unsigned)));
+  SFFG_CUDA(cudaMemset(env->d_work.get(), 0, 8 * sizeof(unsigned)));
+  for (Stream &s : env->streams) SFFG_CUDA(make_stream(s));
+  SFFG_CUDA(make_event(env->order_ev));
+  d.robot = env->d_robot.get();
+  d.robot64 = env->d_robot64.get();
   d.counters = nullptr;
-  d.status = env->h_status;   // unified addressing: the mapped host pointer is valid on the device
-  d.work_counter = env->d_work;
+  d.status = env->h_status.get();   // unified addressing: the mapped host pointer is valid on the device
+  d.work_counter = env->d_work.get();
   env->cfg.sm_count = g_rt.sm_count;
   env->cfg.blocks_per_sm = 0;
 
   env->info.n_robot_tris = n_robot;
   env->robot_bytes = (int64_t)bytes;
-  rc = set_obstacles(env, obst_tris, n_obst, build_mode);
-  if (rc != SFFG_OK) return bail(rc);
+  rc = set_obstacles(env.get(), obst_tris, n_obst, build_mode);
+  if (rc != SFFG_OK) return rc;
   env->info.build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  *out = env;
+  *out = env.release();
   return SFFG_OK;
-#undef SFFG_ENV_CUDA
 }
 
 int sffg_env_create(const double *obst_tris, int64_t n_obst, const double *robot_tris, int64_t n_robot, sffg_env **out) {
@@ -574,11 +618,13 @@ int sffg_env_create(const double *obst_tris, int64_t n_obst, const double *robot
 int sffg_env_set_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obst, int build_mode) {
   if (!env || n_obst < 0 || (n_obst > 0 && !obst_tris) || n_obst > 0x3fffffff || build_mode < 0 || build_mode > 2)
     return fail(SFFG_ERR_ARG, "sffg_env_set_obstacles: bad arguments");
+  int rc = env_busy(env, "sffg_env_set_obstacles");
+  if (rc != SFFG_OK) return rc;
   SFFG_CUDA(cudaDeviceSynchronize());   // nothing may still be traversing the old hierarchy
   const auto t0 = std::chrono::steady_clock::now();
   env->dev.n_obst = 0;
   *env->h_status = 4;                   // until the new set is complete every verdict call reports an error, never "free"
-  int rc = set_obstacles(env, obst_tris, n_obst, build_mode);
+  rc = set_obstacles(env, obst_tris, n_obst, build_mode);
   if (rc == SFFG_OK) *env->h_status = 0;
   env->info.build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return rc;
@@ -586,32 +632,31 @@ int sffg_env_set_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obs
 
 int sffg_env_refit_obstacles(sffg_env *env, const double *obst_tris, int64_t n_obst) {
   if (!env || !obst_tris || n_obst <= 0) return fail(SFFG_ERR_ARG, "sffg_env_refit_obstacles: bad arguments");
+  int rc = env_busy(env, "sffg_env_refit_obstacles");
+  if (rc != SFFG_OK) return rc;
   if (n_obst != env->info.n_obst_tris || !env->d_order || env->level_base.empty())
     return fail(SFFG_ERR_ARG, "sffg_env_refit_obstacles: the soup must have the " + std::to_string(env->info.n_obst_tris) +
                                   " triangles of the current obstacle set, in the same order (use sffg_env_set_obstacles otherwise)");
   SFFG_CUDA(cudaDeviceSynchronize());   // nothing may still be traversing the boxes that are about to move
   const auto t0 = std::chrono::steady_clock::now();
   *env->h_status = 4;                   // until the refit is complete every verdict call reports an error, never "free"
-  void *d_soup = nullptr;
-  SFFG_CUDA(cudaMalloc(&d_soup, 9 * (size_t)n_obst * sizeof(double)));
-  cudaError_t e = cudaMemcpyAsync(d_soup, obst_tris, 9 * (size_t)n_obst * sizeof(double), cudaMemcpyHostToDevice, env->streams[0]);
+  DevPtr<double> d_soup;
+  cudaError_t e = upload_soup(env, d_soup, obst_tris, n_obst);
   double root_lo[3], root_hi[3];
   if (e == cudaSuccess)
-    e = refit_bvh_device((const double *)d_soup, (int)n_obst, (ChildSlot *)env->d_slots, (double *)env->d_tris64, (float4 *)env->d_tris32,
-                         (const int *)env->d_order, env->level_base, env->level_count, env->streams[0], root_lo, root_hi);
-  cudaFree(d_soup);
+    e = refit_bvh_device(d_soup.get(), (int)n_obst, env->d_slots.get(), env->d_tris64.get(), env->d_tris32.get(), env->d_order.get(),
+                         env->level_base, env->level_count, env->streams[0].get(), root_lo, root_hi);
+  d_soup.reset();
   if (e != cudaSuccess) {
     cudaGetLastError();
     return fail(SFFG_ERR_CUDA, std::string("refit: ") + cudaGetErrorString(e));
   }
-  // the cut through the top of the hierarchy is re-chosen from the refitted head (its boxes changed)
-  HostBvh head;
-  head.slots.resize((size_t)std::min<int64_t>(env->info.n_nodes, 1 + 8 + 64) * kWide);
-  SFFG_CUDA(cudaMemcpy(head.slots.data(), env->d_slots, head.slots.size() * sizeof(ChildSlot), cudaMemcpyDeviceToHost));
+  // the top cut is re-chosen from the refitted head (its boxes changed)
   std::vector<ChildSlot> top;
-  top_cut(head, &top);
-  int rc = finish_obstacles(env, top, root_lo, root_hi, n_obst, env->info.n_nodes, env->info.depth, env->info.built_on_device != 0,
-                            (size_t)env->obst_bytes);
+  rc = read_top_cut(env, env->info.n_nodes, &top);
+  if (rc != SFFG_OK) return rc;
+  rc = finish_obstacles(env, top, root_lo, root_hi, n_obst, env->info.n_nodes, env->info.depth, env->info.built_on_device != 0,
+                        (size_t)env->obst_bytes);
   if (rc == SFFG_OK) *env->h_status = 0;
   env->info.build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return rc;
@@ -626,7 +671,7 @@ int sffg_env_info(const sffg_env *env, sffg_env_info_t *out) {
 int sffg_env_enable_counters(sffg_env *env, int on) {
   if (!env) return fail(SFFG_ERR_ARG, "null env");
   env->count = on != 0;
-  SFFG_CUDA(cudaMemset(env->d_counters, 0, 10 * sizeof(unsigned long long)));
+  SFFG_CUDA(cudaMemset(env->d_counters.get(), 0, 10 * sizeof(unsigned long long)));
   return SFFG_OK;
 }
 
@@ -634,7 +679,7 @@ int sffg_env_read_counters(sffg_env *env, sffg_counters_t *out) {
   if (!env || !out) return fail(SFFG_ERR_ARG, "null argument");
   unsigned long long h[10];
   SFFG_CUDA(cudaDeviceSynchronize());
-  SFFG_CUDA(cudaMemcpy(h, env->d_counters, sizeof h, cudaMemcpyDeviceToHost));
+  SFFG_CUDA(cudaMemcpy(h, env->d_counters.get(), sizeof h, cudaMemcpyDeviceToHost));
   out->poses = (int64_t)h[0];
   out->poses_past_root = (int64_t)h[1];
   out->box_tests = (int64_t)h[2];
@@ -652,19 +697,19 @@ int sffg_env_read_counters(sffg_env *env, sffg_counters_t *out) {
 static EnvDev env_view(sffg_env *env, unsigned **base_io) {
   EnvDev v = env->dev;
   const int slot = env->work_next++ & 7;
-  v.counters = env->count ? env->d_counters : nullptr;
-  v.work_counter = env->d_work + slot;
+  v.counters = env->count ? env->d_counters.get() : nullptr;
+  v.work_counter = env->d_work.get() + slot;
   *base_io = &env->work_base[slot];
   return v;
 }
 
 // stream ordering of the launches of one environment (see sffg_env::order_ev)
 static int env_enter(sffg_env *env, cudaStream_t st) {
-  if (env->order_pending && env->last_stream != st) SFFG_CUDA(cudaStreamWaitEvent(st, env->order_ev, 0));
+  if (env->order_pending && env->last_stream != st) SFFG_CUDA(cudaStreamWaitEvent(st, env->order_ev.get(), 0));
   return SFFG_OK;
 }
 static int env_leave(sffg_env *env, cudaStream_t st) {
-  SFFG_CUDA(cudaEventRecord(env->order_ev, st));
+  SFFG_CUDA(cudaEventRecord(env->order_ev.get(), st));
   env->last_stream = st;
   env->order_pending = true;
   return SFFG_OK;
@@ -676,8 +721,7 @@ static int env_enter_host(sffg_env *env) {
     if (rc != SFFG_OK) return rc;
   }
   if (env->order_pending) {
-    SFFG_CUDA(cudaStreamWaitEvent(env->streams[0], env->order_ev, 0));
-    SFFG_CUDA(cudaStreamWaitEvent(env->streams[1], env->order_ev, 0));
+    for (const Stream &s : env->streams) SFFG_CUDA(cudaStreamWaitEvent(s.get(), env->order_ev.get(), 0));
     env->order_pending = false;   // everything recorded so far is complete once this call has synchronised
   }
   return SFFG_OK;
@@ -685,10 +729,11 @@ static int env_enter_host(sffg_env *env) {
 
 // call after the streams were synchronised
 static int check_status(sffg_env *env) {
-  const int st = *reinterpret_cast<volatile int *>(env->h_status);
+  const int st = *reinterpret_cast<volatile int *>(env->h_status.get());
   if (st != 0) {
-    if (st == 4)   // sticky: stays until sffg_env_set_obstacles succeeds
-      return fail(SFFG_ERR_INTERNAL, "the environment has no valid obstacle set: the last sffg_env_set_obstacles failed");
+    if (st == 4)   // sticky: stays until sffg_env_set_obstacles or sffg_env_refit_obstacles succeeds
+      return fail(SFFG_ERR_INTERNAL,
+                  "the environment has no valid obstacle set: the last sffg_env_set_obstacles or sffg_env_refit_obstacles failed");
     *env->h_status = 0;
     if (st == 3) return fail(SFFG_ERR_INTERNAL, "peer barrier timed out: a rank of the gather group never signalled");
     return fail(SFFG_ERR_INTERNAL, "BVH traversal stack overflow: results of this call are invalid");
@@ -811,7 +856,7 @@ int sffg_peer_wait_device(sffg_env *env, uint32_t *const *d_flags, int n_ranks, 
   FlagSet f;
   int rc = fill_flags(&f, d_flags, n_ranks, my_rank, "sffg_peer_wait_device");
   if (rc != SFFG_OK) return rc;
-  SFFG_CUDA(launch_peer_barrier(f, epoch, false, env ? env->h_status : nullptr, (cudaStream_t)stream));
+  SFFG_CUDA(launch_peer_barrier(f, epoch, false, env ? env->h_status.get() : nullptr, (cudaStream_t)stream));
   return SFFG_OK;
 }
 
@@ -820,7 +865,7 @@ int sffg_peer_barrier_device(sffg_env *env, uint32_t *const *d_flags, int n_rank
   int rc = fill_flags(&f, d_flags, n_ranks, my_rank, "sffg_peer_barrier_device");
   if (rc != SFFG_OK) return rc;
   SFFG_CUDA(launch_peer_barrier(f, epoch, true, nullptr, (cudaStream_t)stream));
-  SFFG_CUDA(launch_peer_barrier(f, epoch, false, env ? env->h_status : nullptr, (cudaStream_t)stream));
+  SFFG_CUDA(launch_peer_barrier(f, epoch, false, env ? env->h_status.get() : nullptr, (cudaStream_t)stream));
   return SFFG_OK;
 }
 
@@ -833,21 +878,22 @@ static int collide_poses_host(sffg_env *env, const void *poses, int fmt, int64_t
     const int rc0 = env_enter_host(env);
     if (rc0 != SFFG_OK) return rc0;
   }
-  if ((size_t)n * psz <= kSmallIn && (size_t)n <= kSmallBytes - kSmallIn) {
+  if ((size_t)n * psz <= EnvStaging::kInBytes && (size_t)n <= EnvStaging::kOutBytes) {
     // planner-sized call: one kernel reading/writing pinned mapped memory, one synchronisation, no DMA copies
-    cudaStream_t st = env->streams[0];
-    std::memcpy(env->h_small, poses, (size_t)n * psz);
+    cudaStream_t st = env->streams[0].get();
+    const EnvStaging h = env->staging();
+    std::memcpy(h.in(), poses, (size_t)n * psz);
     EnvDev v = env_view(env, &base);
-    SFFG_CUDA(launch_collide_poses(v, env->h_small, fmt, n, env->h_small + kSmallIn, st, env->cfg, env->count, base));
+    SFFG_CUDA(launch_collide_poses(v, h.in(), fmt, n, h.out(), st, env->cfg, env->count, base));
     SFFG_CUDA(cudaStreamSynchronize(st));
-    std::memcpy(verdict_out, env->h_small + kSmallIn, (size_t)n);
+    std::memcpy(verdict_out, h.out(), (size_t)n);
     return check_status(env);
   }
   const int64_t chunk = 1 << 20;
   int s = 0;
   for (int64_t off = 0; off < n; off += chunk, s ^= 1) {
     const int64_t cnt = std::min(chunk, n - off);
-    cudaStream_t st = env->streams[s];
+    cudaStream_t st = env->streams[s].get();
     SFFG_CUDA(cudaStreamSynchronize(st));   // buffers of this stream are free again
     int rc = env->in[s].reserve((size_t)cnt * psz);
     if (rc == SFFG_OK) rc = env->out[s].reserve((size_t)cnt);
@@ -857,8 +903,7 @@ static int collide_poses_host(sffg_env *env, const void *poses, int fmt, int64_t
     SFFG_CUDA(launch_collide_poses(v, env->in[s].p, fmt, cnt, (uint8_t *)env->out[s].p, st, env->cfg, env->count, base));
     SFFG_CUDA(cudaMemcpyAsync(verdict_out + off, env->out[s].p, (size_t)cnt, cudaMemcpyDeviceToHost, st));
   }
-  SFFG_CUDA(cudaStreamSynchronize(env->streams[0]));
-  SFFG_CUDA(cudaStreamSynchronize(env->streams[1]));
+  for (const Stream &st : env->streams) SFFG_CUDA(cudaStreamSynchronize(st.get()));
   return check_status(env);
 }
 
@@ -872,13 +917,21 @@ int sffg_collide_transforms_f64(sffg_env *env, const double *rt, int64_t n, uint
   return collide_poses_host(env, rt, 2, n, verdict_out);
 }
 
+// arguments of the edge and move calls
+static int check_segment_args(const sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist,
+                              int rot_mode, const uint8_t *out, const char *who) {
+  if (!env || m < 0 || (m > 0 && (!starts || !ends || !out)) || !(sample_dist > 0) ||
+      (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
+    return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments");
+  return SFFG_OK;
+}
+
 int sffg_check_edges_device(sffg_env *env, const double *d_starts, const double *d_ends, int64_t m, double sample_dist,
                             int rot_mode, uint8_t *d_free_out, int32_t *d_first_hit_out, void *stream) {
-  if (!env || m < 0 || (m > 0 && (!d_starts || !d_ends || !d_free_out)) || !(sample_dist > 0) ||
-      (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
-    return fail(SFFG_ERR_ARG, "sffg_check_edges_device: bad arguments");
+  int rc = check_segment_args(env, d_starts, d_ends, m, sample_dist, rot_mode, d_free_out, "sffg_check_edges_device");
+  if (rc != SFFG_OK) return rc;
   unsigned *base;
-  int rc = env_enter(env, (cudaStream_t)stream);
+  rc = env_enter(env, (cudaStream_t)stream);
   if (rc != SFFG_OK) return rc;
   EnvDev v = env_view(env, &base);
   int *scratch = nullptr;
@@ -910,60 +963,68 @@ int sffg_env_end(sffg_env *env) {
   if (env->pend.kind == 0) return SFFG_OK;
   const sffg_env::Pending c = env->pend;
   env->pend.kind = 0;
-  SFFG_CUDA(cudaStreamSynchronize(env->streams[0]));
+  SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
+  const EnvStaging h = env->staging();
   if (c.kind == 1) {
-    const int32_t *h_first = reinterpret_cast<const int32_t *>(env->h_small + kSmallIn);
-    const uint8_t *h_free = env->h_small + kSmallIn + (size_t)c.m * 4;
-    std::memcpy(c.out, h_free, (size_t)c.m);
-    if (c.first_out) std::memcpy(c.first_out, h_first, (size_t)c.m * 4);
+    std::memcpy(c.out, h.edge_free(c.m), (size_t)c.m);
+    if (c.first_out) std::memcpy(c.first_out, h.edge_first_hit(), (size_t)c.m * 4);
   } else {
-    const uint8_t *h_free = env->h_small + kSmallIn, *h_hit = h_free + (size_t)c.m;
+    const uint8_t *h_free = h.move_free(), *h_hit = h.move_hit(c.m);
     for (int64_t i = 0; i < c.m; ++i) c.out[i] = (uint8_t)(h_free[i] && !h_hit[i]);
   }
   return check_status(env);
 }
 
+// planner-sized edge and move calls: the end points go to device memory (starts, then ends) with one DMA from the
+// staging area, because every warp that shares an edge re-reads them
+static int stage_segments(sffg_env *env, const double *starts, const double *ends, int64_t m, double **ds, double **de) {
+  int rc = env->in[0].reserve((size_t)m * 96);
+  if (rc == SFFG_OK) rc = env->fh.reserve((size_t)m * sizeof(int));
+  if (rc != SFFG_OK) return rc;
+  unsigned char *h_in = env->staging().in();
+  std::memcpy(h_in, starts, (size_t)m * 48);
+  std::memcpy(h_in + (size_t)m * 48, ends, (size_t)m * 48);
+  *ds = (double *)env->in[0].p;
+  *de = *ds + 6 * m;
+  SFFG_CUDA(cudaMemcpyAsync(*ds, h_in, (size_t)m * 96, cudaMemcpyHostToDevice, env->streams[0].get()));
+  return SFFG_OK;
+}
+
+// the last step of a planner-sized edge or move call, once all of it is enqueued on the first stream: the blocking form
+// completes it, the asynchronous form leaves it pending for sffg_env_end (*_device launches issued before the end call are
+// ordered behind it)
+static int env_commit(sffg_env *env, const sffg_env::Pending &p, bool async) {
+  if (async) {
+    const int rc = env_leave(env, env->streams[0].get());
+    if (rc != SFFG_OK) return rc;
+  }
+  env->pend = p;
+  return async ? SFFG_OK : sffg_env_end(env);
+}
+
 static int check_edges_impl(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist, int rot_mode,
                             uint8_t *free_out, int32_t *first_hit_out, bool async) {
-  if (!env || m < 0 || (m > 0 && (!starts || !ends || !free_out)) || !(sample_dist > 0) ||
-      (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
-    return fail(SFFG_ERR_ARG, "sffg_check_edges: bad arguments");
-  if (m == 0) return SFFG_OK;
+  int rc = check_segment_args(env, starts, ends, m, sample_dist, rot_mode, free_out, "sffg_check_edges");
+  if (rc != SFFG_OK || m == 0) return rc;
+  if ((rc = env_enter_host(env)) != SFFG_OK) return rc;
   unsigned *base;
-  {
-    const int rc0 = env_enter_host(env);
-    if (rc0 != SFFG_OK) return rc0;
-  }
-  if ((size_t)m * 96 <= kSmallIn && (size_t)m * 5 <= kSmallBytes - kSmallIn) {
-    // planner-sized call.  The endpoints are re-read by every warp that shares an edge, so they go to device memory with
-    // one DMA from the pinned staging area; the results are written straight into pinned mapped memory.
-    cudaStream_t st = env->streams[0];
-    int rc = env->in[0].reserve((size_t)m * 96);
-    if (rc == SFFG_OK) rc = env->fh.reserve((size_t)m * sizeof(int));
-    if (rc != SFFG_OK) return rc;
-    std::memcpy(env->h_small, starts, (size_t)m * 48);
-    std::memcpy(env->h_small + (size_t)m * 48, ends, (size_t)m * 48);
-    double *ds = (double *)env->in[0].p, *de = ds + 6 * m;
-    SFFG_CUDA(cudaMemcpyAsync(ds, env->h_small, (size_t)m * 96, cudaMemcpyHostToDevice, st));
-    int32_t *h_first = reinterpret_cast<int32_t *>(env->h_small + kSmallIn);
-    uint8_t *h_free = env->h_small + kSmallIn + (size_t)m * 4;
+  if ((size_t)m * 96 <= EnvStaging::kInBytes && (size_t)m * 5 <= EnvStaging::kOutBytes) {
+    // planner-sized call: the results are written straight into pinned mapped memory
+    const EnvStaging h = env->staging();
+    double *ds, *de;
+    if ((rc = stage_segments(env, starts, ends, m, &ds, &de)) != SFFG_OK) return rc;
     EnvDev v = env_view(env, &base);
-    SFFG_CUDA(launch_check_edges(v, ds, de, m, sample_dist, rot_mode, h_free, h_first, st, env->cfg, env->count, base,
-                                 (int *)env->fh.p));
-    env->pend.kind = 1;
-    env->pend.m = m;
-    env->pend.out = free_out;
-    env->pend.first_out = first_hit_out;
-    if (async) return env_leave(env, st);   // *_device launches issued before the end call are ordered behind this one
-    return sffg_env_end(env);
+    SFFG_CUDA(launch_check_edges(v, ds, de, m, sample_dist, rot_mode, h.edge_free(m), h.edge_first_hit(), env->streams[0].get(),
+                                 env->cfg, env->count, base, (int *)env->fh.p));
+    return env_commit(env, sffg_env::Pending{1, m, free_out, first_hit_out}, async);
   }
   const int64_t chunk = 1 << 18;
   int s = 0;
   for (int64_t off = 0; off < m; off += chunk, s ^= 1) {
     const int64_t cnt = std::min(chunk, m - off);
-    cudaStream_t st = env->streams[s];
+    cudaStream_t st = env->streams[s].get();
     SFFG_CUDA(cudaStreamSynchronize(st));
-    int rc = env->in[s].reserve((size_t)cnt * 96);
+    rc = env->in[s].reserve((size_t)cnt * 96);
     if (rc == SFFG_OK) rc = env->out[s].reserve((size_t)cnt);
     if (rc == SFFG_OK) rc = env->aux[s].reserve((size_t)cnt * 4);
     if (rc != SFFG_OK) return rc;
@@ -977,8 +1038,7 @@ static int check_edges_impl(sffg_env *env, const double *starts, const double *e
     if (first_hit_out)
       SFFG_CUDA(cudaMemcpyAsync(first_hit_out + off, env->aux[s].p, (size_t)cnt * 4, cudaMemcpyDeviceToHost, st));
   }
-  SFFG_CUDA(cudaStreamSynchronize(env->streams[0]));
-  SFFG_CUDA(cudaStreamSynchronize(env->streams[1]));
+  for (const Stream &st : env->streams) SFFG_CUDA(cudaStreamSynchronize(st.get()));
   return check_status(env);
 }
 
@@ -994,41 +1054,26 @@ int sffg_check_moves_begin(sffg_env *env, const double *starts, const double *en
 }
 static int check_moves_impl(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist, int rot_mode,
                             uint8_t *ok_out, bool async) {
-  if (!env || m < 0 || (m > 0 && (!starts || !ends || !ok_out)) || !(sample_dist > 0) ||
-      (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
-    return fail(SFFG_ERR_ARG, "sffg_check_moves: bad arguments");
-  if (m == 0) return SFFG_OK;
-  unsigned *base;
-  {
-    const int rc0 = env_enter_host(env);
-    if (rc0 != SFFG_OK) return rc0;
-  }
-  if ((size_t)m * 96 <= kSmallIn && (size_t)m * 6 <= kSmallBytes - kSmallIn) {
+  int rc = check_segment_args(env, starts, ends, m, sample_dist, rot_mode, ok_out, "sffg_check_moves");
+  if (rc != SFFG_OK || m == 0) return rc;
+  if ((rc = env_enter_host(env)) != SFFG_OK) return rc;
+  if ((size_t)m * 96 <= EnvStaging::kInBytes && (size_t)m * 6 <= EnvStaging::kOutBytes) {
     // planner-sized call: one upload, the pose kernel on the end points and the edge kernel on the segments back to back
     // on one stream, results straight into pinned mapped memory, one synchronisation
-    cudaStream_t st = env->streams[0];
-    int rc = env->in[0].reserve((size_t)m * 96);
-    if (rc == SFFG_OK) rc = env->fh.reserve((size_t)m * sizeof(int));
-    if (rc != SFFG_OK) return rc;
-    std::memcpy(env->h_small, starts, (size_t)m * 48);
-    std::memcpy(env->h_small + (size_t)m * 48, ends, (size_t)m * 48);
-    double *ds = (double *)env->in[0].p, *de = ds + 6 * m;
-    SFFG_CUDA(cudaMemcpyAsync(ds, env->h_small, (size_t)m * 96, cudaMemcpyHostToDevice, st));
-    uint8_t *h_free = env->h_small + kSmallIn, *h_hit = h_free + (size_t)m;
+    cudaStream_t st = env->streams[0].get();
+    const EnvStaging h = env->staging();
+    double *ds, *de;
+    if ((rc = stage_segments(env, starts, ends, m, &ds, &de)) != SFFG_OK) return rc;
+    unsigned *base;
     EnvDev v = env_view(env, &base);
-    SFFG_CUDA(launch_collide_poses(v, de, 1, m, h_hit, st, env->cfg, env->count, base));
+    SFFG_CUDA(launch_collide_poses(v, de, 1, m, h.move_hit(m), st, env->cfg, env->count, base));
     EnvDev w = env_view(env, &base);
-    SFFG_CUDA(launch_check_edges(w, ds, de, m, sample_dist, rot_mode, h_free, nullptr, st, env->cfg, env->count, base,
+    SFFG_CUDA(launch_check_edges(w, ds, de, m, sample_dist, rot_mode, h.move_free(), nullptr, st, env->cfg, env->count, base,
                                  (int *)env->fh.p));
-    env->pend.kind = 2;
-    env->pend.m = m;
-    env->pend.out = ok_out;
-    env->pend.first_out = nullptr;
-    if (async) return env_leave(env, st);
-    return sffg_env_end(env);
+    return env_commit(env, sffg_env::Pending{2, m, ok_out, nullptr}, async);
   }
   std::vector<uint8_t> hit((size_t)m);
-  int rc = sffg_collide_poses_f64(env, ends, m, hit.data());
+  rc = sffg_collide_poses_f64(env, ends, m, hit.data());
   if (rc == SFFG_OK) rc = sffg_check_edges(env, starts, ends, m, sample_dist, rot_mode, ok_out, nullptr);
   if (rc != SFFG_OK) return rc;
   for (int64_t i = 0; i < m; ++i) ok_out[i] = (uint8_t)(ok_out[i] && !hit[(size_t)i]);
@@ -1049,53 +1094,28 @@ int sffg_index_create(int dim, sffg_index **out) {
   if (!out || (dim != 2 && dim != 6)) return fail(SFFG_ERR_ARG, "sffg_index_create: dim must be 2 or 6");
   int rc = ensure_runtime();
   if (rc != SFFG_OK) return rc;
-  sffg_index *idx = new sffg_index();
+  std::unique_ptr<sffg_index, int (*)(sffg_index *)> idx(new sffg_index(), sffg_index_destroy);   // released on every error return
   idx->dim = dim;
   const char *pr = std::getenv("SFFG_KNN_PRUNING");
   idx->pruning = !(pr && pr[0] == '0');
-  cudaError_t e = cudaStreamCreateWithFlags(&idx->stream, cudaStreamNonBlocking);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&idx->ev, cudaEventDisableTiming);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&idx->add_ev, cudaEventDisableTiming);
-  if (e == cudaSuccess) e = cudaMalloc((void **)&idx->d_total, sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaHostAlloc((void **)&idx->h_small, kSmallBytes, cudaHostAllocMapped);
-  if (e == cudaSuccess) {   // storage exists from the start: the scan kernels may touch the first block of an empty index
-    idx->cap = 4096 + 128;
-    e = cudaMalloc((void **)&idx->d_coords, (size_t)idx->cap * dim * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemset(idx->d_coords, 0, (size_t)idx->cap * dim * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&idx->d_amax, 256);
-    if (e == cudaSuccess) e = cudaMemset(idx->d_amax, 0, 256);
-  }
-  if (e != cudaSuccess) {
-    cudaFree(idx->d_coords);
-    cudaFree(idx->d_amax);
-    if (idx->stream) cudaStreamDestroy(idx->stream);
-    if (idx->ev) cudaEventDestroy(idx->ev);
-  if (idx->add_ev) cudaEventDestroy(idx->add_ev);
-  if (idx->d_total) cudaFree(idx->d_total);
-    if (idx->add_ev) cudaEventDestroy(idx->add_ev);
-  if (idx->d_total) cudaFree(idx->d_total);
-    if (idx->d_total) cudaFree(idx->d_total);
-    if (idx->h_small) cudaFreeHost(idx->h_small);
-    delete idx;
-    return fail(SFFG_ERR_CUDA, cudaGetErrorString(e));
-  }
-  *out = idx;
+  SFFG_CUDA(make_stream(idx->stream));
+  SFFG_CUDA(make_event(idx->ev));
+  SFFG_CUDA(make_event(idx->add_ev));
+  SFFG_CUDA(dev_alloc(idx->d_total, sizeof(unsigned long long)));
+  SFFG_CUDA(host_alloc(idx->h_small, kSmallBytes));
+  // storage exists from the start: the scan kernels may touch the first block of an empty index
+  idx->cap = 4096 + 128;
+  SFFG_CUDA(dev_alloc(idx->d_coords, (size_t)idx->cap * dim * sizeof(float)));
+  SFFG_CUDA(cudaMemset(idx->d_coords.get(), 0, (size_t)idx->cap * dim * sizeof(float)));
+  SFFG_CUDA(dev_alloc(idx->d_amax, 256));
+  SFFG_CUDA(cudaMemset(idx->d_amax.get(), 0, 256));
+  *out = idx.release();
   return SFFG_OK;
 }
 
 int sffg_index_destroy(sffg_index *idx) {
   if (!idx) return SFFG_OK;
-  if (idx->stream) cudaStreamSynchronize(idx->stream);
-  cudaFree(idx->d_coords);
-  cudaFree(idx->d_amax);
-  DevBuf *bufs[] = {&idx->q, &idx->ids, &idx->d2, &idx->scratch, &idx->counts, &idx->offsets, &idx->cursor, &idx->keys, &idx->stage,
-                    &idx->s_coords, &idx->s_ids, &idx->s_bb, &idx->s_keys, &idx->s_vals, &idx->s_temp, &idx->s_bounds};
-  for (DevBuf *b : bufs) b->release();
-  if (idx->h_small) cudaFreeHost(idx->h_small);
-  if (idx->ev) cudaEventDestroy(idx->ev);
-  if (idx->add_ev) cudaEventDestroy(idx->add_ev);
-  if (idx->d_total) cudaFree(idx->d_total);
-  if (idx->stream) cudaStreamDestroy(idx->stream);
+  if (idx->stream) cudaStreamSynchronize(idx->stream.get());
   delete idx;
   return SFFG_OK;
 }
@@ -1106,14 +1126,13 @@ static int index_grow(sffg_index *idx, int64_t need, cudaStream_t st) {
   if (need + 128 <= idx->cap) return SFFG_OK;
   int64_t ncap = std::max<int64_t>({need, idx->cap * 2, 4096});
   ncap = (ncap + 31) / 32 * 32 + 128;   // spare blocks: the scan kernels prefetch up to 3 blocks past the end of a slice
-  float *nc = nullptr;
-  SFFG_CUDA(cudaMalloc((void **)&nc, (size_t)ncap * idx->dim * sizeof(float)));
+  DevPtr<float> nc;
+  SFFG_CUDA(dev_alloc(nc, (size_t)ncap * idx->dim * sizeof(float)));
   for (int c = 0; c < idx->dim && idx->n > 0; ++c)
-    SFFG_CUDA(cudaMemcpyAsync(nc + (size_t)c * ncap, idx->d_coords + (size_t)c * idx->cap, (size_t)idx->n * sizeof(float),
+    SFFG_CUDA(cudaMemcpyAsync(nc.get() + (size_t)c * ncap, idx->d_coords.get() + (size_t)c * idx->cap, (size_t)idx->n * sizeof(float),
                               cudaMemcpyDeviceToDevice, st));
   SFFG_CUDA(cudaStreamSynchronize(st));
-  cudaFree(idx->d_coords);
-  idx->d_coords = nc;
+  idx->d_coords = std::move(nc);
   idx->cap = ncap;
   return SFFG_OK;
 }
@@ -1124,7 +1143,7 @@ int sffg_index_add_device(sffg_index *idx, const float *d_pts, int64_t n, void *
   cudaStream_t st = (cudaStream_t)stream;
   int rc = index_grow(idx, idx->n + n, st);
   if (rc != SFFG_OK) return rc;
-  SFFG_CUDA(launch_index_append(idx->d_coords, idx->cap, idx->dim, idx->n, d_pts, n, idx->d_amax, st));
+  SFFG_CUDA(launch_index_append(idx->d_coords.get(), idx->cap, idx->dim, idx->n, d_pts, n, idx->d_amax.get(), st));
   idx->n += n;
   return SFFG_OK;
 }
@@ -1136,10 +1155,10 @@ int sffg_index_add(sffg_index *idx, const float *pts, int64_t n) {
   if (rc != SFFG_OK) return rc;
   rc = idx->stage.reserve((size_t)n * idx->dim * sizeof(float));
   if (rc != SFFG_OK) return rc;
-  SFFG_CUDA(cudaMemcpyAsync(idx->stage.p, pts, (size_t)n * idx->dim * sizeof(float), cudaMemcpyHostToDevice, idx->stream));
-  rc = sffg_index_add_device(idx, (const float *)idx->stage.p, n, idx->stream);
+  SFFG_CUDA(cudaMemcpyAsync(idx->stage.p, pts, (size_t)n * idx->dim * sizeof(float), cudaMemcpyHostToDevice, idx->stream.get()));
+  rc = sffg_index_add_device(idx, (const float *)idx->stage.p, n, idx->stream.get());
   if (rc != SFFG_OK) return rc;
-  SFFG_CUDA(cudaStreamSynchronize(idx->stream));
+  SFFG_CUDA(cudaStreamSynchronize(idx->stream.get()));
   return SFFG_OK;
 }
 
@@ -1157,16 +1176,12 @@ int sffg_index_add_multi_begin(sffg_index *const *idx, const int64_t *n_per, int
   sffg_index *lead = idx[0];   // one staging buffer, one upload, one synchronisation for all indices
   for (int i = 0; i < n_idx; ++i)
     if ((rc = index_busy(idx[i], "sffg_index_add_multi")) != SFFG_OK) return rc;
-  cudaStream_t st = lead->stream;
+  cudaStream_t st = lead->stream.get();
   const size_t bytes = (size_t)total * dim * sizeof(float);
   rc = lead->stage.reserve(bytes);
   if (rc != SFFG_OK) return rc;
-  if (bytes <= kSmallBytes) {
-    std::memcpy(lead->h_small, pts, bytes);
-    SFFG_CUDA(cudaMemcpyAsync(lead->stage.p, lead->h_small, bytes, cudaMemcpyHostToDevice, st));
-  } else {
-    SFFG_CUDA(cudaMemcpyAsync(lead->stage.p, pts, bytes, cudaMemcpyHostToDevice, st));
-  }
+  // (small batches: the whole staging area holds the rows)
+  SFFG_CUDA(upload_async(lead->stage.p, pts, bytes, bytes <= kSmallBytes ? lead->h_small.get() : nullptr, st));
   int64_t off = 0;
   for (int i = 0; i < n_idx; ++i) {
     if (n_per[i] == 0) continue;
@@ -1175,11 +1190,12 @@ int sffg_index_add_multi_begin(sffg_index *const *idx, const int64_t *n_per, int
     off += n_per[i];
   }
   // the appends ran on the lead's stream: later work on the other indices' own streams is ordered behind them
-  SFFG_CUDA(cudaEventRecord(lead->add_ev, st));
+  SFFG_CUDA(cudaEventRecord(lead->add_ev.get(), st));
   for (int i = 0; i < n_idx; ++i)
-    if (idx[i] != lead && n_per[i] > 0) SFFG_CUDA(cudaStreamWaitEvent(idx[i]->stream, lead->add_ev, 0));
-  lead->pend = sffg_index::Pending{};
-  lead->pend.kind = 3;   // (the staging area of the lead is in use until sffg_index_end)
+    if (idx[i] != lead && n_per[i] > 0) SFFG_CUDA(cudaStreamWaitEvent(idx[i]->stream.get(), lead->add_ev.get(), 0));
+  sffg_index::Pending p{};
+  p.kind = 3;   // (the staging area of the lead is in use until sffg_index_end)
+  lead->pend = p;
   return SFFG_OK;
 }
 
@@ -1187,6 +1203,26 @@ int sffg_index_add_multi(sffg_index *const *idx, const int64_t *n_per, int n_idx
   const int rc = sffg_index_add_multi_begin(idx, n_per, n_idx, pts);
   if (rc != SFFG_OK) return rc;
   return idx[0]->pend.kind == 3 ? sffg_index_end(idx[0]) : SFFG_OK;
+}
+
+static IndexDev index_view(const sffg_index *idx) {
+  return IndexDev{idx->d_coords.get(), idx->cap, idx->n, idx->dim, idx->d_amax.get()};
+}
+
+static SortedDev sorted_view(const sffg_index *idx) {
+  SortedDev sv;
+  sv.coords = (const float *)idx->s_coords.p;
+  sv.ids = (const int *)idx->s_ids.p;
+  sv.bb = (const float *)idx->s_bb.p;
+  sv.cap_s = idx->s_cap;
+  sv.nblk_cap = idx->s_nblk_cap;
+  sv.nsb_cap = idx->s_nblk_cap / 32 + 2;
+  sv.sbb = sv.bb + (size_t)idx->s_nblk_cap * 2 * (idx->dim == 6 ? 3 : 2);
+  sv.n_sorted = (int)idx->n_sorted;
+  sv.nblk = (int)((idx->n_sorted + 31) / 32);
+  sv.amax = idx->d_amax.get();
+  sv.bounds = (const int *)idx->s_bounds.p;
+  return sv;
 }
 
 constexpr int64_t kSortMinNodes = 8192;   // below this the exhaustive scan is already latency-bound
@@ -1231,30 +1267,14 @@ static int ensure_sorted(sffg_index *idx, cudaStream_t st) {
   b.nblk_cap = idx->s_nblk_cap;
   b.nsb_cap = idx->s_nblk_cap / 32 + 2;
   b.sbb = b.bb + (size_t)idx->s_nblk_cap * 2 * lin;
-  IndexDev v{idx->d_coords, idx->cap, idx->n, idx->dim, idx->d_amax};
+  const IndexDev v = index_view(idx);
   SFFG_CUDA(launch_sorted_build(v, n, b, st));
   idx->n_sorted = n;
   return SFFG_OK;
 }
 
-static SortedDev sorted_view(const sffg_index *idx) {
-  SortedDev sv;
-  sv.coords = (const float *)idx->s_coords.p;
-  sv.ids = (const int *)idx->s_ids.p;
-  sv.bb = (const float *)idx->s_bb.p;
-  sv.cap_s = idx->s_cap;
-  sv.nblk_cap = idx->s_nblk_cap;
-  sv.nsb_cap = idx->s_nblk_cap / 32 + 2;
-  sv.sbb = sv.bb + (size_t)idx->s_nblk_cap * 2 * (idx->dim == 6 ? 3 : 2);
-  sv.n_sorted = (int)idx->n_sorted;
-  sv.nblk = (int)((idx->n_sorted + 31) / 32);
-  sv.amax = idx->d_amax;
-  sv.bounds = (const int *)idx->s_bounds.p;
-  return sv;
-}
-
 static int knn_rows_device(sffg_index *idx, const float *d_queries, int64_t nq, int k, const RowDests &out, cudaStream_t st) {
-  IndexDev v{idx->d_coords, idx->cap, idx->n, idx->dim, idx->d_amax};
+  const IndexDev v = index_view(idx);
   int rc = ensure_sorted(idx, st);
   if (rc != SFFG_OK) return rc;
   if (idx->n_sorted > 0) {
@@ -1303,14 +1323,15 @@ int sffg_knn(sffg_index *idx, const float *queries, int64_t nq, int k, int32_t *
   int rc = index_busy(idx, "sffg_knn");
   if (rc != SFFG_OK) return rc;
   const size_t qbytes = (size_t)nq * idx->dim * 4, obytes = (size_t)nq * k * 4;
-  if (qbytes <= (64 << 10) && 2 * obytes <= kSmallBytes - (64 << 10)) {
+  if (qbytes <= IndexStaging::kQueryBytes && 2 * obytes <= IndexStaging::kKnnOutBytes) {
     // planner-sized call: queries and results live in pinned mapped memory, one synchronisation
-    std::memcpy(idx->h_small, queries, qbytes);
-    int32_t *h_ids = reinterpret_cast<int32_t *>(idx->h_small + (64 << 10));
-    float *h_d2 = reinterpret_cast<float *>(idx->h_small + (64 << 10) + obytes);
-    rc = sffg_knn_device(idx, reinterpret_cast<const float *>(idx->h_small), nq, k, h_ids, h_d2, idx->stream);
+    const IndexStaging h = idx->staging();
+    std::memcpy(h.queries(), queries, qbytes);
+    int32_t *h_ids = h.knn_ids();
+    float *h_d2 = h.knn_d2(obytes);
+    rc = sffg_knn_device(idx, reinterpret_cast<const float *>(h.queries()), nq, k, h_ids, h_d2, idx->stream.get());
     if (rc != SFFG_OK) return rc;
-    SFFG_CUDA(cudaStreamSynchronize(idx->stream));
+    SFFG_CUDA(cudaStreamSynchronize(idx->stream.get()));
     std::memcpy(ids_out, h_ids, obytes);
     std::memcpy(d2_out, h_d2, obytes);
     return SFFG_OK;
@@ -1322,12 +1343,12 @@ int sffg_knn(sffg_index *idx, const float *queries, int64_t nq, int k, int32_t *
     if (rc == SFFG_OK) rc = idx->ids.reserve((size_t)cnt * k * 4);
     if (rc == SFFG_OK) rc = idx->d2.reserve((size_t)cnt * k * 4);
     if (rc != SFFG_OK) return rc;
-    SFFG_CUDA(cudaMemcpyAsync(idx->q.p, queries + off * idx->dim, (size_t)cnt * idx->dim * 4, cudaMemcpyHostToDevice, idx->stream));
-    rc = sffg_knn_device(idx, (const float *)idx->q.p, cnt, k, (int32_t *)idx->ids.p, (float *)idx->d2.p, idx->stream);
+    SFFG_CUDA(cudaMemcpyAsync(idx->q.p, queries + off * idx->dim, (size_t)cnt * idx->dim * 4, cudaMemcpyHostToDevice, idx->stream.get()));
+    rc = sffg_knn_device(idx, (const float *)idx->q.p, cnt, k, (int32_t *)idx->ids.p, (float *)idx->d2.p, idx->stream.get());
     if (rc != SFFG_OK) return rc;
-    SFFG_CUDA(cudaMemcpyAsync(ids_out + off * k, idx->ids.p, (size_t)cnt * k * 4, cudaMemcpyDeviceToHost, idx->stream));
-    SFFG_CUDA(cudaMemcpyAsync(d2_out + off * k, idx->d2.p, (size_t)cnt * k * 4, cudaMemcpyDeviceToHost, idx->stream));
-    SFFG_CUDA(cudaStreamSynchronize(idx->stream));
+    SFFG_CUDA(cudaMemcpyAsync(ids_out + off * k, idx->ids.p, (size_t)cnt * k * 4, cudaMemcpyDeviceToHost, idx->stream.get()));
+    SFFG_CUDA(cudaMemcpyAsync(d2_out + off * k, idx->d2.p, (size_t)cnt * k * 4, cudaMemcpyDeviceToHost, idx->stream.get()));
+    SFFG_CUDA(cudaStreamSynchronize(idx->stream.get()));
   }
   return SFFG_OK;
 }
@@ -1347,48 +1368,44 @@ int sffg_knn_multi_begin(sffg_index *const *idx, const int64_t *nq_per, int n_id
   sffg_index *lead = idx[0];   // its stream and staging carry the whole call
   for (int i = 0; i < n_idx; ++i)
     if ((rc = index_busy(idx[i], "sffg_knn_multi")) != SFFG_OK) return rc;
-  cudaStream_t st = lead->stream;
+  cudaStream_t st = lead->stream.get();
   const size_t qbytes = (size_t)total * dim * 4, obytes = (size_t)total * k * 4;
-  const bool small = qbytes <= (64 << 10) && 2 * obytes <= kSmallBytes - (64 << 10);
+  const bool small = qbytes <= IndexStaging::kQueryBytes && 2 * obytes <= IndexStaging::kKnnOutBytes;
+  const IndexStaging h = lead->staging();
   rc = lead->q.reserve(qbytes);
   if (rc == SFFG_OK) rc = lead->ids.reserve(obytes);
   if (rc == SFFG_OK) rc = lead->d2.reserve(obytes);
   if (rc != SFFG_OK) return rc;
-  if (small) {
-    std::memcpy(lead->h_small, queries, qbytes);
-    SFFG_CUDA(cudaMemcpyAsync(lead->q.p, lead->h_small, qbytes, cudaMemcpyHostToDevice, st));
-  } else {
-    SFFG_CUDA(cudaMemcpyAsync(lead->q.p, queries, qbytes, cudaMemcpyHostToDevice, st));
-  }
+  SFFG_CUDA(upload_async(lead->q.p, queries, qbytes, small ? h.queries() : nullptr, st));
   // fork: every index searches on its own stream once the queries have arrived; join: the lead stream waits for all
-  SFFG_CUDA(cudaEventRecord(lead->ev, st));
+  SFFG_CUDA(cudaEventRecord(lead->ev.get(), st));
   int64_t off = 0;
   for (int i = 0; i < n_idx; ++i) {
     if (nq_per[i] == 0) continue;
-    cudaStream_t si = idx[i] == lead ? st : idx[i]->stream;
-    if (si != st) SFFG_CUDA(cudaStreamWaitEvent(si, lead->ev, 0));
+    cudaStream_t si = idx[i] == lead ? st : idx[i]->stream.get();
+    if (si != st) SFFG_CUDA(cudaStreamWaitEvent(si, lead->ev.get(), 0));
     rc = sffg_knn_device(idx[i], (const float *)lead->q.p + off * dim, nq_per[i], k, (int32_t *)lead->ids.p + off * k,
                          (float *)lead->d2.p + off * k, si);
     if (rc != SFFG_OK) return rc;
     if (si != st) {
-      SFFG_CUDA(cudaEventRecord(idx[i]->ev, si));
-      SFFG_CUDA(cudaStreamWaitEvent(st, idx[i]->ev, 0));
+      SFFG_CUDA(cudaEventRecord(idx[i]->ev.get(), si));
+      SFFG_CUDA(cudaStreamWaitEvent(st, idx[i]->ev.get(), 0));
     }
     off += nq_per[i];
   }
-  lead->pend = sffg_index::Pending{};
-  lead->pend.kind = 1;
+  sffg_index::Pending p{};
+  p.kind = 1;
   if (small) {
-    unsigned char *ho = lead->h_small + (64 << 10);
-    SFFG_CUDA(cudaMemcpyAsync(ho, lead->ids.p, obytes, cudaMemcpyDeviceToHost, st));
-    SFFG_CUDA(cudaMemcpyAsync(ho + obytes, lead->d2.p, obytes, cudaMemcpyDeviceToHost, st));
-    lead->pend.copy[0] = {ids_out, ho, obytes};
-    lead->pend.copy[1] = {d2_out, ho + obytes, obytes};
-    lead->pend.n_copy = 2;
+    SFFG_CUDA(cudaMemcpyAsync(h.knn_ids(), lead->ids.p, obytes, cudaMemcpyDeviceToHost, st));
+    SFFG_CUDA(cudaMemcpyAsync(h.knn_d2(obytes), lead->d2.p, obytes, cudaMemcpyDeviceToHost, st));
+    p.copy[0] = {ids_out, h.knn_ids(), obytes};
+    p.copy[1] = {d2_out, h.knn_d2(obytes), obytes};
+    p.n_copy = 2;
   } else {
     SFFG_CUDA(cudaMemcpyAsync(ids_out, lead->ids.p, obytes, cudaMemcpyDeviceToHost, st));
     SFFG_CUDA(cudaMemcpyAsync(d2_out, lead->d2.p, obytes, cudaMemcpyDeviceToHost, st));
   }
+  lead->pend = p;
   return SFFG_OK;
 }
 
@@ -1399,54 +1416,51 @@ int sffg_knn_multi(sffg_index *const *idx, const int64_t *nq_per, int n_idx, con
   return idx[0]->pend.kind == 1 ? sffg_index_end(idx[0]) : SFFG_OK;
 }
 
+// fill and per-row sort of a radius call once idx->offsets holds the row offsets: the sorted rows go to ids_dst / d2_dst
+static int radius_fill_sort(sffg_index *idx, bool pruned, int64_t nq, float r2, int32_t *ids_dst, float *d2_dst) {
+  cudaStream_t st = idx->stream.get();
+  const IndexDev v = index_view(idx);
+  const float *q = (const float *)idx->q.p;
+  const int64_t *offs = (const int64_t *)idx->offsets.p;
+  int32_t *cursor = (int32_t *)idx->cursor.p;
+  unsigned long long *keys = (unsigned long long *)idx->keys.p;
+  SFFG_CUDA(cudaMemsetAsync(cursor, 0, (size_t)nq * 4, st));
+  if (pruned) SFFG_CUDA(launch_radius_fill_pruned(v, sorted_view(idx), q, nq, r2, offs, cursor, keys, g_rt.sm_count, st));
+  else SFFG_CUDA(launch_radius_fill(v, q, nq, r2, offs, cursor, keys, plan_knn(nq, idx->n, g_rt.sm_count), st));
+  SFFG_CUDA(launch_radius_sort(keys, offs, (const int32_t *)idx->counts.p, nq, ids_dst, d2_dst, st));
+  return SFFG_OK;
+}
+
 // second half of a radius call once the counts are on the host: exclusive scan, fill, per-row sort, download
 static int radius_fill_from_host_counts(sffg_index *idx, const sffg_index::Pending &c, int64_t total) {
-  int rc;
-  cudaStream_t st = idx->stream;
-  IndexDev v{idx->d_coords, idx->cap, idx->n, idx->dim, idx->d_amax};
-  const KnnPlan plan = plan_knn(c.nq, idx->n, g_rt.sm_count);
-  const SortedDev sv = sorted_view(idx);
+  cudaStream_t st = idx->stream.get();
+  const IndexStaging h = idx->staging();
   const size_t cbytes = (size_t)c.nq * 4;
-  unsigned char *hq = idx->h_small, *hr = idx->h_small + (128 << 10);
-  const size_t hr_bytes = kSmallBytes - (128 << 10);
   std::vector<int64_t> offs((size_t)c.nq);
   int64_t run = 0;
   for (int64_t i = 0; i < c.nq; ++i) {
     offs[(size_t)i] = run;
     run += c.counts_out[i];
   }
-  rc = idx->offsets.reserve((size_t)c.nq * 8);
+  int rc = idx->offsets.reserve((size_t)c.nq * 8);
   if (rc == SFFG_OK) rc = idx->cursor.reserve(cbytes);
   if (rc == SFFG_OK) rc = idx->keys.reserve((size_t)total * 8);
   if (rc == SFFG_OK) rc = idx->ids.reserve((size_t)total * 4);
   if (rc == SFFG_OK) rc = idx->d2.reserve((size_t)total * 4);
   if (rc != SFFG_OK) return rc;
-  const bool small_out = c.small && (size_t)c.nq * 8 <= (64 << 10) && (size_t)total * 8 <= hr_bytes;
+  // two-sync staging: the row offsets in the query part (free again), the rows without a head
+  const bool small_out = c.small && (size_t)c.nq * 8 <= IndexStaging::kQueryBytes && (size_t)total * 8 <= IndexStaging::kRowsBytes;
+  SFFG_CUDA(upload_async(idx->offsets.p, offs.data(), (size_t)c.nq * 8, small_out ? h.queries() : nullptr, st));
+  rc = radius_fill_sort(idx, c.pruned, c.nq, c.r2, (int32_t *)idx->ids.p, (float *)idx->d2.p);
+  if (rc != SFFG_OK) return rc;
+  int32_t *ids_dst = small_out ? h.rows_ids(0) : c.ids_out;
+  float *d2_dst = small_out ? h.rows_d2(0, total) : c.d2_out;
+  SFFG_CUDA(cudaMemcpyAsync(ids_dst, idx->ids.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+  SFFG_CUDA(cudaMemcpyAsync(d2_dst, idx->d2.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+  SFFG_CUDA(cudaStreamSynchronize(st));
   if (small_out) {
-    std::memcpy(hq, offs.data(), (size_t)c.nq * 8);   // the query staging area is free again
-    SFFG_CUDA(cudaMemcpyAsync(idx->offsets.p, hq, (size_t)c.nq * 8, cudaMemcpyHostToDevice, st));
-  } else {
-    SFFG_CUDA(cudaMemcpyAsync(idx->offsets.p, offs.data(), (size_t)c.nq * 8, cudaMemcpyHostToDevice, st));
-  }
-  SFFG_CUDA(cudaMemsetAsync(idx->cursor.p, 0, cbytes, st));
-  if (c.pruned)
-    SFFG_CUDA(launch_radius_fill_pruned(v, sv, (const float *)idx->q.p, c.nq, c.r2, (const int64_t *)idx->offsets.p, (int32_t *)idx->cursor.p,
-                                        (unsigned long long *)idx->keys.p, g_rt.sm_count, st));
-  else
-    SFFG_CUDA(launch_radius_fill(v, (const float *)idx->q.p, c.nq, c.r2, (const int64_t *)idx->offsets.p, (int32_t *)idx->cursor.p,
-                                 (unsigned long long *)idx->keys.p, plan, st));
-  SFFG_CUDA(launch_radius_sort((unsigned long long *)idx->keys.p, (const int64_t *)idx->offsets.p, (const int32_t *)idx->counts.p,
-                               c.nq, (int32_t *)idx->ids.p, (float *)idx->d2.p, st));
-  if (small_out) {
-    SFFG_CUDA(cudaMemcpyAsync(hr, idx->ids.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
-    SFFG_CUDA(cudaMemcpyAsync(hr + (size_t)total * 4, idx->d2.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
-    SFFG_CUDA(cudaStreamSynchronize(st));
-    std::memcpy(c.ids_out, hr, (size_t)total * 4);
-    std::memcpy(c.d2_out, hr + (size_t)total * 4, (size_t)total * 4);
-  } else {
-    SFFG_CUDA(cudaMemcpyAsync(c.ids_out, idx->ids.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
-    SFFG_CUDA(cudaMemcpyAsync(c.d2_out, idx->d2.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
-    SFFG_CUDA(cudaStreamSynchronize(st));
+    std::memcpy(c.ids_out, ids_dst, (size_t)total * 4);
+    std::memcpy(c.d2_out, d2_dst, (size_t)total * 4);
   }
   return SFFG_OK;
 }
@@ -1461,105 +1475,69 @@ static int radius_begin_impl(sffg_index *idx, const float *queries, int64_t nq, 
   if (nq == 0) return SFFG_OK;
   int rc = index_busy(idx, "sffg_radius");
   if (rc != SFFG_OK) return rc;
-  cudaStream_t st = idx->stream;
-  IndexDev v{idx->d_coords, idx->cap, idx->n, idx->dim, idx->d_amax};
-  KnnPlan plan = plan_knn(nq, idx->n, g_rt.sm_count);
+  cudaStream_t st = idx->stream.get();
+  const IndexDev v = index_view(idx);
+  const IndexStaging h = idx->staging();
   const size_t qbytes = (size_t)nq * idx->dim * 4, cbytes = (size_t)nq * 4;
   // planner-sized calls stage through pinned memory so that every copy is an asynchronous DMA
-  const bool small = qbytes <= (64 << 10) && cbytes <= (64 << 10);
-  unsigned char *hq = idx->h_small, *hc = idx->h_small + (64 << 10), *hr = idx->h_small + (128 << 10);
-  const size_t hr_bytes = kSmallBytes - (128 << 10);
-  if (allow_fused && small && ids_out && capacity > 0 && idx->n <= kFusedRadiusMaxNodes && qbytes <= (64 << 10) - 16 &&
-      (size_t)nq * 8 + 64 <= hr_bytes / 2) {
-    // planner-sized search on a small index: ONE kernel (block per query) that reads the queries from and writes counts,
-    // row offsets and sorted rows to pinned mapped memory -- one stream operation besides zeroing the row allocator, one
-    // host synchronisation.  Staging: [queries | flag] [counts] [row offsets | ids | d2].
-    std::memcpy(hq, queries, qbytes);
-    int *h_flag = reinterpret_cast<int *>(hq + (64 << 10) - 16);
-    *h_flag = 0;
-    int64_t *h_rowoff = reinterpret_cast<int64_t *>(hr);
-    const int64_t cap1 = (int64_t)((hr_bytes - (size_t)nq * 8) / 8);
-    int32_t *h_ids = reinterpret_cast<int32_t *>(hr + (size_t)nq * 8);
-    float *h_d2 = reinterpret_cast<float *>(hr + (size_t)nq * 8 + (size_t)cap1 * 4);
-    SFFG_CUDA(cudaMemsetAsync(idx->d_total, 0, sizeof(unsigned long long), st));
-    SFFG_CUDA(launch_radius_fused(v, reinterpret_cast<const float *>(hq), nq, r2, cap1, reinterpret_cast<int32_t *>(hc), h_rowoff, h_ids,
-                                  h_d2, idx->d_total, h_flag, st));
-    sffg_index::Pending &c = idx->pend;
-    c = sffg_index::Pending{};
-    c.kind = 2;
-    c.fused = true;
-    c.nq = nq;
-    c.capacity = capacity;
-    c.cap1 = cap1;
-    c.r2 = r2;
-    c.queries = queries;
-    c.counts_out = counts_out;
-    c.ids_out = ids_out;
-    c.d2_out = d2_out;
-    c.total_out = total_out;
-    c.small = true;
-    c.copy[c.n_copy++] = {counts_out, hc, cbytes};
-    return SFFG_OK;
-  }
-  rc = idx->q.reserve(qbytes);
-  if (rc == SFFG_OK) rc = idx->counts.reserve(cbytes);
-  if (rc != SFFG_OK) return rc;
-  if (small) {
-    std::memcpy(hq, queries, qbytes);
-    SFFG_CUDA(cudaMemcpyAsync(idx->q.p, hq, qbytes, cudaMemcpyHostToDevice, st));
-  } else {
-    SFFG_CUDA(cudaMemcpyAsync(idx->q.p, queries, qbytes, cudaMemcpyHostToDevice, st));
-  }
-  SFFG_CUDA(cudaMemsetAsync(idx->counts.p, 0, cbytes, st));
-  rc = ensure_sorted(idx, st);
-  if (rc != SFFG_OK) return rc;
-  const bool pruned = idx->n_sorted > 0;
-  const SortedDev sv = sorted_view(idx);
-  if (pruned) SFFG_CUDA(launch_radius_count_pruned(v, sv, (const float *)idx->q.p, nq, r2, (int32_t *)idx->counts.p, g_rt.sm_count, st));
-  else SFFG_CUDA(launch_radius_count(v, (const float *)idx->q.p, nq, r2, (int32_t *)idx->counts.p, plan, st));
-  SFFG_CUDA(cudaMemcpyAsync(small ? (void *)hc : (void *)counts_out, idx->counts.p, cbytes, cudaMemcpyDeviceToHost, st));
-  sffg_index::Pending &c = idx->pend;
-  c = sffg_index::Pending{};
+  const bool small = qbytes <= IndexStaging::kQueryBytes && cbytes <= IndexStaging::kCountBytes;
+  sffg_index::Pending c{};
   c.kind = 2;
   c.nq = nq;
   c.capacity = capacity;
   c.r2 = r2;
+  c.queries = queries;
   c.counts_out = counts_out;
   c.ids_out = ids_out;
   c.d2_out = d2_out;
   c.total_out = total_out;
   c.small = small;
-  c.pruned = pruned;
-  if (small) c.copy[c.n_copy++] = {counts_out, hc, cbytes};
+  if (small) c.copy[c.n_copy++] = {counts_out, h.counts(), cbytes};
+  const size_t rowoff_bytes = (size_t)nq * sizeof(int64_t);
+  if (allow_fused && small && ids_out && capacity > 0 && idx->n <= kFusedRadiusMaxNodes && qbytes <= IndexStaging::kFlagAt &&
+      rowoff_bytes + 64 <= IndexStaging::kRowsBytes / 2) {
+    // planner-sized search on a small index: ONE kernel (block per query) that reads the queries from and writes counts,
+    // row offsets and sorted rows to pinned mapped memory -- one stream operation besides zeroing the row allocator, one
+    // host synchronisation.  Staging: [queries | flag] [counts] [row offsets | ids | d2].
+    std::memcpy(h.queries(), queries, qbytes);
+    *h.fused_flag() = 0;
+    c.fused = true;
+    c.cap1 = IndexStaging::rows_cap(rowoff_bytes);
+    SFFG_CUDA(cudaMemsetAsync(idx->d_total.get(), 0, sizeof(unsigned long long), st));
+    SFFG_CUDA(launch_radius_fused(v, reinterpret_cast<const float *>(h.queries()), nq, r2, c.cap1, h.counts(), h.rows_head(),
+                                  h.rows_ids(rowoff_bytes), h.rows_d2(rowoff_bytes, c.cap1), idx->d_total.get(), h.fused_flag(), st));
+    idx->pend = c;
+    return SFFG_OK;
+  }
+  rc = idx->q.reserve(qbytes);
+  if (rc == SFFG_OK) rc = idx->counts.reserve(cbytes);
+  if (rc != SFFG_OK) return rc;
+  SFFG_CUDA(upload_async(idx->q.p, queries, qbytes, small ? h.queries() : nullptr, st));
+  SFFG_CUDA(cudaMemsetAsync(idx->counts.p, 0, cbytes, st));
+  rc = ensure_sorted(idx, st);
+  if (rc != SFFG_OK) return rc;
+  c.pruned = idx->n_sorted > 0;
+  const float *q = (const float *)idx->q.p;
+  if (c.pruned) SFFG_CUDA(launch_radius_count_pruned(v, sorted_view(idx), q, nq, r2, (int32_t *)idx->counts.p, g_rt.sm_count, st));
+  else SFFG_CUDA(launch_radius_count(v, q, nq, r2, (int32_t *)idx->counts.p, plan_knn(nq, idx->n, g_rt.sm_count), st));
+  SFFG_CUDA(cudaMemcpyAsync(small ? (void *)h.counts() : (void *)counts_out, idx->counts.p, cbytes, cudaMemcpyDeviceToHost, st));
   // Planner-sized call with result buffers: the exclusive scan of the counts runs on the device, so that count, scan, fill
   // and sort are enqueued back to back and the call costs ONE host synchronisation.  The rows land in pinned mapped
-  // memory ([total][ids][d2] in the result part of the staging area); when they do not fit there, or not into the
+  // memory ([total][ids][d2] in the rows part of the staging area); when they do not fit there, or not into the
   // caller's capacity, the kernels after the scan do nothing and sffg_index_end takes the two-synchronisation route.
-  c.cap1 = std::min<int64_t>(capacity, (int64_t)((hr_bytes - 8) / 8));
+  c.cap1 = std::min<int64_t>(capacity, IndexStaging::rows_cap(sizeof(int64_t)));
   c.one_sync = small && ids_out && c.cap1 > 0;
   if (c.one_sync) {
     rc = idx->offsets.reserve((size_t)nq * 8);
     if (rc == SFFG_OK) rc = idx->cursor.reserve(cbytes);
     if (rc == SFFG_OK) rc = idx->keys.reserve((size_t)c.cap1 * 8);
-    if (rc != SFFG_OK) {
-      c.kind = 0;
-      return rc;
-    }
-    int64_t *h_total = reinterpret_cast<int64_t *>(hr);
-    int32_t *h_ids = reinterpret_cast<int32_t *>(hr + 8);
-    float *h_d2 = reinterpret_cast<float *>(hr + 8 + (size_t)c.cap1 * 4);
-    *h_total = -1;
-    SFFG_CUDA(launch_radius_offsets((const int32_t *)idx->counts.p, nq, c.cap1, (int64_t *)idx->offsets.p, h_total, st));
-    SFFG_CUDA(cudaMemsetAsync(idx->cursor.p, 0, cbytes, st));
-    if (pruned)
-      SFFG_CUDA(launch_radius_fill_pruned(v, sv, (const float *)idx->q.p, nq, r2, (const int64_t *)idx->offsets.p, (int32_t *)idx->cursor.p,
-                                          (unsigned long long *)idx->keys.p, g_rt.sm_count, st));
-    else
-      SFFG_CUDA(launch_radius_fill(v, (const float *)idx->q.p, nq, r2, (const int64_t *)idx->offsets.p, (int32_t *)idx->cursor.p,
-                                   (unsigned long long *)idx->keys.p, plan, st));
-    SFFG_CUDA(launch_radius_sort((unsigned long long *)idx->keys.p, (const int64_t *)idx->offsets.p, (const int32_t *)idx->counts.p, nq,
-                                 h_ids, h_d2, st));
+    if (rc != SFFG_OK) return rc;
+    *h.rows_head() = -1;
+    SFFG_CUDA(launch_radius_offsets((const int32_t *)idx->counts.p, nq, c.cap1, (int64_t *)idx->offsets.p, h.rows_head(), st));
+    rc = radius_fill_sort(idx, c.pruned, nq, r2, h.rows_ids(sizeof(int64_t)), h.rows_d2(sizeof(int64_t), c.cap1));
+    if (rc != SFFG_OK) return rc;
   }
+  idx->pend = c;
   return SFFG_OK;
 }
 
@@ -1574,12 +1552,13 @@ int sffg_index_end(sffg_index *idx) {
   if (idx->pend.kind == 0) return SFFG_OK;
   const sffg_index::Pending c = idx->pend;
   idx->pend.kind = 0;
-  SFFG_CUDA(cudaStreamSynchronize(idx->stream));
+  SFFG_CUDA(cudaStreamSynchronize(idx->stream.get()));
   for (int i = 0; i < c.n_copy; ++i) std::memcpy(c.copy[i].dst, c.copy[i].src, c.copy[i].bytes);
   if (c.kind != 2) return SFFG_OK;
+  const IndexStaging h = idx->staging();
   int64_t total = 0;
   if (c.fused) {
-    const int flag = *reinterpret_cast<const volatile int *>(idx->h_small + (64 << 10) - 16);
+    const int flag = *reinterpret_cast<const volatile int *>(h.fused_flag());
     for (int64_t i = 0; i < c.nq; ++i) total += c.counts_out[i];
     if (c.total_out) *c.total_out = total;
     if (total == 0) return SFFG_OK;
@@ -1590,10 +1569,10 @@ int sffg_index_end(sffg_index *idx) {
       const int rc = radius_begin_impl(idx, c.queries, c.nq, c.r2, c.counts_out, c.ids_out, c.d2_out, c.capacity, c.total_out, false);
       return rc != SFFG_OK ? rc : sffg_index_end(idx);
     }
-    const unsigned char *hr = idx->h_small + (128 << 10);
-    const int64_t *h_rowoff = reinterpret_cast<const int64_t *>(hr);
-    const int32_t *h_ids = reinterpret_cast<const int32_t *>(hr + (size_t)c.nq * 8);
-    const float *h_d2 = reinterpret_cast<const float *>(hr + (size_t)c.nq * 8 + (size_t)c.cap1 * 4);
+    const size_t rowoff_bytes = (size_t)c.nq * sizeof(int64_t);
+    const int64_t *h_rowoff = h.rows_head();
+    const int32_t *h_ids = h.rows_ids(rowoff_bytes);
+    const float *h_d2 = h.rows_d2(rowoff_bytes, c.cap1);
     int64_t run = 0;
     for (int64_t i = 0; i < c.nq; ++i) {   // rows were packed in the order the blocks finished: back into query order
       const int64_t n_i = c.counts_out[i];
@@ -1606,14 +1585,13 @@ int sffg_index_end(sffg_index *idx) {
     return SFFG_OK;
   }
   if (c.one_sync) {
-    unsigned char *hr = idx->h_small + (128 << 10);
-    total = *reinterpret_cast<const int64_t *>(hr);
+    total = *h.rows_head();
     if (total < 0) return fail(SFFG_ERR_INTERNAL, "sffg_radius: the device-side scan did not report a total");
     if (c.total_out) *c.total_out = total;
     if (total == 0) return SFFG_OK;
     if (total <= c.cap1) {
-      std::memcpy(c.ids_out, hr + 8, (size_t)total * 4);
-      std::memcpy(c.d2_out, hr + 8 + (size_t)c.cap1 * 4, (size_t)total * 4);
+      std::memcpy(c.ids_out, h.rows_ids(sizeof(int64_t)), (size_t)total * 4);
+      std::memcpy(c.d2_out, h.rows_d2(sizeof(int64_t), c.cap1), (size_t)total * 4);
       return SFFG_OK;
     }
   } else {

@@ -83,6 +83,32 @@ def test_rounds_in_flight_match_blocking_calls(sff, orc, meshes):
     env.close()
 
 
+def test_obstacle_changes_are_refused_while_edges_are_pending(sff, orc, meshes):
+    """refit and set-obstacles are host-pointer calls too: between sffg_check_edges_begin and sffg_env_end both are refused
+    and the obstacle set stays as it was, so the pending results equal the blocking call's"""
+    from space_filling_forest_star_b200 import _lib
+    L = _lib.load()
+    on, rn, _ = CASES["B"]
+    env = sff.Environment(meshes[on], meshes[rn])
+    s = orc.gen_poses(SEED + 42, 0, 500, [-45, 45, -45, 45, 0, 125]).astype(np.float64)
+    e = s.copy()
+    e[:, :3] += np.random.RandomState(4).normal(size=(500, 3))
+    free_w, first_w = env.isPathFree(s, e, 0.1, 0, want_first_hit=True)
+    free = np.zeros(500, np.uint8)
+    first = np.zeros(500, np.int32)
+    _lib.check(L.sffg_check_edges_begin(env._h, _p(s), _p(e), 500, 0.1, 0, _p(free), _p(first)))
+    with pytest.raises(_lib.SffgError) as refit:
+        env.refit_obstacles(meshes[on])
+    assert refit.value.code == 3
+    with pytest.raises(_lib.SffgError) as replace:
+        env.set_obstacles(meshes[on][: len(meshes[on]) // 2])
+    assert replace.value.code == 3
+    _lib.check(L.sffg_env_end(env._h))
+    np.testing.assert_array_equal(free, free_w)
+    np.testing.assert_array_equal(first, first_w)
+    env.close()
+
+
 def test_radius_one_synchronisation_keeps_the_capacity_protocol(sff, orc):
     """device-side scan: rows that fit come back from the single pass; a caller buffer that is too small gives
     SFFG_ERR_CAPACITY with the needed size; results larger than the pinned staging area take the two-pass route"""
