@@ -10,7 +10,9 @@
  *   - all functions return an int status (SFFG_OK == 0) unless stated; sffg_last_error() gives the text
  *   - triangle soups are double [n][9] = p1.xyz p2.xyz p3.xyz, already offset+scaled the way
  *     Obstacle<T>::addPoint does it (src/environment.h:198-211)
- *   - poses are [n][6] = x y z yaw pitch roll (Point<T>, src/primitives.h:86-102), angles in radians
+ *   - poses are [n][6] = x y z yaw pitch roll (Point<T>, src/primitives.h:86-102), angles in radians; any finite
+ *     angle is accepted and the verdict is exact for it (no range reduction by the caller: a double angle of 1000 rad is
+ *     judged at that angle, not at its float neighbour)
  *   - "host" calls take caller-owned host pointers and block until results are in the output arrays
  *   - "_device" calls take device pointers + a cudaStream_t (as void*), enqueue, and return immediately
  *   - one host thread per handle at a time

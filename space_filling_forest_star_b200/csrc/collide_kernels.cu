@@ -45,6 +45,10 @@ constexpr unsigned kFull = 0xffffffffu;
 #endif
 constexpr float kEpsBox = 1.52587890625e-05f;   // 2^-16, relative slack of the box culls   (>= 140 ulp, see DESIGN.md)
 constexpr float kEpsSat = 1.52587890625e-05f;   // 2^-16, relative position error of the FP32 SAT stage
+// Both budgets include the FP32 rotation's error against FillRotationMatrix of the pose's own angles: every sin / cos
+// within 2^-21 of the exact value (sincosf <= 2 ulp, plus up to 2^-23 from narrowing a double angle |a| <= float(pi) to
+// float; wider double angles are never narrowed, see sincos_narrow), every entry of R within 2^-19.  Unbounded, the
+// narrowing alone would be 2^-15 at |a| ~ 1000 rad, and an FP32 certificate could be issued for the wrong pose.
 
 struct XTri {        // obstacle triangle in the robot frame (FP32); 13 words = odd stride, bank-conflict free
   float v[9];
@@ -362,12 +366,8 @@ template <> struct LanePose<kFmtMatrixF64> {
   }
 };
 
-// Point<T>::FillRotationMatrix in FP32 (certificate stage only)
-__device__ __forceinline__ void rotation_f32(float yaw, float pitch, float roll, float *m) {
-  float sy, cy, sp, cp, sr, cr;
-  sincosf(yaw, &sy, &cy);
-  sincosf(pitch, &sp, &cp);
-  sincosf(roll, &sr, &cr);
+// Point<T>::FillRotationMatrix in FP32 (certificate stage only), from the sines and cosines of yaw, pitch and roll
+__device__ __forceinline__ void rotation_f32_sc(float sy, float cy, float sp, float cp, float sr, float cr, float *m) {
   m[0] = cy * cp;
   m[1] = cy * sp * sr - sy * cr;
   m[2] = cy * sp * cr + sy * sr;
@@ -378,12 +378,37 @@ __device__ __forceinline__ void rotation_f32(float yaw, float pitch, float roll,
   m[7] = cp * sr;
   m[8] = cp * cr;
 }
-__device__ __forceinline__ void LanePose<kFmtEulerF32>::rot32(float *R) const { rotation_f32(a[0], a[1], a[2], R); }
+__device__ __forceinline__ void LanePose<kFmtEulerF32>::rot32(float *R) const {
+  float sy, cy, sp, cp, sr, cr;
+  sincosf(a[0], &sy, &cy);
+  sincosf(a[1], &sp, &cp);
+  sincosf(a[2], &sr, &cr);
+  rotation_f32_sc(sy, cy, sp, cp, sr, cr, R);
+}
+// sin and cos of a double angle for the FP32 rotation.  Narrowing the angle to float moves it by up to half an ulp of the
+// angle: at most 2^-23 while |a| <= float(pi), which the error budget covers (see kEpsSat), but 2^-15 at 1000 rad, more
+// than the whole budget.  Angles beyond float(pi) therefore take sincos(double) of the angle itself, rounded to float
+// (within 2^-25 plus sincos's 1 ulp in double, for every finite angle); in-range angles keep the FP32 path.
+__device__ __forceinline__ void sincos_narrow(double a, float *s, float *c) {
+  const float af = (float)a;
+  if (fabsf(af) <= 3.14159274f) {
+    sincosf(af, s, c);
+  } else {
+    double sd, cd;
+    sincos(a, &sd, &cd);
+    *s = (float)sd;
+    *c = (float)cd;
+  }
+}
 __device__ __forceinline__ void LanePose<kFmtEulerF64>::rot32(float *R) const {
   if (identity) {
     R[0] = 1.f; R[1] = 0.f; R[2] = 0.f; R[3] = 0.f; R[4] = 1.f; R[5] = 0.f; R[6] = 0.f; R[7] = 0.f; R[8] = 1.f;
   } else {
-    rotation_f32((float)a[0], (float)a[1], (float)a[2], R);
+    float sy, cy, sp, cp, sr, cr;
+    sincos_narrow(a[0], &sy, &cy);
+    sincos_narrow(a[1], &sp, &cp);
+    sincos_narrow(a[2], &sr, &cr);
+    rotation_f32_sc(sy, cy, sp, cp, sr, cr, R);
   }
 }
 
