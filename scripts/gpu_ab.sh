@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B of compile-time variants of the collision kernels (libsffg_<tag>.so next to the default library)
+# A/B of other builds of the library (libsffg_<tag>.so next to the default library, e.g. built from another commit)
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 for v in "" "$@"; do

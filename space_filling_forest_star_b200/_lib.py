@@ -103,7 +103,7 @@ def load() -> C.CDLL:
     global _lib
     if _lib is None:
         import os
-        variant = os.environ.get("SFFG_LIB")   # tuning variants built by scripts/; the default is the in-tree library
+        variant = os.environ.get("SFFG_LIB")   # another build for A/B measurements; the default is the in-tree library
         path = Path(variant) if variant else _build.build_native()
         L = C.CDLL(str(path))
         for name, (res, args) in SIGNATURES.items():

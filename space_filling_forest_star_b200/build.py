@@ -32,17 +32,14 @@ def is_stale() -> bool:
     return any((CSRC / f).resolve().stat().st_mtime > t for f in SOURCES + HEADERS)
 
 
-def build_native(force: bool = False, verbose: bool = False, defines=(), out: Path = None) -> Path:
-    """Compile every CUDA/C++ source of the engine for sm_100a into space_filling_forest_star_b200/libsffg.so.
-
-    ``defines``/``out`` build tuning variants next to the default library (used by scripts/ for A/B measurements)."""
-    target = Path(out) if out else LIB
-    if out is None and not force and not is_stale():
+def build_native(force: bool = False, verbose: bool = False) -> Path:
+    """Compile every CUDA/C++ source of the engine for sm_100a into space_filling_forest_star_b200/libsffg.so."""
+    if not force and not is_stale():
         return LIB
     host_cxx = "/usr/bin/g++" if Path("/usr/bin/g++").exists() else "g++"
     cmd = [_nvcc(), "-O3", "-std=c++17", *ARCH, "-lineinfo", "-ccbin", host_cxx,
            "-Xcompiler", "-fPIC,-fvisibility=hidden", "-shared", "-cudart", "static",
-           *[f"-D{d}" for d in defines], "-o", str(target), *[str(CSRC / s) for s in SOURCES]]
+           "-o", str(LIB), *[str(CSRC / s) for s in SOURCES]]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     res = subprocess.run(cmd, capture_output=True, text=True)
@@ -50,7 +47,7 @@ def build_native(force: bool = False, verbose: bool = False, defines=(), out: Pa
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)
     if verbose:
         print(res.stderr)
-    return target
+    return LIB
 
 
 HOST_SRC = PKG / "host" / "sff_planner.cpp"

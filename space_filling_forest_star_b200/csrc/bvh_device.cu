@@ -26,12 +26,6 @@
 namespace sffg {
 namespace {
 
-__device__ __forceinline__ int f2o(float f) {   // order-preserving float -> int
-  const int i = __float_as_int(f);
-  return i >= 0 ? i : i ^ 0x7fffffff;
-}
-__device__ __forceinline__ float o2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
-
 // tbox: 6 floats per triangle (lo.xyz rounded down, hi.xyz rounded up); bounds: 3 x min, 3 x max as ordered ints
 __global__ void tri_prepare_kernel(const double *__restrict__ soup, int n, float *__restrict__ tbox, int *bounds) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -49,7 +43,7 @@ __global__ void tri_prepare_kernel(const double *__restrict__ soup, int n, float
   }
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
-    int l = f2o(lo[k]), h = f2o(hi[k]);
+    int l = float_to_ordered(lo[k]), h = float_to_ordered(hi[k]);
 #pragma unroll
     for (int s = 16; s > 0; s >>= 1) {
       l = min(l, __shfl_xor_sync(0xffffffffu, l, s));
@@ -79,7 +73,7 @@ __global__ void morton_kernel(const float *__restrict__ tbox, int n, const int *
   unsigned q[3];
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
-    const float lo = o2f(bounds[k]), hi = o2f(bounds[3 + k]);
+    const float lo = ordered_to_float(bounds[k]), hi = ordered_to_float(bounds[3 + k]);
     const float c = 0.5f * tbox[6 * (size_t)t + k] + 0.5f * tbox[6 * (size_t)t + 3 + k];
     const float ext = hi - lo;
     float u = ext > 0.f ? (c - lo) / ext : 0.f;
@@ -279,6 +273,19 @@ struct Scratch {
     if (e_ != cudaSuccess) return e_; \
   } while (0)
 
+// waits for the stream and reads the scene bounds tri_prepare_kernel left in `bounds` as the root box
+cudaError_t read_root_bounds(const int *bounds, cudaStream_t st, double root_lo[3], double root_hi[3]) {
+  int hb[6];
+  BD_CUDA(cudaMemcpyAsync(hb, bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
+  BD_CUDA(cudaStreamSynchronize(st));
+  BD_CUDA(cudaGetLastError());
+  for (int k = 0; k < 3; ++k) {
+    root_lo[k] = ordered_to_float(hb[k]);
+    root_hi[k] = ordered_to_float(hb[3 + k]);
+  }
+  return cudaSuccess;
+}
+
 }  // namespace
 
 cudaError_t build_bvh_device(const double *d_soup, int n, cudaStream_t st, DeviceBvh *out) {
@@ -376,22 +383,11 @@ cudaError_t build_bvh_device(const double *d_soup, int n, cudaStream_t st, Devic
   }
   cudaMemcpyAsync(slots, slots_big, (size_t)n_nodes * kWide * sizeof(ChildSlot), cudaMemcpyDeviceToDevice, st);
   gather_tris_kernel<<<G, T, 0, st>>>(d_soup, vals_out, n, t64, t32);
-  int hb[6];
-  cudaMemcpyAsync(hb, bounds, sizeof hb, cudaMemcpyDeviceToHost, st);
-  e = cudaStreamSynchronize(st);
-  if (e == cudaSuccess) e = cudaGetLastError();
-  if (e != cudaSuccess) {
+  if ((e = read_root_bounds(bounds, st, out->root_lo, out->root_hi)) != cudaSuccess) {
     cudaFree(slots);
     cudaFree(t64);
     cudaFree(t32);
     return fail_free(e);
-  }
-  for (int k = 0; k < 6; ++k) {
-    const int i = hb[k];
-    const int bits = i >= 0 ? i : i ^ 0x7fffffff;
-    float f;
-    memcpy(&f, &bits, 4);
-    (k < 3 ? out->root_lo[k] : out->root_hi[k - 3]) = (double)f;
   }
   out->d_slots = slots;
   out->d_tris64 = t64;
@@ -421,18 +417,7 @@ cudaError_t refit_bvh_device(const double *d_soup, int n, ChildSlot *d_slots, do
     const int threads = level_count[l] * 8;
     fit_level_kernel<<<(threads + 255) / 256, 256, 0, st>>>(d_slots, level_base[l], level_count[l], tbox, d_order);
   }
-  int hb[6];
-  BD_CUDA(cudaMemcpyAsync(hb, bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
-  BD_CUDA(cudaStreamSynchronize(st));
-  BD_CUDA(cudaGetLastError());
-  for (int k = 0; k < 6; ++k) {
-    const int i = hb[k];
-    const int bits = i >= 0 ? i : i ^ 0x7fffffff;
-    float f;
-    memcpy(&f, &bits, 4);
-    (k < 3 ? root_lo[k] : root_hi[k - 3]) = (double)f;
-  }
-  return cudaSuccess;
+  return read_root_bounds(bounds, st, root_lo, root_hi);
 }
 
 }  // namespace sffg

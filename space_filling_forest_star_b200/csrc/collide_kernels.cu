@@ -28,21 +28,13 @@
 namespace sffg {
 namespace {
 
-#ifndef SFFG_WARPS
-#define SFFG_WARPS 16
-#endif
-#ifndef SFFG_TRI_FLUSH
-#define SFFG_TRI_FLUSH 1
-#endif
-constexpr int kWarpsPerBlock = SFFG_WARPS;
+constexpr int kWarpsPerBlock = 16;
 constexpr int kThreads = kWarpsPerBlock * 32;
+constexpr int kMinBlocksPerSm = 1;   // __launch_bounds__ of the pose and edge kernels
 constexpr int kStackCap = 384;   // node ids pending for one pose
 constexpr int kTriCap = 64;      // candidate triangles pending for one pose
-constexpr int kTriFlush = SFFG_TRI_FLUSH;    // run the triangle stage once this many candidates are pending
+constexpr int kCandCap = 192;    // candidate triangles of one group of edge samples (swept-box traversal)
 constexpr unsigned kFull = 0xffffffffu;
-#ifndef SFFG_MIN_BLOCKS
-#define SFFG_MIN_BLOCKS 1
-#endif
 constexpr float kEpsBox = 1.52587890625e-05f;   // 2^-16, relative slack of the box culls   (>= 140 ulp, see DESIGN.md)
 constexpr float kEpsSat = 1.52587890625e-05f;   // 2^-16, relative position error of the FP32 SAT stage
 // Both budgets include the FP32 rotation's error against FillRotationMatrix of the pose's own angles: every sin / cos
@@ -57,11 +49,6 @@ struct XTri {        // obstacle triangle in the robot frame (FP32); 13 words = 
   int tri;           // triangle index (leaf order) for the exact stage
   int pad;
 };
-
-#ifndef SFFG_CAND_CAP
-#define SFFG_CAND_CAP 192
-#endif
-constexpr int kCandCap = SFFG_CAND_CAP;    // candidate triangles of one group of edge samples (swept-box traversal)
 
 struct WarpScratch {
   int stack[kStackCap];
@@ -570,11 +557,71 @@ __device__ __forceinline__ void triangle_stage(const EnvDev &E, WarpScratch &ws,
   }
 }
 
+// what one step of the hierarchy walk found: the ballot of lanes holding an accepted leaf, and this lane's triangle
+struct StepLeaves {
+  unsigned mask;
+  bool mine;
+  int tri;
+};
+
+// One step of the warp-cooperative walk of the hierarchy.  Step 0 (`first`) tests the precomputed <= 32-slot cut of the
+// top of the hierarchy with all lanes (top_cut emits no empty slot).  Every later step pops up to 4 nodes from the stack,
+// 8 lanes per node; near the cap it pops 1 (strict depth-first grows the stack by at most 7 per level), which keeps any
+// hierarchy of depth <= 45 inside the stack.  Interior children that `overlaps(a, b)` accepts are pushed; `sp` may end
+// above kStackCap (those pushes are dropped), and the caller decides what that means.  Accepted leaves are returned for
+// the caller to append where it keeps them.
+template <bool COUNT, class Overlaps>
+__device__ __forceinline__ StepLeaves walk_step(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, bool first, int &sp,
+                                                int lane, const Overlaps &overlaps, Tally &tally) {
+  bool ov = false;
+  int child = kEmptyChild;
+  bool active;
+  if (first) {
+    active = lane < E.n_top;
+    if (active) {
+      const float4 a = cs.top[lane], b = cs.top[kTopSlots + lane];
+      child = __float_as_int(a.w);
+      ov = overlaps(a, b);
+    }
+  } else {
+    const int take = sp > kStackCap - 64 ? 1 : (sp < 4 ? sp : 4);
+    const int grp = lane >> 3;
+    active = grp < take;
+    const int node = active ? ws.stack[sp - 1 - grp] : 0;
+    __syncwarp();
+    sp -= take;
+    if (active) {
+      float4 a, b;
+      if (node < cs.n_stage) {   // (nodes of one step are popped together: mostly one side of this branch)
+        const int si = node * kWide + (lane & 7);
+        a = cs.nodes[si];                             // staged as two arrays (all `a` halves, then all `b` halves):
+        b = cs.nodes[cs.n_stage * kWide + si];        // 8 lanes read 128 contiguous bytes, no bank conflicts
+      } else {
+        const float4 *gn = E.slots + ((size_t)node * kWide + (lane & 7)) * 2;
+        a = __ldg(gn);
+        b = __ldg(gn + 1);
+      }
+      child = __float_as_int(a.w);
+      if (child != kEmptyChild) ov = overlaps(a, b);
+    }
+  }
+  const unsigned m_int = __ballot_sync(kFull, ov && child >= 0);
+  const unsigned m_leaf = __ballot_sync(kFull, ov && child < 0);
+  if (COUNT) { tally.box += __popc(__ballot_sync(kFull, active && child != kEmptyChild)); tally.steps += 1; }
+  if (ov && child >= 0) {
+    const int pos = sp + __popc(m_int & ((1u << lane) - 1u));
+    if (pos < kStackCap) ws.stack[pos] = child;
+  }
+  sp += __popc(m_int);
+  return {m_leaf, ov && child < 0, ~child};
+}
+
 template <int FMT, bool COUNT>
 __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const PoseU &P,
                               const LanePose<FMT> &lp, int src, int lane, Tally &tally) {
   const RobotTri *srob = cs.rob;
   const BoxTest bt = make_box_test(E, P);
+  const auto overlaps = [&](const float4 a, const float4 b) { return slot_overlaps(E, P, bt, a, b); };
   const unsigned lt = (1u << lane) - 1u;
 
   int sp = 0, ntri = 0;
@@ -582,60 +629,20 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
   PairCtx pc;
   if (COUNT) tally.past_root += 1;
 
-  bool first = true;   // step 0 tests the precomputed <=32-box cut of the top of the hierarchy with all lanes
+  bool first = true;
   while (true) {
+    // walk until a candidate triangle is pending, then run the triangle stage over what the last step found
     if (first || (sp > 0 && ntri <= kTriCap - 32)) {
-      bool ov = false;
-      int child = kEmptyChild;
-      bool active;
-      if (first) {
-        active = lane < E.n_top;
-        if (active) {
-          const float4 a = cs.top[lane], b = cs.top[kTopSlots + lane];
-          child = __float_as_int(a.w);
-          ov = slot_overlaps(E, P, bt, a, b);
-        }
-        first = false;
-      } else {
-        // 4 nodes per step while there is room; near the cap fall back to strict depth-first (1 node per step grows the
-        // stack by at most 7 per level), which keeps any hierarchy of depth <= 45 inside the stack
-        const int take = sp > kStackCap - 64 ? 1 : (sp < 4 ? sp : 4);
-        const int grp = lane >> 3;
-        active = grp < take;
-        const int node = active ? ws.stack[sp - 1 - grp] : 0;
-        __syncwarp();
-        sp -= take;
-        if (active) {
-          float4 a, b;
-          if (node < cs.n_stage) {   // (nodes of one step are popped together: mostly one side of this branch)
-            const int si = node * kWide + (lane & 7);
-            a = cs.nodes[si];                             // staged as two arrays (all `a` halves, then all `b` halves):
-            b = cs.nodes[cs.n_stage * kWide + si];        // 8 lanes read 128 contiguous bytes, no bank conflicts
-          } else {
-            const float4 *gn = E.slots + ((size_t)node * kWide + (lane & 7)) * 2;
-            a = __ldg(gn);
-            b = __ldg(gn + 1);
-          }
-          child = __float_as_int(a.w);
-          if (child != kEmptyChild) ov = slot_overlaps(E, P, bt, a, b);
-        }
-      }
-      const unsigned m_int = __ballot_sync(kFull, ov && child >= 0);
-      const unsigned m_leaf = __ballot_sync(kFull, ov && child < 0);
-      if (COUNT) { tally.box += __popc(__ballot_sync(kFull, active && child != kEmptyChild)); tally.steps += 1; }
-      if (ov && child >= 0) {
-        const int pos = sp + __popc(m_int & lt);
-        if (pos < kStackCap) ws.stack[pos] = child;
-      }
-      if (ov && child < 0) ws.tri[ntri + __popc(m_leaf & lt)] = ~child;
-      sp += __popc(m_int);
-      ntri += __popc(m_leaf);
+      const StepLeaves lv = walk_step<COUNT>(E, ws, cs, first, sp, lane, overlaps, tally);
+      first = false;
+      if (lv.mine) ws.tri[ntri + __popc(lv.mask & lt)] = lv.tri;
+      ntri += __popc(lv.mask);
       if (sp > kStackCap) {     // never silently drop work: flag the launch as failed
         if (lane == 0) *reinterpret_cast<volatile int *>(E.status) = 1;
         sp = kStackCap;
       }
       __syncwarp();
-      if (sp > 0 && ntri < kTriFlush) continue;
+      if (sp > 0 && ntri == 0) continue;
     }
     if (ntri == 0) {
       if (sp == 0) break;
@@ -658,69 +665,27 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
 // traversal was 63 % of the edge kernel's instructions.)  The list is a superset of what the per-sample traversal would
 // deliver and every stage after it is unchanged, so the verdicts are the same.
 // ---------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ int f2ord(float f) {   // order-preserving float -> int
-  const int i = __float_as_int(f);
-  return i >= 0 ? i : i ^ 0x7fffffff;
-}
-__device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
-
 // every leaf triangle whose slot box meets [lo, hi] -> ws.cand; returns their number, or -1 when the list would overflow
 template <bool COUNT>
 __device__ int collect_box_candidates(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const float *lo, const float *hi, int lane,
                                       Tally &tally) {
+  // slot box [c - h, c + h] against [lo, hi], directed rounding keeps the test conservative
+  const auto overlaps = [&](const float4 a, const float4 b) {
+    return __fadd_ru(a.x, b.x) >= lo[0] && __fsub_rd(a.x, b.x) <= hi[0] && __fadd_ru(a.y, b.y) >= lo[1] &&
+           __fsub_rd(a.y, b.y) <= hi[1] && __fadd_ru(a.z, b.z) >= lo[2] && __fsub_rd(a.z, b.z) <= hi[2];
+  };
   const unsigned lt = (1u << lane) - 1u;
   int sp = 0, ncand = 0;
   bool first = true;
   while (first || sp > 0) {
-    bool ov = false;
-    int child = kEmptyChild;
-    bool active;
-    float4 a, b;
-    if (first) {
-      active = lane < E.n_top;
-      if (active) {
-        a = cs.top[lane];
-        b = cs.top[kTopSlots + lane];
-      }
-      first = false;
-    } else {
-      const int take = sp > kStackCap - 64 ? 1 : (sp < 4 ? sp : 4);
-      const int grp = lane >> 3;
-      active = grp < take;
-      const int node = active ? ws.stack[sp - 1 - grp] : 0;
-      __syncwarp();
-      sp -= take;
-      if (active) {
-        if (node < cs.n_stage) {
-          const int si = node * kWide + (lane & 7);
-          a = cs.nodes[si];
-          b = cs.nodes[cs.n_stage * kWide + si];
-        } else {
-          const float4 *gn = E.slots + ((size_t)node * kWide + (lane & 7)) * 2;
-          a = __ldg(gn);
-          b = __ldg(gn + 1);
-        }
-      }
+    const StepLeaves lv = walk_step<COUNT>(E, ws, cs, first, sp, lane, overlaps, tally);
+    first = false;
+    if (ncand + __popc(lv.mask) > kCandCap || sp > kStackCap) {
+      __syncwarp();   // the caller falls back to the per-sample traversal (which reports stack overflows) on this stack
+      return -1;
     }
-    if (active) {
-      child = __float_as_int(a.w);
-      // slot box [c - h, c + h] against [lo, hi], directed rounding keeps the test conservative
-      if (child != kEmptyChild)
-        ov = __fadd_ru(a.x, b.x) >= lo[0] && __fsub_rd(a.x, b.x) <= hi[0] && __fadd_ru(a.y, b.y) >= lo[1] && __fsub_rd(a.y, b.y) <= hi[1] &&
-             __fadd_ru(a.z, b.z) >= lo[2] && __fsub_rd(a.z, b.z) <= hi[2];
-    }
-    const unsigned m_int = __ballot_sync(kFull, ov && child >= 0);
-    const unsigned m_leaf = __ballot_sync(kFull, ov && child < 0);
-    if (COUNT) { tally.box += __popc(__ballot_sync(kFull, active && child != kEmptyChild)); tally.steps += 1; }
-    if (ncand + __popc(m_leaf) > kCandCap) return -1;
-    if (ov && child >= 0) {
-      const int pos = sp + __popc(m_int & lt);
-      if (pos < kStackCap) ws.stack[pos] = child;
-    }
-    if (ov && child < 0) ws.cand[ncand + __popc(m_leaf & lt)] = ~child;
-    sp += __popc(m_int);
-    ncand += __popc(m_leaf);
-    if (sp > kStackCap) return -1;   // (the caller falls back to the per-sample traversal, which reports overflows)
+    if (lv.mine) ws.cand[ncand + __popc(lv.mask & lt)] = lv.tri;
+    ncand += __popc(lv.mask);
     __syncwarp();
   }
   return ncand;
@@ -823,6 +788,7 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
   if (alive) lp.rot32(R);
   unsigned todo = __ballot_sync(kFull, alive);
   unsigned hitmask = 0;
+  int ncand = -1;   // >= 0: every sample runs the triangle stage over the swept-box candidate list ws.cand[0, ncand)
   if (SWEPT_CAPABLE && swept && __popc(todo) >= 2) {
     // one traversal with the box that holds the robot at every surviving sample, outward rounded: with the identity
     // rotation (reference mode) the robot's own axis-aligned box, with interpolated angles the cube around its bounding
@@ -836,32 +802,13 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
       const float rh = swept_identity ? __fadd_ru(E.rob_c[k], E.rob_h[k]) : E.rob_radius;
       const float l = __fsub_rd(__fadd_rd(c, rl), pad);
       const float h = __fadd_ru(__fadd_ru(cu, rh), pad);
-      blo[k] = __reduce_min_sync(kFull, alive ? f2ord(l) : 0x7fffffff);
-      bhi[k] = __reduce_max_sync(kFull, alive ? f2ord(h) : (int)0x80000000);
+      blo[k] = __reduce_min_sync(kFull, alive ? float_to_ordered(l) : 0x7fffffff);
+      bhi[k] = __reduce_max_sync(kFull, alive ? float_to_ordered(h) : (int)0x80000000);
     }
-    const float lo[3] = {ord2f(blo[0]), ord2f(blo[1]), ord2f(blo[2])}, hi[3] = {ord2f(bhi[0]), ord2f(bhi[1]), ord2f(bhi[2])};
-    const int ncand = collect_box_candidates<COUNT>(E, ws, cs, lo, hi, lane, tally);
+    const float lo[3] = {ordered_to_float(blo[0]), ordered_to_float(blo[1]), ordered_to_float(blo[2])},
+                hi[3] = {ordered_to_float(bhi[0]), ordered_to_float(bhi[1]), ordered_to_float(bhi[2])};
+    ncand = collect_box_candidates<COUNT>(E, ws, cs, lo, hi, lane, tally);   // -1 (overflow): per-sample traversal
     if (ncand == 0) return 0;
-    if (ncand > 0) {
-      while (todo) {
-        const int src = __ffs(todo) - 1;
-        todo &= todo - 1;
-        PoseU P;
-#pragma unroll
-        for (int k = 0; k < 9; ++k) P.R[k] = __shfl_sync(kFull, R[k], src);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          P.Thi[k] = __shfl_sync(kFull, thi[k], src);
-          P.Tlo[k] = FMT == kFmtEulerF32 ? 0.f : __shfl_sync(kFull, tlo[k], src);
-        }
-        if (pose_hits_candidates<FMT, COUNT>(E, ws, cs, P, lp, src, lane, ncand, tally)) {
-          hitmask |= 1u << src;
-          if (first_only) break;
-        }
-      }
-      return hitmask;
-    }
-    // (list overflow: fall through to the per-sample traversal)
   }
   while (todo) {
     const int src = __ffs(todo) - 1;
@@ -874,7 +821,8 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
       P.Thi[k] = __shfl_sync(kFull, thi[k], src);
       P.Tlo[k] = FMT == kFmtEulerF32 ? 0.f : __shfl_sync(kFull, tlo[k], src);
     }
-    if (warp_pose_hit<FMT, COUNT>(E, ws, cs, P, lp, src, lane, tally)) {
+    if (SWEPT_CAPABLE && ncand > 0 ? pose_hits_candidates<FMT, COUNT>(E, ws, cs, P, lp, src, lane, ncand, tally)
+                                   : warp_pose_hit<FMT, COUNT>(E, ws, cs, P, lp, src, lane, tally)) {
       hitmask |= 1u << src;
       if (first_only) break;
     }
@@ -905,7 +853,7 @@ __device__ __forceinline__ void wait_flags(const FlagSet &f, unsigned epoch, int
 }
 
 template <int FMT, bool COUNT>
-__global__ void __launch_bounds__(kThreads, SFFG_MIN_BLOCKS) collide_poses_kernel(EnvDev E, const void *poses, long long n,
+__global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) collide_poses_kernel(EnvDev E, const void *poses, long long n,
                                                                                   OutSet outs, GatherSync gs, int chunk) {
   extern __shared__ __align__(16) unsigned char smem[];
   if (gs.flags.n > 0 && gs.wait_epoch != 0 && threadIdx.x == 0) wait_flags(gs.flags, gs.wait_epoch, E.status);
@@ -984,18 +932,13 @@ constexpr int kNoHit = 0x7f7f7f7f;   // what cudaMemsetAsync(..., 0x7f, ...) pro
 // work units (edge, range) a planner-sized batch is cut into per resident warp.  Measured with the swept-box traversal
 // (profiles/r02_edges_swept.md): 1 beats 2 / 4 / 8 for the planner's short edges (2 048 edges of length 4: 41.6 us per call
 // against 44.9 / 50.9 / 69.6), long edges lose a little (length 12: 68 against 62 us at 4).
-#ifndef SFFG_EDGE_UNITS_PER_WARP
-#define SFFG_EDGE_UNITS_PER_WARP 1
-#endif
+constexpr int kEdgeUnitsPerWarp = 1;
 
-#ifndef SFFG_EDGE_MIN_BLOCKS
-#define SFFG_EDGE_MIN_BLOCKS SFFG_MIN_BLOCKS
-#endif
 template <bool COUNT>
-__global__ void __launch_bounds__(kThreads, SFFG_EDGE_MIN_BLOCKS) check_edges_kernel(EnvDev E, const double *starts,
-                                                                                const double *ends, long long m, double sample,
-                                                                                int rot_mode, uint8_t *free_out,
-                                                                                int32_t *first_hit, int split, int *fh) {
+__global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) check_edges_kernel(EnvDev E, const double *starts,
+                                                                           const double *ends, long long m, double sample,
+                                                                           int rot_mode, uint8_t *free_out,
+                                                                           int32_t *first_hit, int split, int *fh) {
   extern __shared__ __align__(16) unsigned char smem[];
   const CtaShared cs = stage_cta(E, smem, E.n_stage_max);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1243,29 +1186,27 @@ size_t collide_smem_bytes(int n_robot, int n_stage_max) {
 }
 
 
+// launches `want` CTAs of kThreads, or as many as are resident at once if fewer (the kernels pull their work units from
+// E.work_counter); the grid size goes to `*grid` for the work-counter bookkeeping
+template <auto Kernel, class... Args>
+static cudaError_t launch_resident(long long want, size_t smem, cudaStream_t stream, const LaunchCfg &cfg, int *grid, Args... args) {
+  const KernelCfg kc = kernel_cfg<Kernel>(smem);
+  if (kc.err != cudaSuccess) return kc.err;
+  *grid = cfg.sm_count * kc.per_sm;
+  if (want < *grid) *grid = (int)want;
+  Kernel<<<*grid, kThreads, smem, stream>>>(args...);
+  return cudaGetLastError();
+}
+
 template <int FMT>
 static cudaError_t launch_poses_fmt(const EnvDev &env, const void *d_poses, int64_t n, const OutSet &d_verdict, const GatherSync &gs,
-                                    cudaStream_t stream, const LaunchCfg &cfg, bool count, int chunk, int *grid_out) {
+                                    cudaStream_t stream, const LaunchCfg &cfg, bool count, int chunk, int *grid) {
   const size_t smem = collide_smem_bytes(env.n_robot, env.n_stage_max);
   const long long chunks = (n + chunk - 1) / chunk;
   const long long want = (chunks + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  cudaError_t e;
-  if (count) {
-    const KernelCfg kc = kernel_cfg<collide_poses_kernel<FMT, true>>(smem);
-    if ((e = kc.err) != cudaSuccess) return e;
-    int grid = cfg.sm_count * kc.per_sm;
-    if (want < grid) grid = (int)want;
-    *grid_out = grid;
-    collide_poses_kernel<FMT, true><<<grid, kThreads, smem, stream>>>(env, d_poses, (long long)n, d_verdict, gs, chunk);
-  } else {
-    const KernelCfg kc = kernel_cfg<collide_poses_kernel<FMT, false>>(smem);
-    if ((e = kc.err) != cudaSuccess) return e;
-    int grid = cfg.sm_count * kc.per_sm;
-    if (want < grid) grid = (int)want;
-    *grid_out = grid;
-    collide_poses_kernel<FMT, false><<<grid, kThreads, smem, stream>>>(env, d_poses, (long long)n, d_verdict, gs, chunk);
-  }
-  return cudaGetLastError();
+  if (count)
+    return launch_resident<collide_poses_kernel<FMT, true>>(want, smem, stream, cfg, grid, env, d_poses, (long long)n, d_verdict, gs, chunk);
+  return launch_resident<collide_poses_kernel<FMT, false>>(want, smem, stream, cfg, grid, env, d_poses, (long long)n, d_verdict, gs, chunk);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1339,28 +1280,20 @@ cudaError_t launch_check_edges(const EnvDev &env_in, const double *d_starts, con
   const size_t smem = collide_smem_bytes(env.n_robot, env.n_stage_max);
   // warps per edge: enough units for ~2 per resident warp, at most 32 (needs the scratch array)
   int split = 1;
-  const long long warps = (long long)cfg.sm_count * kWarpsPerBlock * SFFG_EDGE_UNITS_PER_WARP;
+  const long long warps = (long long)cfg.sm_count * kWarpsPerBlock * kEdgeUnitsPerWarp;
   if (d_fh_scratch)
     while (split < 32 && m * split < warps) split <<= 1;
   const long long units = m * split;
   const long long want = (units + kWarpsPerBlock - 1) / kWarpsPerBlock;
   cudaError_t e;
   if (split > 1 && (e = cudaMemsetAsync(d_fh_scratch, 0x7f, (size_t)m * sizeof(int), stream)) != cudaSuccess) return e;
-  int grid;
-  if (count) {
-    const KernelCfg kc = kernel_cfg<check_edges_kernel<true>>(smem);
-    if ((e = kc.err) != cudaSuccess) return e;
-    grid = cfg.sm_count * kc.per_sm;
-    if (want < grid) grid = (int)want;
-    check_edges_kernel<true><<<grid, kThreads, smem, stream>>>(env, d_starts, d_ends, (long long)m, sample_dist, rot_mode, d_free, d_first_hit, split, d_fh_scratch);
-  } else {
-    const KernelCfg kc = kernel_cfg<check_edges_kernel<false>>(smem);
-    if ((e = kc.err) != cudaSuccess) return e;
-    grid = cfg.sm_count * kc.per_sm;
-    if (want < grid) grid = (int)want;
-    check_edges_kernel<false><<<grid, kThreads, smem, stream>>>(env, d_starts, d_ends, (long long)m, sample_dist, rot_mode, d_free, d_first_hit, split, d_fh_scratch);
-  }
-  e = cudaGetLastError();
+  int grid = 0;
+  if (count)
+    e = launch_resident<check_edges_kernel<true>>(want, smem, stream, cfg, &grid, env, d_starts, d_ends, (long long)m, sample_dist,
+                                                  rot_mode, d_free, d_first_hit, split, d_fh_scratch);
+  else
+    e = launch_resident<check_edges_kernel<false>>(want, smem, stream, cfg, &grid, env, d_starts, d_ends, (long long)m, sample_dist,
+                                                   rot_mode, d_free, d_first_hit, split, d_fh_scratch);
   if (e != cudaSuccess) return e;
   *work_base_io += (unsigned)units + (unsigned)grid * kWarpsPerBlock;
   if (split > 1) {

@@ -1,6 +1,7 @@
 // common.h -- internal declarations shared by the host-side C++ and the CUDA translation units of libsffg.so
 #pragma once
 #include <cstdint>
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -69,5 +70,21 @@ int load_mesh(const char *path, int is_obj, const double position[3], double sca
 
 float round_up_f32(double v);     // smallest float >= v
 float round_down_f32(double v);   // largest float <= v
+
+#ifdef __CUDACC__
+// Order-preserving float <-> int: the ints compare as the (non-NaN) floats do, so integer min / max reductions and
+// atomics can bound floats.  Non-negative floats keep their bits, negative ones flip their magnitude bits.
+__host__ __device__ __forceinline__ int float_to_ordered(float f) {
+  int i;
+  memcpy(&i, &f, sizeof i);
+  return i >= 0 ? i : i ^ 0x7fffffff;
+}
+__host__ __device__ __forceinline__ float ordered_to_float(int i) {
+  i = i >= 0 ? i : i ^ 0x7fffffff;
+  float f;
+  memcpy(&f, &i, sizeof f);
+  return f;
+}
+#endif
 
 }  // namespace sffg

@@ -90,3 +90,40 @@ def test_check_moves_is_collide_or_not_path_free(sff, orc, meshes):
         np.testing.assert_array_equal(ok, (env.isPathFree(s, e).astype(bool) & ~env.Collide(e).astype(bool)).astype(np.uint8))
     assert len(env.checkMoves(np.zeros((0, 6)), np.zeros((0, 6)))) == 0
     env.close()
+
+
+def tube_soup(r):
+    """~32 000 tiny triangles, cleared only from tubes of radius 0.5 around nine parallel lines along (1, 1, 1), and 27
+    edges of length 5 * sqrt(3) per copy: along the tubes (free), half-way between them and out of the tubes into the soup"""
+    u = np.ones(3) / np.sqrt(3)
+    lines = np.array([(x, y, 0.0) for x in (-1.5, 0.0, 1.5) for y in (-1.5, 0.0, 1.5)])
+    c = r.uniform(-2.5, 7.5, (36000, 3))
+    rel = c[:, None, :] - lines[None]
+    c = c[np.linalg.norm(rel - (rel @ u)[..., None] * u, axis=2).min(1) > 0.5]
+    soup = c[:, None, :] + r.uniform(-0.02, 0.02, (len(c), 3, 3))
+    copies = 256
+    s = np.zeros((copies, 27, 6))
+    s[..., :3] = np.concatenate([lines + 0.5, lines + [1.25, 1.25, 0.5], lines + 0.5])[None] + r.uniform(0, 0.5, (copies, 1, 1))
+    e = s.copy()
+    e[:, :18, :3] += 5.0
+    e[:, 18:, :3] += [5.0, 5.0, 2.0]
+    s[..., 3:] = e[..., 3:] = r.uniform(-np.pi, np.pi, (copies, 27, 3))   # constant angles: samples 0.1 apart in position
+    return soup, s.reshape(-1, 6), e.reshape(-1, 6)
+
+
+def test_edges_through_a_soup_that_overflows_the_swept_box_list(sff, orc, meshes):
+    """the swept box of a 32-sample group holds more leaf triangles than its candidate list (192), so the kernel falls back
+    to the per-sample walk for those groups; 6 912 edges so that each edge runs on one warp (a warp's share of a split
+    edge is too short to overflow the list)"""
+    rob = meshes["robot_small_s1"]   # a 0.5 x 0.5 plate: bounding radius 0.35 < tube radius 0.5
+    soup, s, e = tube_soup(np.random.RandomState(5))
+    env = sff.Environment(soup, rob)
+    mo, mr = orc.ObbModel(soup), orc.ObbModel(rob)
+    for mode in (sff.ROT_REFERENCE, sff.ROT_INTERPOLATE):
+        free, first = env.isPathFree(s, e, 0.1, mode, want_first_hit=True)
+        wf, wh, _ = orc.edges_free(soup, rob, s, e, 0.1, mode, models=(mo, mr))
+        np.testing.assert_array_equal(free, wf)
+        np.testing.assert_array_equal(first, wh)
+        wf = wf.reshape(-1, 27)
+        assert wf[:, :9].all() and wf[:, 9:].mean() < 0.1 and (wh > 32).sum() > 100
+    env.close()
