@@ -4,7 +4,8 @@
 // (reference src/environment.h:306-316, :269-276) and of Solver<T,R>::isPathFree (src/problemStruct.h:154-168).
 //
 // Execution model (one warp = one pose at a time):
-//   phase A  lane-per-pose: load 32 poses, cull the robot's bounding sphere against the obstacle AABB, build R
+//   phase A  lane-per-pose: load 32 poses, cull the robot's bounding sphere against the obstacle AABB and the clearance
+//            grid's cell bit, build R, test the robot against the cell's separating plane
 //   phase B  warp-per-pose for the survivors:
 //            - 8-wide AABB BVH (breadth-first node order); the top of the hierarchy -- a <=32-box cut tested by all lanes
 //              in step 0 and the first three levels of nodes -- is staged in shared memory once per CTA; warp-shared DFS
@@ -20,6 +21,8 @@
 //            - __ballot/__any early-out on the first confirmed contact (verdict-equivalent to RAPID's ALL_CONTACTS
 //              because the caller only looks at num_contacts != 0)
 // The result equals "OR over all triangle pairs of the double-precision SAT" -- the oracle's ground truth.
+#include <algorithm>
+#include <cfloat>
 #include <cstdint>
 #include <mutex>
 
@@ -707,15 +710,67 @@ __device__ bool pose_hits_candidates(const EnvDev &E, WarpScratch &ws, const Cta
   return hit;
 }
 
-// O(1) free-space test: the cell of the clearance grid that holds the robot origin.  A clear bit proves that no obstacle
+// The cell of the clearance grid that holds the robot origin, or -1 outside the grid.  A clear bit proves that no obstacle
 // triangle comes within the robot's bounding radius of any point of the cell (the build inflates the reach by the cell's
 // half diagonal plus rounding margins), so the pose is free whatever its orientation.
-__device__ __forceinline__ bool clearance_says_free(const EnvDev &E, float tx, float ty, float tz) {
+__device__ __forceinline__ int grid_cell(const EnvDev &E, float tx, float ty, float tz) {
   const float fx = (tx - E.grid_o[0]) * E.grid_inv_h, fy = (ty - E.grid_o[1]) * E.grid_inv_h, fz = (tz - E.grid_o[2]) * E.grid_inv_h;
   if (!(fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)E.grid_n[0] && fy < (float)E.grid_n[1] && fz < (float)E.grid_n[2]))
-    return false;
-  const unsigned cell = ((unsigned)fz * (unsigned)E.grid_n[1] + (unsigned)fy) * (unsigned)E.grid_n[0] + (unsigned)fx;
-  return ((__ldg(E.clear_bits + (cell >> 5)) >> (cell & 31)) & 1u) == 0u;
+    return -1;
+  return (int)(((unsigned)fz * (unsigned)E.grid_n[1] + (unsigned)fy) * (unsigned)E.grid_n[0] + (unsigned)fx);
+}
+__device__ __forceinline__ bool cell_marked(const EnvDev &E, int cell) {
+  return ((__ldg(E.clear_bits + (cell >> 5)) >> (cell & 31)) & 1u) != 0u;
+}
+
+// Plane directions: the 26 integer vectors m in {-1,0,1}^3 \ {0}, d = 9 (mz + 1) + 3 (my + 1) + (mx + 1); d = 13 (m = 0)
+// is the "no plane" record, whose offset is -FLT_MAX so that no pose passes it.
+constexpr int kNoPlaneDir = 13;
+constexpr unsigned kNoPlane = 0x80800000u | kNoPlaneDir;   // float_to_ordered(-FLT_MAX) = 0x80800000, low 5 bits clear
+__device__ __forceinline__ void plane_dir(int d, float *m) {
+  m[0] = (float)(d % 3 - 1);
+  m[1] = (float)(d / 3 % 3 - 1);
+  m[2] = (float)(d / 9 - 1);
+}
+
+// O(1) free-space test for a marked cell: its plane record `word` holds a direction m and an offset c with m.p >= c for every
+// vertex p of every obstacle triangle that marks the cell (the build's own predicate, so every triangle that can touch a
+// robot whose origin lies in the cell, by the argument of the clear bit).  A convex robot hull strictly below the plane
+// (m.x < c for every robot point x = R v + T) meets none of those triangles, so the pose is free.
+//
+// The test computes s = m.thi + max_v (R^T m).v in FP32 and clears the pose when s + margin < c, c rounded down.  The
+// margin bounds |s - m.(R_o v + T)| for the oracle's FP64 rotation R_o of the pose's own angles (or its matrix):
+//   - R: every entry of the FP32 rotation within 2^-19 of R_o (see kEpsSat); w = R^T m has |m|_1 <= 3 exact terms per
+//     entry, so |w - R_o^T m| <= 3 * 2^-19 + 2^-21 < 2^-17 per entry, times |v|_1 <= sqrt(3) rho; the nearest-float
+//     vertices and the FP32 dot product add < 12 * 2^-24 rho.  The box support (w.c + sum |w_j| h_j, |c_j| + h_j <= rho)
+//     moves by < 3 * 2^-17 rho + 12 * 2^-24 rho.  Allotted 2^-15 rho (plane_pad).
+//   - T = thi + tlo: |m.tlo| <= |tlo|_1, added as is; m.thi and the final sums round by < 2^-22 (|thi|_1 + 3 rho),
+//     allotted 2^-20 |thi|_1 (and the 2^-15 rho above).
+//   - the grid's absolute slack (1e-3 h + maxc * 3.9e-6, as in its reach), carried in plane_pad so that a plane never
+//     clears a pose that the grid's own rounding allowances would hold back.
+// With these the robot stays below the plane by a positive gap in exact arithmetic, and the oracle's FP64 SAT finds
+// separated triangles separated -- the same ground the clear bit and the FP32 certificates stand on (DESIGN.md 4.1).
+__device__ __forceinline__ bool plane_says_free(const EnvDev &E, unsigned word, const float *R, const float *thi, float tlo_mag) {
+  const float c = ordered_to_float((int)(word & ~31u));
+  float m[3];
+  plane_dir((int)(word & 31u), m);
+  const float w0 = m[0] * R[0] + m[1] * R[3] + m[2] * R[6], w1 = m[0] * R[1] + m[1] * R[4] + m[2] * R[7],
+              w2 = m[0] * R[2] + m[1] * R[5] + m[2] * R[8];
+  float sup;
+  if (E.rob_verts) {
+    sup = -FLT_MAX;
+#pragma unroll 1   // (unrolled, the loop costs the edge kernel extra spill reloads)
+    for (int i = 0; i < E.n_rob_verts; ++i) {
+      const float4 v = __ldg(E.rob_verts + i);
+      sup = fmaxf(sup, w0 * v.x + w1 * v.y + w2 * v.z);
+    }
+  } else {
+    sup = w0 * E.rob_c[0] + w1 * E.rob_c[1] + w2 * E.rob_c[2] + fabsf(w0) * E.rob_h[0] + fabsf(w1) * E.rob_h[1] +
+          fabsf(w2) * E.rob_h[2];
+  }
+  const float s = m[0] * thi[0] + m[1] * thi[1] + m[2] * thi[2] + sup;
+  const float margin = E.plane_pad + 9.5367431640625e-07f * (fabsf(thi[0]) + fabsf(thi[1]) + fabsf(thi[2])) + tlo_mag;
+  return s + margin < c;
 }
 
 // lane-per-pose cull: robot bounding sphere (about the robot origin) against the obstacle AABB
@@ -781,11 +836,17 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
                                                    bool swept = false, bool swept_identity = true) {
   float thi[3], tlo[3], R[9];
   lp.split(thi, tlo);
-  bool alive = valid && E.n_obst > 0 &&
-               sphere_hits_root(E, thi[0], thi[1], thi[2], fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]));
-  if (alive && E.grid_n[0] > 0) alive = !clearance_says_free(E, thi[0], thi[1], thi[2]);
-  if (COUNT) tally.past_grid += __popc(__ballot_sync(kFull, alive));
+  const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
+  bool alive = valid && E.n_obst > 0 && sphere_hits_root(E, thi[0], thi[1], thi[2], tlo_mag);
+  unsigned plane = kNoPlane;   // (loaded before the rotation is built, which hides the load)
+  if (alive && E.grid_n[0] > 0) {
+    const int cell = grid_cell(E, thi[0], thi[1], thi[2]);
+    alive = cell < 0 || cell_marked(E, cell);
+    if (alive && cell >= 0) plane = __ldg(E.planes + cell);
+  }
   if (alive) lp.rot32(R);
+  if (alive && plane != kNoPlane) alive = !plane_says_free(E, plane, R, thi, tlo_mag);
+  if (COUNT) tally.past_grid += __popc(__ballot_sync(kFull, alive));
   unsigned todo = __ballot_sync(kFull, alive);
   unsigned hitmask = 0;
   int ncand = -1;   // >= 0: every sample runs the triangle stage over the swept-box candidate list ws.cand[0, ncand)
@@ -1074,13 +1135,37 @@ __device__ __forceinline__ float point_tri_dist2(const float *p, const float *a,
   return dx * dx + dy * dy + dz * dz;
 }
 
+// plane direction of pass slot j (the 26 directions skip d = 13)
+__device__ __forceinline__ int pass_dir(int dir0, int j) {
+  const int k = dir0 + j;
+  return k < kNoPlaneDir ? k : k + 1;
+}
+// m.p rounded down: m has entries in {-1, 0, 1}, so the products are exact and only the two sums round
+__device__ __forceinline__ float dot_dir_rd(const float *m, const float *p) {
+  return __fadd_rd(__fadd_rd(m[0] * p[0], m[1] * p[1]), m[2] * p[2]);
+}
+
+// Marks (bits != null) the cells within `reach` of each triangle and lowers mins[j][cell] to the triangle's bound
+// min over its vertices of m_d.p, d = pass_dir(dir0, j) for j < ndir: the float vertices, rounded down, minus
+// |m|_1 times their representation error, so the bound holds for the FP64 triangle.
+constexpr int kClearanceThreads = 256;
 __global__ void build_clearance_kernel(const float4 *__restrict__ tris, int n_tris, float ox, float oy, float oz, float h, int nx,
-                                       int ny, int nz, float reach, unsigned *bits) {
+                                       int ny, int nz, float reach, unsigned *bits, int *mins, int dir0, int ndir) {
+  __shared__ int tri_min[kClearanceThreads / 32][32];
   const int lane = threadIdx.x & 31;
   const int t = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
   if (t >= n_tris) return;
   const float4 v0 = __ldg(tris + 3 * (size_t)t), v1 = __ldg(tris + 3 * (size_t)t + 1), v2 = __ldg(tris + 3 * (size_t)t + 2);
   const float a[3] = {v0.x, v0.y, v0.z}, b[3] = {v1.x, v1.y, v1.z}, c[3] = {v2.x, v2.y, v2.z};
+  int *tmin = tri_min[threadIdx.x >> 5];
+  if (lane < ndir) {
+    float m[3];
+    plane_dir(pass_dir(dir0, lane), m);
+    const float l1 = fabsf(m[0]) + fabsf(m[1]) + fabsf(m[2]);
+    const float lo = fminf(dot_dir_rd(m, a), fminf(dot_dir_rd(m, b), dot_dir_rd(m, c)));
+    tmin[lane] = float_to_ordered(__fsub_rd(lo, __fmul_ru(l1, v0.w)));
+  }
+  __syncwarp();
   const float inv = 1.0f / h;
   int lo[3], hi[3];
   const float o[3] = {ox, oy, oz};
@@ -1100,9 +1185,45 @@ __global__ void build_clearance_kernel(const float4 *__restrict__ tris, int n_tr
     const float p[3] = {ox + (ix + 0.5f) * h, oy + (iy + 0.5f) * h, oz + (iz + 0.5f) * h};
     if (!(point_tri_dist2(p, a, b, c) > r2)) {   // NaN (degenerate triangle) marks the cell: never optimistic
       const unsigned cell = ((unsigned)iz * (unsigned)ny + (unsigned)iy) * (unsigned)nx + (unsigned)ix;
-      atomicOr(bits + (cell >> 5), 1u << (cell & 31));
+      if (bits) atomicOr(bits + (cell >> 5), 1u << (cell & 31));
+      const size_t cells = (size_t)nx * ny * nz;
+      for (int j = 0; j < ndir; ++j) atomicMin(mins + j * cells + cell, tmin[j]);
     }
   }
+}
+
+// Each marked cell keeps, of the directions of this pass and the record it already holds (`first`: none), the one with the
+// most room c - max_{x in cell} m.x per unit length of m -- what the robot's origin may use before it reaches the plane.
+// A record with no room at all is the no-plane record.  Unmarked cells get the no-plane record on the first pass.
+__global__ void choose_planes_kernel(const unsigned *__restrict__ bits, const int *__restrict__ mins, int nx, int ny, int nz,
+                                     float ox, float oy, float oz, float h, int dir0, int ndir, bool first, unsigned *planes) {
+  const long long cells = (long long)nx * ny * nz;
+  const long long cell = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (cell >= cells) return;
+  if (!((__ldg(bits + (cell >> 5)) >> (cell & 31)) & 1u)) {
+    if (first) planes[cell] = kNoPlane;
+    return;
+  }
+  const int ix = (int)(cell % nx), iy = (int)(cell / nx % ny), iz = (int)(cell / ((long long)nx * ny));
+  const float p[3] = {ox + (ix + 0.5f) * h, oy + (iy + 0.5f) * h, oz + (iz + 0.5f) * h};
+  const auto room = [&](int d, float c) {
+    float m[3];
+    plane_dir(d, m);
+    const float l1 = fabsf(m[0]) + fabsf(m[1]) + fabsf(m[2]);
+    return (c - (m[0] * p[0] + m[1] * p[1] + m[2] * p[2] + 0.5f * h * l1)) * rsqrtf(l1);
+  };
+  unsigned best = first ? kNoPlane : planes[cell];
+  float best_room = (best & 31u) == kNoPlaneDir ? 0.f : room((int)(best & 31u), ordered_to_float((int)(best & ~31u)));
+  for (int j = 0; j < ndir; ++j) {
+    const int d = pass_dir(dir0, j);
+    const int o = __ldg(mins + j * cells + cell);
+    const float r = room(d, ordered_to_float(o));
+    if (r > best_room) {
+      best_room = r;
+      best = ((unsigned)o & ~31u) | (unsigned)d;   // clearing low bits of an ordered int rounds the offset down
+    }
+  }
+  planes[cell] = best;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1304,13 +1425,25 @@ cudaError_t launch_check_edges(const EnvDev &env_in, const double *d_starts, con
 }
 
 cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, cudaStream_t stream) {
+                                   unsigned *d_bits, unsigned *d_planes, int *d_scratch, size_t scratch_words, cudaStream_t stream) {
   if (n_tris <= 0) return cudaSuccess;
-  const int threads = 256;
-  const long long blocks = ((long long)n_tris * 32 + threads - 1) / threads;
-  build_clearance_kernel<<<(unsigned)blocks, threads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h, n[0], n[1],
-                                                                    n[2], reach, d_bits);
-  return cudaGetLastError();
+  const size_t cells = (size_t)n[0] * n[1] * n[2];
+  const int per_pass = (int)std::min<size_t>(26, scratch_words / cells);
+  if (per_pass < 1) return cudaErrorInvalidValue;
+  const long long blocks = ((long long)n_tris * 32 + kClearanceThreads - 1) / kClearanceThreads;
+  const long long cell_blocks = ((long long)cells + 255) / 256;
+  for (int dir0 = 0; dir0 < 26; dir0 += per_pass) {
+    const int ndir = std::min(per_pass, 26 - dir0);
+    cudaError_t e = cudaMemsetAsync(d_scratch, 0x7f, (size_t)ndir * cells * sizeof(int), stream);
+    if (e != cudaSuccess) return e;
+    build_clearance_kernel<<<(unsigned)blocks, kClearanceThreads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h,
+                                                                                n[0], n[1], n[2], reach, dir0 == 0 ? d_bits : nullptr,
+                                                                                d_scratch, dir0, ndir);
+    choose_planes_kernel<<<(unsigned)cell_blocks, 256, 0, stream>>>(d_bits, d_scratch, n[0], n[1], n[2], origin[0], origin[1], origin[2],
+                                                                   h, dir0, ndir, dir0 == 0, d_planes);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  return cudaSuccess;
 }
 
 cudaError_t launch_gen_poses(uint64_t seed, uint64_t first, int64_t n, const float range[6], float *d_out,

@@ -26,6 +26,12 @@ struct EnvDev {
   float grid_o[3];
   float grid_inv_h;
   int grid_n[3];
+  // one separating plane per grid cell (word = direction index in the low 5 bits, offset above them, see plane_says_free),
+  // set whenever clear_bits is
+  const unsigned *planes;
+  float plane_pad;              // absolute part of the plane test's margin, rounded up
+  const float4 *rob_verts;      // distinct robot vertices (nearest floats); null above kPlaneVertCap: the robot box stands in
+  int n_rob_verts;
   unsigned long long *counters; // 5 x u64 (may be null): poses, past_root, box_tests, pair_tests, exact_tests
   int *status;                  // device int, set non-zero on traversal-stack overflow
   unsigned int *work_counter;   // persistent-kernel work distribution: never reset, units are (fetched value - work_base)
@@ -89,8 +95,14 @@ size_t collide_smem_bytes(int n_robot, int n_stage_max);
 #endif
 constexpr int kStageNodesCap = SFFG_STAGE_NODES;
 
-// marks every cell whose centre is within `reach` of an obstacle triangle (one warp per triangle)
+// Marks every cell whose centre is within `reach` of an obstacle triangle (one warp per triangle) in `d_bits`, and picks
+// each marked cell's plane record (`d_planes`, one word per cell).  `d_scratch` holds `scratch_words` ints (at least one
+// per cell); the 26 plane directions take ceil(26 / (scratch_words / cells)) passes over the triangles.
 cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, cudaStream_t stream);
+                                   unsigned *d_bits, unsigned *d_planes, int *d_scratch, size_t scratch_words, cudaStream_t stream);
+
+// Robots with more distinct vertices than this take the support of their box in the plane test (robot_small has 8,
+// robot_cyl_small 64).  One FMA chain per vertex per pose past the grid bit.
+constexpr int kPlaneVertCap = 16;
 
 }  // namespace sffg

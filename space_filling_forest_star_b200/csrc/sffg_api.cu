@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -174,7 +175,8 @@ using namespace sffg;
 struct sffg_env {
   EnvDev dev{};
   DevPtr<ChildSlot> d_slots, d_top;
-  DevPtr<unsigned> d_clear;
+  DevPtr<unsigned> d_clear, d_planes;
+  DevPtr<float4> d_rob_verts;
   DevPtr<float4> d_tris32;
   DevPtr<double> d_tris64, d_robot64;
   DevPtr<RobotTri> d_robot;
@@ -379,6 +381,7 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   EnvDev &d = env->dev;
   env->d_top.reset();
   env->d_clear.reset();
+  env->d_planes.reset();
   SFFG_CUDA(upload(env->d_top, top.data(), top.size() * sizeof(ChildSlot), &bytes));
   d.n_obst = (int)n_obst;
   for (int k = 0; k < 3; ++k) {
@@ -388,6 +391,8 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   }
   // ---- clearance grid (free-space bitmap) over the obstacle AABB dilated by the robot's reach
   d.clear_bits = nullptr;
+  d.planes = nullptr;
+  d.plane_pad = 0.f;
   env->info.grid_cells = 0;
   env->info.grid_cell_size = 0;
   d.grid_n[0] = d.grid_n[1] = d.grid_n[2] = 0;
@@ -412,14 +417,26 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
     }
     // reach = bounding radius + half cell diagonal + margins for float rounding of vertices, cell lookup and distances
     const double reach = (rho + 0.8661 * h) * 1.002 + 1e-3 * h + maxc * 3.9e-6;
-    const size_t words = ((size_t)gn[0] * gn[1] * gn[2] + 31) / 32;
+    const size_t cells = (size_t)gn[0] * gn[1] * gn[2];
+    const size_t words = (cells + 31) / 32;
     SFFG_CUDA(dev_alloc(env->d_clear, words * sizeof(unsigned)));
     SFFG_CUDA(cudaMemset(env->d_clear.get(), 0, words * sizeof(unsigned)));
-    SFFG_CUDA(launch_build_clearance(env->d_tris32.get(), (int)n_obst, go, (float)h, gn, (float)reach, env->d_clear.get(),
-                                     env->streams[0].get()));
-    SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
-    bytes += words * sizeof(unsigned);
+    // one plane word per cell; the per-direction bounds of the build live in a temporary block of at most 512 MB (one
+    // pass over the triangles for grids up to 5.1 M cells, more passes above)
+    SFFG_CUDA(dev_alloc(env->d_planes, cells * sizeof(unsigned)));
+    {
+      const size_t scratch_words = std::min<size_t>(26 * cells, std::max<size_t>(cells, size_t(1) << 27));
+      DevPtr<int> d_scratch;
+      SFFG_CUDA(dev_alloc(d_scratch, scratch_words * sizeof(int)));
+      SFFG_CUDA(launch_build_clearance(env->d_tris32.get(), (int)n_obst, go, (float)h, gn, (float)reach, env->d_clear.get(),
+                                       env->d_planes.get(), d_scratch.get(), scratch_words, env->streams[0].get()));
+      SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
+    }
+    bytes += words * sizeof(unsigned) + cells * sizeof(unsigned);
     d.clear_bits = env->d_clear.get();
+    d.planes = env->d_planes.get();
+    // absolute part of the plane test's margin (see plane_says_free): the grid's slack and 2^-15 rho for the rotated robot
+    d.plane_pad = round_up_f32((1e-3 * h + maxc * 3.9e-6 + rho * std::ldexp(1.0, -15)) * 1.001);
     for (int k = 0; k < 3; ++k) {
       d.grid_o[k] = go[k];
       d.grid_n[k] = gn[k];
@@ -581,9 +598,20 @@ int sffg_env_create_ex(const double *obst_tris, int64_t n_obst, const double *ro
     d.rob_h[k] = round_up_f32(std::max(rhi[k] - (double)d.rob_c[k], (double)d.rob_c[k] - rlo[k]) * 1.0000001);
   }
   d.rob_radius = round_up_f32(std::sqrt(rad2) * 1.000001);
+  // distinct robot vertices for the plane test of the clearance grid (nearest floats; the test's margin covers the rounding)
+  std::vector<float4> verts;
+  {
+    std::vector<std::array<double, 3>> dv;
+    for (int64_t i = 0; i < 3 * n_robot; ++i) dv.push_back({robot_tris[3 * i], robot_tris[3 * i + 1], robot_tris[3 * i + 2]});
+    std::sort(dv.begin(), dv.end());
+    dv.erase(std::unique(dv.begin(), dv.end()), dv.end());
+    if (dv.size() <= (size_t)kPlaneVertCap)
+      for (const auto &v : dv) verts.push_back(make_float4((float)v[0], (float)v[1], (float)v[2], 0.f));
+  }
 
   size_t bytes = 0;
   SFFG_CUDA(upload(env->d_robot, rob.data(), rob.size() * sizeof(RobotTri), &bytes));
+  if (!verts.empty()) SFFG_CUDA(upload(env->d_rob_verts, verts.data(), verts.size() * sizeof(float4), &bytes));
   SFFG_CUDA(upload(env->d_robot64, robot_tris, 9 * (size_t)n_robot * sizeof(double), &bytes));
   SFFG_CUDA(dev_alloc(env->d_counters, 10 * sizeof(unsigned long long)));
   SFFG_CUDA(cudaMemset(env->d_counters.get(), 0, 10 * sizeof(unsigned long long)));
@@ -596,6 +624,8 @@ int sffg_env_create_ex(const double *obst_tris, int64_t n_obst, const double *ro
   SFFG_CUDA(make_event(env->order_ev));
   d.robot = env->d_robot.get();
   d.robot64 = env->d_robot64.get();
+  d.rob_verts = verts.empty() ? nullptr : env->d_rob_verts.get();
+  d.n_rob_verts = (int)verts.size();
   d.counters = nullptr;
   d.status = env->h_status.get();   // unified addressing: the mapped host pointer is valid on the device
   d.work_counter = env->d_work.get();
