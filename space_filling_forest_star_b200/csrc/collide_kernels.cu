@@ -619,7 +619,17 @@ __device__ __forceinline__ StepLeaves walk_step(const EnvDev &E, WarpScratch &ws
   return {m_leaf, ov && child < 0, ~child};
 }
 
-template <int FMT, bool COUNT>
+// The cell of the clearance grid that holds the robot origin, or -1 outside the grid.  A clear bit proves that no obstacle
+// triangle comes within the robot's bounding radius of any point of the cell (the build inflates the reach by the cell's
+// half diagonal plus rounding margins), so the pose is free whatever its orientation.
+__device__ __forceinline__ int grid_cell(const EnvDev &E, float tx, float ty, float tz) {
+  const float fx = (tx - E.grid_o[0]) * E.grid_inv_h, fy = (ty - E.grid_o[1]) * E.grid_inv_h, fz = (tz - E.grid_o[2]) * E.grid_inv_h;
+  if (!(fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)E.grid_n[0] && fy < (float)E.grid_n[1] && fz < (float)E.grid_n[2]))
+    return -1;
+  return (int)(((unsigned)fz * (unsigned)E.grid_n[1] + (unsigned)fy) * (unsigned)E.grid_n[0] + (unsigned)fx);
+}
+
+template <int FMT, bool COUNT, bool PROBE>
 __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const PoseU &P,
                               const LanePose<FMT> &lp, int src, int lane, Tally &tally) {
   const RobotTri *srob = cs.rob;
@@ -632,10 +642,28 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
   PairCtx pc;
   if (COUNT) tally.past_root += 1;
 
+  // Contact probe: a pose that reaches phase B mostly collides, and mostly with one of its cell's two witnesses (the
+  // triangles that mark the cell nearest its centre).  The first pass of the loop below runs the triangle stage over them
+  // alone; a confirmed contact ends the pose without a walk, anything else walks from the root as if there were no probe.
+  // (The cell is derived again from the same Thi as in phase A: cheaper than holding it in a register through phase A.)
+  // The edge kernel is built without it (PROBE = false): its samples mostly share the swept-box candidate list, and the
+  // probe's code alone cost its per-sample loop 2 % of the edge rate in spills.
+  bool probe = false;
+  if (PROBE && E.witness) {
+    const int cell = grid_cell(E, P.Thi[0], P.Thi[1], P.Thi[2]);
+    if (cell >= 0) {
+      const int2 w = __ldg(E.witness + cell);
+      if (lane < 2) ws.tri[lane] = lane ? w.y : w.x;
+      ntri = (w.x >= 0) + (w.y >= 0);   // (w.y >= 0 only with w.x >= 0)
+      probe = ntri > 0;
+      __syncwarp();
+    }
+  }
+
   bool first = true;
   while (true) {
     // walk until a candidate triangle is pending, then run the triangle stage over what the last step found
-    if (first || (sp > 0 && ntri <= kTriCap - 32)) {
+    if (!probe && (first || (sp > 0 && ntri <= kTriCap - 32))) {
       const StepLeaves lv = walk_step<COUNT>(E, ws, cs, first, sp, lane, overlaps, tally);
       first = false;
       if (lv.mine) ws.tri[ntri + __popc(lv.mask & lt)] = lv.tri;
@@ -655,6 +683,10 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
     triangle_stage<FMT, COUNT>(E, ws, srob, P, lp, src, lane, ntri, hit, have_R2, pc, tally);
     if (hit) break;
     ntri = 0;
+    if (probe) {   // no contact with the witnesses: the walk starts (it may deliver them again, which is harmless)
+      probe = false;
+      continue;
+    }
     if (sp == 0) break;
   }
   return hit;
@@ -710,15 +742,6 @@ __device__ bool pose_hits_candidates(const EnvDev &E, WarpScratch &ws, const Cta
   return hit;
 }
 
-// The cell of the clearance grid that holds the robot origin, or -1 outside the grid.  A clear bit proves that no obstacle
-// triangle comes within the robot's bounding radius of any point of the cell (the build inflates the reach by the cell's
-// half diagonal plus rounding margins), so the pose is free whatever its orientation.
-__device__ __forceinline__ int grid_cell(const EnvDev &E, float tx, float ty, float tz) {
-  const float fx = (tx - E.grid_o[0]) * E.grid_inv_h, fy = (ty - E.grid_o[1]) * E.grid_inv_h, fz = (tz - E.grid_o[2]) * E.grid_inv_h;
-  if (!(fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)E.grid_n[0] && fy < (float)E.grid_n[1] && fz < (float)E.grid_n[2]))
-    return -1;
-  return (int)(((unsigned)fz * (unsigned)E.grid_n[1] + (unsigned)fy) * (unsigned)E.grid_n[0] + (unsigned)fx);
-}
 __device__ __forceinline__ bool cell_marked(const EnvDev &E, int cell) {
   return ((__ldg(E.clear_bits + (cell >> 5)) >> (cell & 31)) & 1u) != 0u;
 }
@@ -883,7 +906,7 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
       P.Tlo[k] = FMT == kFmtEulerF32 ? 0.f : __shfl_sync(kFull, tlo[k], src);
     }
     if (SWEPT_CAPABLE && ncand > 0 ? pose_hits_candidates<FMT, COUNT>(E, ws, cs, P, lp, src, lane, ncand, tally)
-                                   : warp_pose_hit<FMT, COUNT>(E, ws, cs, P, lp, src, lane, tally)) {
+                                   : warp_pose_hit<FMT, COUNT, !SWEPT_CAPABLE>(E, ws, cs, P, lp, src, lane, tally)) {
       hitmask |= 1u << src;
       if (first_only) break;
     }
@@ -1148,9 +1171,12 @@ __device__ __forceinline__ float dot_dir_rd(const float *m, const float *p) {
 // Marks (bits != null) the cells within `reach` of each triangle and lowers mins[j][cell] to the triangle's bound
 // min over its vertices of m_d.p, d = pass_dir(dir0, j) for j < ndir: the float vertices, rounded down, minus
 // |m|_1 times their representation error, so the bound holds for the FP64 triangle.
+// With `keys` (witness passes, ndir = 0) it lowers keys[cell] to (distance^2 bits, triangle) of every triangle that marks
+// the cell, except the cell's first witness `excl[cell].x` when `excl` is given.
 constexpr int kClearanceThreads = 256;
 __global__ void build_clearance_kernel(const float4 *__restrict__ tris, int n_tris, float ox, float oy, float oz, float h, int nx,
-                                       int ny, int nz, float reach, unsigned *bits, int *mins, int dir0, int ndir) {
+                                       int ny, int nz, float reach, unsigned *bits, int *mins, int dir0, int ndir,
+                                       unsigned long long *keys, const int2 *excl) {
   __shared__ int tri_min[kClearanceThreads / 32][32];
   const int lane = threadIdx.x & 31;
   const int t = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
@@ -1183,11 +1209,14 @@ __global__ void build_clearance_kernel(const float4 *__restrict__ tris, int n_tr
   for (long long i = lane; i < total; i += 32) {
     const int ix = lo[0] + (int)(i % sx), iy = lo[1] + (int)((i / sx) % sy), iz = lo[2] + (int)(i / ((long long)sx * sy));
     const float p[3] = {ox + (ix + 0.5f) * h, oy + (iy + 0.5f) * h, oz + (iz + 0.5f) * h};
-    if (!(point_tri_dist2(p, a, b, c) > r2)) {   // NaN (degenerate triangle) marks the cell: never optimistic
+    const float d2 = point_tri_dist2(p, a, b, c);
+    if (!(d2 > r2)) {   // NaN (degenerate triangle) marks the cell: never optimistic
       const unsigned cell = ((unsigned)iz * (unsigned)ny + (unsigned)iy) * (unsigned)nx + (unsigned)ix;
       if (bits) atomicOr(bits + (cell >> 5), 1u << (cell & 31));
       const size_t cells = (size_t)nx * ny * nz;
       for (int j = 0; j < ndir; ++j) atomicMin(mins + j * cells + cell, tmin[j]);
+      if (keys && !(excl && excl[cell].x == t))   // (d2 >= 0 or NaN: its bits order like the value, NaN last)
+        atomicMin(keys + cell, ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)t);
     }
   }
 }
@@ -1224,6 +1253,16 @@ __global__ void choose_planes_kernel(const unsigned *__restrict__ bits, const in
     }
   }
   planes[cell] = best;
+}
+
+// witness `slot` (0: .x, 1: .y) of every cell from the keys of its pass; a key left at ~0 (no triangle) gives -1
+__global__ void take_witness_kernel(const unsigned long long *__restrict__ keys, long long cells, int slot, int2 *witness) {
+  const long long cell = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (cell >= cells) return;
+  const unsigned long long k = keys[cell];
+  const int t = k == ~0ull ? -1 : (int)(unsigned)k;
+  if (slot == 0) witness[cell] = make_int2(t, -1);
+  else witness[cell].y = t;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1425,11 +1464,12 @@ cudaError_t launch_check_edges(const EnvDev &env_in, const double *d_starts, con
 }
 
 cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, unsigned *d_planes, int *d_scratch, size_t scratch_words, cudaStream_t stream) {
+                                   unsigned *d_bits, unsigned *d_planes, int2 *d_witness, int *d_scratch, size_t scratch_words,
+                                   cudaStream_t stream) {
   if (n_tris <= 0) return cudaSuccess;
   const size_t cells = (size_t)n[0] * n[1] * n[2];
   const int per_pass = (int)std::min<size_t>(26, scratch_words / cells);
-  if (per_pass < 1) return cudaErrorInvalidValue;
+  if (per_pass < 1 || (d_witness && scratch_words < 2 * cells)) return cudaErrorInvalidValue;
   const long long blocks = ((long long)n_tris * 32 + kClearanceThreads - 1) / kClearanceThreads;
   const long long cell_blocks = ((long long)cells + 255) / 256;
   for (int dir0 = 0; dir0 < 26; dir0 += per_pass) {
@@ -1438,9 +1478,20 @@ cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const flo
     if (e != cudaSuccess) return e;
     build_clearance_kernel<<<(unsigned)blocks, kClearanceThreads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h,
                                                                                 n[0], n[1], n[2], reach, dir0 == 0 ? d_bits : nullptr,
-                                                                                d_scratch, dir0, ndir);
+                                                                                d_scratch, dir0, ndir, nullptr, nullptr);
     choose_planes_kernel<<<(unsigned)cell_blocks, 256, 0, stream>>>(d_bits, d_scratch, n[0], n[1], n[2], origin[0], origin[1], origin[2],
                                                                    h, dir0, ndir, dir0 == 0, d_planes);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  // contact witnesses: pass 0 takes each cell's nearest triangle, pass 1 the nearest of the others
+  unsigned long long *keys = reinterpret_cast<unsigned long long *>(d_scratch);   // (cudaMalloc'd: 8-byte aligned)
+  for (int slot = 0; d_witness && slot < 2; ++slot) {
+    cudaError_t e = cudaMemsetAsync(keys, 0xff, cells * sizeof(unsigned long long), stream);
+    if (e != cudaSuccess) return e;
+    build_clearance_kernel<<<(unsigned)blocks, kClearanceThreads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h,
+                                                                                n[0], n[1], n[2], reach, nullptr, nullptr, 0, 0,
+                                                                                keys, slot ? d_witness : nullptr);
+    take_witness_kernel<<<(unsigned)cell_blocks, 256, 0, stream>>>(keys, (long long)cells, slot, d_witness);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
   }
   return cudaSuccess;

@@ -32,6 +32,9 @@ struct EnvDev {
   float plane_pad;              // absolute part of the plane test's margin, rounded up
   const float4 *rob_verts;      // distinct robot vertices (nearest floats); null above kPlaneVertCap: the robot box stands in
   int n_rob_verts;
+  // per grid cell, the two triangles (leaf order, -1 for none) that mark it with their points nearest the cell centre:
+  // phase B tries them before the walk (contact probe).  Null when the grid or the probe is off.
+  const int2 *witness;
   unsigned long long *counters; // 5 x u64 (may be null): poses, past_root, box_tests, pair_tests, exact_tests
   int *status;                  // device int, set non-zero on traversal-stack overflow
   unsigned int *work_counter;   // persistent-kernel work distribution: never reset, units are (fetched value - work_base)
@@ -98,8 +101,11 @@ constexpr int kStageNodesCap = SFFG_STAGE_NODES;
 // Marks every cell whose centre is within `reach` of an obstacle triangle (one warp per triangle) in `d_bits`, and picks
 // each marked cell's plane record (`d_planes`, one word per cell).  `d_scratch` holds `scratch_words` ints (at least one
 // per cell); the 26 plane directions take ceil(26 / (scratch_words / cells)) passes over the triangles.
+// With `d_witness` (one int2 per cell) it then stores each cell's two contact witnesses -- of the triangles that mark the cell,
+// the two nearest its centre -- in two more passes over the triangles; that needs scratch_words >= 2 * cells.
 cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, unsigned *d_planes, int *d_scratch, size_t scratch_words, cudaStream_t stream);
+                                   unsigned *d_bits, unsigned *d_planes, int2 *d_witness, int *d_scratch, size_t scratch_words,
+                                   cudaStream_t stream);
 
 // Robots with more distinct vertices than this take the support of their box in the plane test (robot_small has 8,
 // robot_cyl_small 64).  One FMA chain per vertex per pose past the grid bit.

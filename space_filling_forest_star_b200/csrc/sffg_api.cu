@@ -176,6 +176,7 @@ struct sffg_env {
   EnvDev dev{};
   DevPtr<ChildSlot> d_slots, d_top;
   DevPtr<unsigned> d_clear, d_planes;
+  DevPtr<int2> d_witness;
   DevPtr<float4> d_rob_verts;
   DevPtr<float4> d_tris32;
   DevPtr<double> d_tris64, d_robot64;
@@ -382,6 +383,7 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   env->d_top.reset();
   env->d_clear.reset();
   env->d_planes.reset();
+  env->d_witness.reset();
   SFFG_CUDA(upload(env->d_top, top.data(), top.size() * sizeof(ChildSlot), &bytes));
   d.n_obst = (int)n_obst;
   for (int k = 0; k < 3; ++k) {
@@ -392,6 +394,7 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   // ---- clearance grid (free-space bitmap) over the obstacle AABB dilated by the robot's reach
   d.clear_bits = nullptr;
   d.planes = nullptr;
+  d.witness = nullptr;
   d.plane_pad = 0.f;
   env->info.grid_cells = 0;
   env->info.grid_cell_size = 0;
@@ -424,17 +427,23 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
     // one plane word per cell; the per-direction bounds of the build live in a temporary block of at most 512 MB (one
     // pass over the triangles for grids up to 5.1 M cells, more passes above)
     SFFG_CUDA(dev_alloc(env->d_planes, cells * sizeof(unsigned)));
+    // two contact witnesses per cell (8 bytes), unless SFFG_WITNESS=0; their build keys take 2 ints per cell of the block
+    const char *witness_env = std::getenv("SFFG_WITNESS");
+    const bool witness = !(witness_env && witness_env[0] == '0');
+    if (witness) SFFG_CUDA(dev_alloc(env->d_witness, cells * sizeof(int2)));
     {
-      const size_t scratch_words = std::min<size_t>(26 * cells, std::max<size_t>(cells, size_t(1) << 27));
+      const size_t scratch_words = std::min<size_t>(26 * cells, std::max<size_t>(2 * cells, size_t(1) << 27));
       DevPtr<int> d_scratch;
       SFFG_CUDA(dev_alloc(d_scratch, scratch_words * sizeof(int)));
       SFFG_CUDA(launch_build_clearance(env->d_tris32.get(), (int)n_obst, go, (float)h, gn, (float)reach, env->d_clear.get(),
-                                       env->d_planes.get(), d_scratch.get(), scratch_words, env->streams[0].get()));
+                                       env->d_planes.get(), env->d_witness.get(), d_scratch.get(), scratch_words,
+                                       env->streams[0].get()));
       SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
     }
-    bytes += words * sizeof(unsigned) + cells * sizeof(unsigned);
+    bytes += words * sizeof(unsigned) + cells * sizeof(unsigned) + (witness ? cells * sizeof(int2) : 0);
     d.clear_bits = env->d_clear.get();
     d.planes = env->d_planes.get();
+    d.witness = env->d_witness.get();
     // absolute part of the plane test's margin (see plane_says_free): the grid's slack and 2^-15 rho for the rotated robot
     d.plane_pad = round_up_f32((1e-3 * h + maxc * 3.9e-6 + rho * std::ldexp(1.0, -15)) * 1.001);
     for (int k = 0; k < 3; ++k) {
