@@ -13,8 +13,8 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libsffg.so"
-SOURCES = ["sffg_api.cu", "collide_kernels.cu", "knn_kernels.cu", "knn_pruned.cu", "bvh_device.cu", "bvh_build.cpp", "mesh_loader.cpp"]
-HEADERS = ["common.h", "collide_kernels.cuh", "knn_kernels.cuh", "knn_common.cuh", "knn_pruned.cuh", "bvh_device.cuh", "../../include/sffg.h"]
+SOURCES = ["sffg_api.cu", "collide_kernels.cu", "clearance_grid.cu", "knn_kernels.cu", "knn_pruned.cu", "bvh_device.cu", "bvh_build.cpp", "mesh_loader.cpp"]
+HEADERS = ["common.h", "collide_kernels.cuh", "clearance_grid.cuh", "cuda_handles.h", "knn_kernels.cuh", "knn_common.cuh", "knn_pruned.cuh", "bvh_device.cuh", "../../include/sffg.h"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

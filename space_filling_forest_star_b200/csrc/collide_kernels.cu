@@ -619,16 +619,6 @@ __device__ __forceinline__ StepLeaves walk_step(const EnvDev &E, WarpScratch &ws
   return {m_leaf, ov && child < 0, ~child};
 }
 
-// The cell of the clearance grid that holds the robot origin, or -1 outside the grid.  A clear bit proves that no obstacle
-// triangle comes within the robot's bounding radius of any point of the cell (the build inflates the reach by the cell's
-// half diagonal plus rounding margins), so the pose is free whatever its orientation.
-__device__ __forceinline__ int grid_cell(const EnvDev &E, float tx, float ty, float tz) {
-  const float fx = (tx - E.grid_o[0]) * E.grid_inv_h, fy = (ty - E.grid_o[1]) * E.grid_inv_h, fz = (tz - E.grid_o[2]) * E.grid_inv_h;
-  if (!(fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)E.grid_n[0] && fy < (float)E.grid_n[1] && fz < (float)E.grid_n[2]))
-    return -1;
-  return (int)(((unsigned)fz * (unsigned)E.grid_n[1] + (unsigned)fy) * (unsigned)E.grid_n[0] + (unsigned)fx);
-}
-
 template <int FMT, bool COUNT, bool PROBE>
 __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const PoseU &P,
                               const LanePose<FMT> &lp, int src, int lane, Tally &tally) {
@@ -649,10 +639,10 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
   // The edge kernel is built without it (PROBE = false): its samples mostly share the swept-box candidate list, and the
   // probe's code alone cost its per-sample loop 2 % of the edge rate in spills.
   bool probe = false;
-  if (PROBE && E.witness) {
-    const int cell = grid_cell(E, P.Thi[0], P.Thi[1], P.Thi[2]);
+  if (PROBE && E.grid.witness) {
+    const int cell = grid_cell(E.grid, P.Thi[0], P.Thi[1], P.Thi[2]);
     if (cell >= 0) {
-      const int2 w = __ldg(E.witness + cell);
+      const int2 w = __ldg(E.grid.witness + cell);
       if (lane < 2) ws.tri[lane] = lane ? w.y : w.x;
       ntri = (w.x >= 0) + (w.y >= 0);   // (w.y >= 0 only with w.x >= 0)
       probe = ntri > 0;
@@ -742,18 +732,10 @@ __device__ bool pose_hits_candidates(const EnvDev &E, WarpScratch &ws, const Cta
   return hit;
 }
 
+// A clear bit proves that no obstacle triangle comes within the robot's bounding radius of any point of the cell (the
+// build inflates the reach by the cell's half diagonal plus rounding margins), so the pose is free whatever its orientation.
 __device__ __forceinline__ bool cell_marked(const EnvDev &E, int cell) {
-  return ((__ldg(E.clear_bits + (cell >> 5)) >> (cell & 31)) & 1u) != 0u;
-}
-
-// Plane directions: the 26 integer vectors m in {-1,0,1}^3 \ {0}, d = 9 (mz + 1) + 3 (my + 1) + (mx + 1); d = 13 (m = 0)
-// is the "no plane" record, whose offset is -FLT_MAX so that no pose passes it.
-constexpr int kNoPlaneDir = 13;
-constexpr unsigned kNoPlane = 0x80800000u | kNoPlaneDir;   // float_to_ordered(-FLT_MAX) = 0x80800000, low 5 bits clear
-__device__ __forceinline__ void plane_dir(int d, float *m) {
-  m[0] = (float)(d % 3 - 1);
-  m[1] = (float)(d / 3 % 3 - 1);
-  m[2] = (float)(d / 9 - 1);
+  return ((__ldg(E.grid.bits + (cell >> 5)) >> (cell & 31)) & 1u) != 0u;
 }
 
 // O(1) free-space test for a marked cell: its plane record `word` holds a direction m and an offset c with m.p >= c for every
@@ -769,8 +751,8 @@ __device__ __forceinline__ void plane_dir(int d, float *m) {
 //     moves by < 3 * 2^-17 rho + 12 * 2^-24 rho.  Allotted 2^-15 rho (plane_pad).
 //   - T = thi + tlo: |m.tlo| <= |tlo|_1, added as is; m.thi and the final sums round by < 2^-22 (|thi|_1 + 3 rho),
 //     allotted 2^-20 |thi|_1 (and the 2^-15 rho above).
-//   - the grid's absolute slack (1e-3 h + maxc * 3.9e-6, as in its reach), carried in plane_pad so that a plane never
-//     clears a pose that the grid's own rounding allowances would hold back.
+//   - the grid's absolute slack (stated once, in clearance_margins of clearance_grid.cu, which adds it to the reach too),
+//     carried in plane_pad so that a plane never clears a pose that the grid's own rounding allowances would hold back.
 // With these the robot stays below the plane by a positive gap in exact arithmetic, and the oracle's FP64 SAT finds
 // separated triangles separated -- the same ground the clear bit and the FP32 certificates stand on (DESIGN.md 4.1).
 __device__ __forceinline__ bool plane_says_free(const EnvDev &E, unsigned word, const float *R, const float *thi, float tlo_mag) {
@@ -792,7 +774,7 @@ __device__ __forceinline__ bool plane_says_free(const EnvDev &E, unsigned word, 
           fabsf(w2) * E.rob_h[2];
   }
   const float s = m[0] * thi[0] + m[1] * thi[1] + m[2] * thi[2] + sup;
-  const float margin = E.plane_pad + 9.5367431640625e-07f * (fabsf(thi[0]) + fabsf(thi[1]) + fabsf(thi[2])) + tlo_mag;
+  const float margin = E.grid.plane_pad + 9.5367431640625e-07f * (fabsf(thi[0]) + fabsf(thi[1]) + fabsf(thi[2])) + tlo_mag;
   return s + margin < c;
 }
 
@@ -862,10 +844,10 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
   const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
   bool alive = valid && E.n_obst > 0 && sphere_hits_root(E, thi[0], thi[1], thi[2], tlo_mag);
   unsigned plane = kNoPlane;   // (loaded before the rotation is built, which hides the load)
-  if (alive && E.grid_n[0] > 0) {
-    const int cell = grid_cell(E, thi[0], thi[1], thi[2]);
+  if (alive && E.grid.n[0] > 0) {
+    const int cell = grid_cell(E.grid, thi[0], thi[1], thi[2]);
     alive = cell < 0 || cell_marked(E, cell);
-    if (alive && cell >= 0) plane = __ldg(E.planes + cell);
+    if (alive && cell >= 0) plane = __ldg(E.grid.planes + cell);
   }
   if (alive) lp.rot32(R);
   if (alive && plane != kNoPlane) alive = !plane_says_free(E, plane, R, thi, tlo_mag);
@@ -1113,159 +1095,6 @@ __global__ void finalize_edges_kernel(const int *fh, long long m, uint8_t *free_
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// clearance grid build: one warp per obstacle triangle marks the cells whose centre lies within `reach` of the triangle
-// ---------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float point_tri_dist2(const float *p, const float *a, const float *b, const float *c) {
-  // closest point on a triangle (Voronoi-region walk), squared distance
-  const float ab[3] = {b[0] - a[0], b[1] - a[1], b[2] - a[2]}, ac[3] = {c[0] - a[0], c[1] - a[1], c[2] - a[2]};
-  const float ap[3] = {p[0] - a[0], p[1] - a[1], p[2] - a[2]};
-  const float d1 = ab[0] * ap[0] + ab[1] * ap[1] + ab[2] * ap[2], d2 = ac[0] * ap[0] + ac[1] * ap[1] + ac[2] * ap[2];
-  float q[3];
-  if (d1 <= 0.f && d2 <= 0.f) { q[0] = a[0]; q[1] = a[1]; q[2] = a[2]; }
-  else {
-    const float bp[3] = {p[0] - b[0], p[1] - b[1], p[2] - b[2]};
-    const float d3 = ab[0] * bp[0] + ab[1] * bp[1] + ab[2] * bp[2], d4 = ac[0] * bp[0] + ac[1] * bp[1] + ac[2] * bp[2];
-    if (d3 >= 0.f && d4 <= d3) { q[0] = b[0]; q[1] = b[1]; q[2] = b[2]; }
-    else {
-      const float vc = d1 * d4 - d3 * d2;
-      if (vc <= 0.f && d1 >= 0.f && d3 <= 0.f) {
-        const float v = d1 / (d1 - d3);
-        q[0] = a[0] + v * ab[0]; q[1] = a[1] + v * ab[1]; q[2] = a[2] + v * ab[2];
-      } else {
-        const float cp[3] = {p[0] - c[0], p[1] - c[1], p[2] - c[2]};
-        const float d5 = ab[0] * cp[0] + ab[1] * cp[1] + ab[2] * cp[2], d6 = ac[0] * cp[0] + ac[1] * cp[1] + ac[2] * cp[2];
-        if (d6 >= 0.f && d5 <= d6) { q[0] = c[0]; q[1] = c[1]; q[2] = c[2]; }
-        else {
-          const float vb = d5 * d2 - d1 * d6;
-          if (vb <= 0.f && d2 >= 0.f && d6 <= 0.f) {
-            const float w = d2 / (d2 - d6);
-            q[0] = a[0] + w * ac[0]; q[1] = a[1] + w * ac[1]; q[2] = a[2] + w * ac[2];
-          } else {
-            const float va = d3 * d6 - d5 * d4;
-            if (va <= 0.f && (d4 - d3) >= 0.f && (d5 - d6) >= 0.f) {
-              const float w = (d4 - d3) / ((d4 - d3) + (d5 - d6));
-              q[0] = b[0] + w * (c[0] - b[0]); q[1] = b[1] + w * (c[1] - b[1]); q[2] = b[2] + w * (c[2] - b[2]);
-            } else {
-              const float den = 1.f / (va + vb + vc), v = vb * den, w = vc * den;
-              q[0] = a[0] + ab[0] * v + ac[0] * w; q[1] = a[1] + ab[1] * v + ac[1] * w; q[2] = a[2] + ab[2] * v + ac[2] * w;
-            }
-          }
-        }
-      }
-    }
-  }
-  const float dx = p[0] - q[0], dy = p[1] - q[1], dz = p[2] - q[2];
-  return dx * dx + dy * dy + dz * dz;
-}
-
-// plane direction of pass slot j (the 26 directions skip d = 13)
-__device__ __forceinline__ int pass_dir(int dir0, int j) {
-  const int k = dir0 + j;
-  return k < kNoPlaneDir ? k : k + 1;
-}
-// m.p rounded down: m has entries in {-1, 0, 1}, so the products are exact and only the two sums round
-__device__ __forceinline__ float dot_dir_rd(const float *m, const float *p) {
-  return __fadd_rd(__fadd_rd(m[0] * p[0], m[1] * p[1]), m[2] * p[2]);
-}
-
-// Marks (bits != null) the cells within `reach` of each triangle and lowers mins[j][cell] to the triangle's bound
-// min over its vertices of m_d.p, d = pass_dir(dir0, j) for j < ndir: the float vertices, rounded down, minus
-// |m|_1 times their representation error, so the bound holds for the FP64 triangle.
-// With `keys` (witness passes, ndir = 0) it lowers keys[cell] to (distance^2 bits, triangle) of every triangle that marks
-// the cell, except the cell's first witness `excl[cell].x` when `excl` is given.
-constexpr int kClearanceThreads = 256;
-__global__ void build_clearance_kernel(const float4 *__restrict__ tris, int n_tris, float ox, float oy, float oz, float h, int nx,
-                                       int ny, int nz, float reach, unsigned *bits, int *mins, int dir0, int ndir,
-                                       unsigned long long *keys, const int2 *excl) {
-  __shared__ int tri_min[kClearanceThreads / 32][32];
-  const int lane = threadIdx.x & 31;
-  const int t = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-  if (t >= n_tris) return;
-  const float4 v0 = __ldg(tris + 3 * (size_t)t), v1 = __ldg(tris + 3 * (size_t)t + 1), v2 = __ldg(tris + 3 * (size_t)t + 2);
-  const float a[3] = {v0.x, v0.y, v0.z}, b[3] = {v1.x, v1.y, v1.z}, c[3] = {v2.x, v2.y, v2.z};
-  int *tmin = tri_min[threadIdx.x >> 5];
-  if (lane < ndir) {
-    float m[3];
-    plane_dir(pass_dir(dir0, lane), m);
-    const float l1 = fabsf(m[0]) + fabsf(m[1]) + fabsf(m[2]);
-    const float lo = fminf(dot_dir_rd(m, a), fminf(dot_dir_rd(m, b), dot_dir_rd(m, c)));
-    tmin[lane] = float_to_ordered(__fsub_rd(lo, __fmul_ru(l1, v0.w)));
-  }
-  __syncwarp();
-  const float inv = 1.0f / h;
-  int lo[3], hi[3];
-  const float o[3] = {ox, oy, oz};
-  const int n[3] = {nx, ny, nz};
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const float mn = fminf(a[k], fminf(b[k], c[k])) - reach, mx = fmaxf(a[k], fmaxf(b[k], c[k])) + reach;
-    lo[k] = max(0, (int)floorf((mn - o[k]) * inv) - 1);
-    hi[k] = min(n[k] - 1, (int)floorf((mx - o[k]) * inv) + 1);
-  }
-  const int sx = hi[0] - lo[0] + 1, sy = hi[1] - lo[1] + 1, sz = hi[2] - lo[2] + 1;
-  if (sx <= 0 || sy <= 0 || sz <= 0) return;
-  const long long total = (long long)sx * sy * sz;
-  const float r2 = reach * reach;
-  for (long long i = lane; i < total; i += 32) {
-    const int ix = lo[0] + (int)(i % sx), iy = lo[1] + (int)((i / sx) % sy), iz = lo[2] + (int)(i / ((long long)sx * sy));
-    const float p[3] = {ox + (ix + 0.5f) * h, oy + (iy + 0.5f) * h, oz + (iz + 0.5f) * h};
-    const float d2 = point_tri_dist2(p, a, b, c);
-    if (!(d2 > r2)) {   // NaN (degenerate triangle) marks the cell: never optimistic
-      const unsigned cell = ((unsigned)iz * (unsigned)ny + (unsigned)iy) * (unsigned)nx + (unsigned)ix;
-      if (bits) atomicOr(bits + (cell >> 5), 1u << (cell & 31));
-      const size_t cells = (size_t)nx * ny * nz;
-      for (int j = 0; j < ndir; ++j) atomicMin(mins + j * cells + cell, tmin[j]);
-      if (keys && !(excl && excl[cell].x == t))   // (d2 >= 0 or NaN: its bits order like the value, NaN last)
-        atomicMin(keys + cell, ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)t);
-    }
-  }
-}
-
-// Each marked cell keeps, of the directions of this pass and the record it already holds (`first`: none), the one with the
-// most room c - max_{x in cell} m.x per unit length of m -- what the robot's origin may use before it reaches the plane.
-// A record with no room at all is the no-plane record.  Unmarked cells get the no-plane record on the first pass.
-__global__ void choose_planes_kernel(const unsigned *__restrict__ bits, const int *__restrict__ mins, int nx, int ny, int nz,
-                                     float ox, float oy, float oz, float h, int dir0, int ndir, bool first, unsigned *planes) {
-  const long long cells = (long long)nx * ny * nz;
-  const long long cell = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (cell >= cells) return;
-  if (!((__ldg(bits + (cell >> 5)) >> (cell & 31)) & 1u)) {
-    if (first) planes[cell] = kNoPlane;
-    return;
-  }
-  const int ix = (int)(cell % nx), iy = (int)(cell / nx % ny), iz = (int)(cell / ((long long)nx * ny));
-  const float p[3] = {ox + (ix + 0.5f) * h, oy + (iy + 0.5f) * h, oz + (iz + 0.5f) * h};
-  const auto room = [&](int d, float c) {
-    float m[3];
-    plane_dir(d, m);
-    const float l1 = fabsf(m[0]) + fabsf(m[1]) + fabsf(m[2]);
-    return (c - (m[0] * p[0] + m[1] * p[1] + m[2] * p[2] + 0.5f * h * l1)) * rsqrtf(l1);
-  };
-  unsigned best = first ? kNoPlane : planes[cell];
-  float best_room = (best & 31u) == kNoPlaneDir ? 0.f : room((int)(best & 31u), ordered_to_float((int)(best & ~31u)));
-  for (int j = 0; j < ndir; ++j) {
-    const int d = pass_dir(dir0, j);
-    const int o = __ldg(mins + j * cells + cell);
-    const float r = room(d, ordered_to_float(o));
-    if (r > best_room) {
-      best_room = r;
-      best = ((unsigned)o & ~31u) | (unsigned)d;   // clearing low bits of an ordered int rounds the offset down
-    }
-  }
-  planes[cell] = best;
-}
-
-// witness `slot` (0: .x, 1: .y) of every cell from the keys of its pass; a key left at ~0 (no triangle) gives -1
-__global__ void take_witness_kernel(const unsigned long long *__restrict__ keys, long long cells, int slot, int2 *witness) {
-  const long long cell = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (cell >= cells) return;
-  const unsigned long long k = keys[cell];
-  const int t = k == ~0ull ? -1 : (int)(unsigned)k;
-  if (slot == 0) witness[cell] = make_int2(t, -1);
-  else witness[cell].y = t;
-}
-
-// ---------------------------------------------------------------------------------------------------------
 // synthetic pose stream: Philox4x32-10, bit-identical to oracle/sff_oracle.c::orc_gen_poses
 // ---------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void philox10(unsigned long long seed, unsigned long long index, unsigned stream, unsigned *o) {
@@ -1461,40 +1290,6 @@ cudaError_t launch_check_edges(const EnvDev &env_in, const double *d_starts, con
     e = cudaGetLastError();
   }
   return e;
-}
-
-cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, unsigned *d_planes, int2 *d_witness, int *d_scratch, size_t scratch_words,
-                                   cudaStream_t stream) {
-  if (n_tris <= 0) return cudaSuccess;
-  const size_t cells = (size_t)n[0] * n[1] * n[2];
-  const int per_pass = (int)std::min<size_t>(26, scratch_words / cells);
-  if (per_pass < 1 || (d_witness && scratch_words < 2 * cells)) return cudaErrorInvalidValue;
-  const long long blocks = ((long long)n_tris * 32 + kClearanceThreads - 1) / kClearanceThreads;
-  const long long cell_blocks = ((long long)cells + 255) / 256;
-  for (int dir0 = 0; dir0 < 26; dir0 += per_pass) {
-    const int ndir = std::min(per_pass, 26 - dir0);
-    cudaError_t e = cudaMemsetAsync(d_scratch, 0x7f, (size_t)ndir * cells * sizeof(int), stream);
-    if (e != cudaSuccess) return e;
-    build_clearance_kernel<<<(unsigned)blocks, kClearanceThreads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h,
-                                                                                n[0], n[1], n[2], reach, dir0 == 0 ? d_bits : nullptr,
-                                                                                d_scratch, dir0, ndir, nullptr, nullptr);
-    choose_planes_kernel<<<(unsigned)cell_blocks, 256, 0, stream>>>(d_bits, d_scratch, n[0], n[1], n[2], origin[0], origin[1], origin[2],
-                                                                   h, dir0, ndir, dir0 == 0, d_planes);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  }
-  // contact witnesses: pass 0 takes each cell's nearest triangle, pass 1 the nearest of the others
-  unsigned long long *keys = reinterpret_cast<unsigned long long *>(d_scratch);   // (cudaMalloc'd: 8-byte aligned)
-  for (int slot = 0; d_witness && slot < 2; ++slot) {
-    cudaError_t e = cudaMemsetAsync(keys, 0xff, cells * sizeof(unsigned long long), stream);
-    if (e != cudaSuccess) return e;
-    build_clearance_kernel<<<(unsigned)blocks, kClearanceThreads, 0, stream>>>(d_tris32, n_tris, origin[0], origin[1], origin[2], h,
-                                                                                n[0], n[1], n[2], reach, nullptr, nullptr, 0, 0,
-                                                                                keys, slot ? d_witness : nullptr);
-    take_witness_kernel<<<(unsigned)cell_blocks, 256, 0, stream>>>(keys, (long long)cells, slot, d_witness);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  }
-  return cudaSuccess;
 }
 
 cudaError_t launch_gen_poses(uint64_t seed, uint64_t first, int64_t n, const float range[6], float *d_out,

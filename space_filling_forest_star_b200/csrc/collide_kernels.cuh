@@ -6,6 +6,59 @@
 
 namespace sffg {
 
+// Device view of the clearance grid (built by clearance_grid.cu): n[0] * n[1] * n[2] cubic cells of edge h from the
+// corner o, cell (ix, iy, iz) at index (iz * n[1] + iy) * n[0] + ix.  n[0] == 0 means "no grid": every other field is
+// then unset.
+//   bits     1 bit per cell: set when some obstacle triangle may lie within the robot's bounding radius of a robot origin
+//            in the cell; clear proves every pose with its origin in the cell collision free
+//   planes   1 word per cell: a separating-plane record (direction index in the low 5 bits, offset above them, see
+//            plane_says_free); kNoPlane for unmarked cells
+//   witness  1 int2 per cell: the two triangles (leaf order, -1 for none) that mark the cell with their points nearest
+//            its centre, which phase B tries before the walk (contact probe); null when the probe is off
+//   plane_pad  absolute part of the plane test's margin, rounded up (see clearance_margins in clearance_grid.cu)
+// (The fields the pose kernels read keep the order they had as loose EnvDev fields: that order leaves their code as it was.)
+struct GridDev {
+  const unsigned *bits;
+  float o[3];
+  float inv_h;   // float(1 / h), rounded from double
+  int n[3];
+  const unsigned *planes;
+  float plane_pad;
+  float h;
+  const int2 *witness;
+};
+
+__host__ __device__ __forceinline__ long long cell_count(const GridDev &g) { return (long long)g.n[0] * g.n[1] * g.n[2]; }
+// The index of cell (ix, iy, iz).
+__device__ __forceinline__ unsigned cell_index(const GridDev &g, unsigned ix, unsigned iy, unsigned iz) {
+  return (iz * (unsigned)g.n[1] + iy) * (unsigned)g.n[0] + ix;
+}
+// The cell that holds position (x, y, z), or -1 outside the grid.
+__device__ __forceinline__ int grid_cell(const GridDev &g, float x, float y, float z) {
+  const float fx = (x - g.o[0]) * g.inv_h, fy = (y - g.o[1]) * g.inv_h, fz = (z - g.o[2]) * g.inv_h;
+  if (!(fx >= 0.f && fy >= 0.f && fz >= 0.f && fx < (float)g.n[0] && fy < (float)g.n[1] && fz < (float)g.n[2])) return -1;
+  return (int)cell_index(g, (unsigned)fx, (unsigned)fy, (unsigned)fz);
+}
+// The centre of cell (ix, iy, iz), and of the cell at `cell`.
+__device__ __forceinline__ void cell_centre(const GridDev &g, int ix, int iy, int iz, float p[3]) {
+  p[0] = g.o[0] + (ix + 0.5f) * g.h;
+  p[1] = g.o[1] + (iy + 0.5f) * g.h;
+  p[2] = g.o[2] + (iz + 0.5f) * g.h;
+}
+__device__ __forceinline__ void cell_centre(const GridDev &g, long long cell, float p[3]) {
+  cell_centre(g, (int)(cell % g.n[0]), (int)(cell / g.n[0] % g.n[1]), (int)(cell / ((long long)g.n[0] * g.n[1])), p);
+}
+
+// Plane records: the 26 integer directions m in {-1,0,1}^3 \ {0}, d = 9 (mz + 1) + 3 (my + 1) + (mx + 1); d = 13 (m = 0)
+// is the "no plane" record, whose offset is -FLT_MAX so that no pose passes it.
+constexpr int kNoPlaneDir = 13;
+constexpr unsigned kNoPlane = 0x80800000u | kNoPlaneDir;   // float_to_ordered(-FLT_MAX) = 0x80800000, low 5 bits clear
+__device__ __forceinline__ void plane_dir(int d, float *m) {
+  m[0] = (float)(d % 3 - 1);
+  m[1] = (float)(d / 3 % 3 - 1);
+  m[2] = (float)(d / 9 - 1);
+}
+
 struct EnvDev {
   const float4 *slots;      // 2 float4 per child slot, kWide slots per node
   const float4 *top;        // <= 32 slots: a cut through the top of the hierarchy, tested by all lanes in step 0
@@ -20,21 +73,9 @@ struct EnvDev {
   float root_c[3], root_h[3];   // obstacle AABB, centre / half extents (outward rounded)
   float rob_c[3], rob_h[3];     // robot AABB in the robot frame (outward rounded)
   float rob_radius;             // max |robot vertex| about the robot origin (rounded up)
-  // free-space (clearance) grid: bit = 1 -> some obstacle triangle may be within rob_radius of a robot origin placed in
-  // that cell; bit = 0 -> every pose with its origin in the cell is collision free.  grid_n[0] == 0 disables it.
-  const unsigned *clear_bits;
-  float grid_o[3];
-  float grid_inv_h;
-  int grid_n[3];
-  // one separating plane per grid cell (word = direction index in the low 5 bits, offset above them, see plane_says_free),
-  // set whenever clear_bits is
-  const unsigned *planes;
-  float plane_pad;              // absolute part of the plane test's margin, rounded up
+  GridDev grid;                 // clearance grid over the obstacle AABB dilated by rob_radius
   const float4 *rob_verts;      // distinct robot vertices (nearest floats); null above kPlaneVertCap: the robot box stands in
   int n_rob_verts;
-  // per grid cell, the two triangles (leaf order, -1 for none) that mark it with their points nearest the cell centre:
-  // phase B tries them before the walk (contact probe).  Null when the grid or the probe is off.
-  const int2 *witness;
   unsigned long long *counters; // 5 x u64 (may be null): poses, past_root, box_tests, pair_tests, exact_tests
   int *status;                  // device int, set non-zero on traversal-stack overflow
   unsigned int *work_counter;   // persistent-kernel work distribution: never reset, units are (fetched value - work_base)
@@ -97,15 +138,6 @@ size_t collide_smem_bytes(int n_robot, int n_stage_max);
 #define SFFG_STAGE_NODES 73
 #endif
 constexpr int kStageNodesCap = SFFG_STAGE_NODES;
-
-// Marks every cell whose centre is within `reach` of an obstacle triangle (one warp per triangle) in `d_bits`, and picks
-// each marked cell's plane record (`d_planes`, one word per cell).  `d_scratch` holds `scratch_words` ints (at least one
-// per cell); the 26 plane directions take ceil(26 / (scratch_words / cells)) passes over the triangles.
-// With `d_witness` (one int2 per cell) it then stores each cell's two contact witnesses -- of the triangles that mark the cell,
-// the two nearest its centre -- in two more passes over the triangles; that needs scratch_words >= 2 * cells.
-cudaError_t launch_build_clearance(const float4 *d_tris32, int n_tris, const float origin[3], float h, const int n[3], float reach,
-                                   unsigned *d_bits, unsigned *d_planes, int2 *d_witness, int *d_scratch, size_t scratch_words,
-                                   cudaStream_t stream);
 
 // Robots with more distinct vertices than this take the support of their box in the plane test (robot_small has 8,
 // robot_cyl_small 64).  One FMA chain per vertex per pose past the grid bit.

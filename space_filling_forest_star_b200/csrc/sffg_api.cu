@@ -12,12 +12,13 @@
 #include <limits>
 #include <memory>
 #include <string>
-#include <type_traits>
 #include <vector>
 
 #include "bvh_device.cuh"
+#include "clearance_grid.cuh"
 #include "collide_kernels.cuh"
 #include "common.h"
+#include "cuda_handles.h"
 #include "knn_kernels.cuh"
 #include "knn_pruned.cuh"
 
@@ -84,35 +85,6 @@ cudaError_t upload_async(void *dst, const void *src, size_t bytes, unsigned char
   return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
 }
 
-// owners of CUDA resources: released when the owning object goes away
-struct CudaFree { void operator()(void *p) const { cudaFree(p); } };
-struct CudaFreeHost { void operator()(void *p) const { cudaFreeHost(p); } };
-struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
-struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
-template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;
-template <class T> using PinnedPtr = std::unique_ptr<T, CudaFreeHost>;   // cudaHostAllocMapped
-using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
-using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
-
-// hands the handle that `create` writes to the owner, once the call has succeeded
-template <class Owner, class Create> cudaError_t make(Owner &o, Create create) {
-  typename Owner::pointer h = nullptr;
-  const cudaError_t e = create(&h);
-  if (e == cudaSuccess) o.reset(h);
-  return e;
-}
-template <class T> cudaError_t dev_alloc(DevPtr<T> &o, size_t bytes) {
-  return make(o, [&](T **p) { return cudaMalloc(p, bytes); });
-}
-template <class T> cudaError_t host_alloc(PinnedPtr<T> &o, size_t bytes) {
-  return make(o, [&](T **p) { return cudaHostAlloc(p, bytes, cudaHostAllocMapped); });
-}
-cudaError_t make_stream(Stream &o) {
-  return make(o, [](cudaStream_t *s) { return cudaStreamCreateWithFlags(s, cudaStreamNonBlocking); });
-}
-cudaError_t make_event(Event &o) {
-  return make(o, [](cudaEvent_t *e) { return cudaEventCreateWithFlags(e, cudaEventDisableTiming); });
-}
 // a device copy of `n` bytes of host data (at least 16 bytes allocated); adds `n` to *counted
 template <class T> cudaError_t upload(DevPtr<T> &dst, const void *src, size_t n, size_t *counted) {
   cudaError_t e = dev_alloc(dst, std::max<size_t>(n, 16));
@@ -175,8 +147,7 @@ using namespace sffg;
 struct sffg_env {
   EnvDev dev{};
   DevPtr<ChildSlot> d_slots, d_top;
-  DevPtr<unsigned> d_clear, d_planes;
-  DevPtr<int2> d_witness;
+  ClearanceGrid grid;
   DevPtr<float4> d_rob_verts;
   DevPtr<float4> d_tris32;
   DevPtr<double> d_tris64, d_robot64;
@@ -381,9 +352,6 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
                             int64_t n_obst, int64_t n_nodes, int depth, bool on_device, size_t bytes) {
   EnvDev &d = env->dev;
   env->d_top.reset();
-  env->d_clear.reset();
-  env->d_planes.reset();
-  env->d_witness.reset();
   SFFG_CUDA(upload(env->d_top, top.data(), top.size() * sizeof(ChildSlot), &bytes));
   d.n_obst = (int)n_obst;
   for (int k = 0; k < 3; ++k) {
@@ -391,69 +359,15 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
     d.root_c[k] = (float)oc;
     d.root_h[k] = n_obst ? round_up_f32(std::max(root_hi[k] - (double)d.root_c[k], (double)d.root_c[k] - root_lo[k]) * 1.0000001) : 0.f;
   }
-  // ---- clearance grid (free-space bitmap) over the obstacle AABB dilated by the robot's reach
-  d.clear_bits = nullptr;
-  d.planes = nullptr;
-  d.witness = nullptr;
-  d.plane_pad = 0.f;
-  env->info.grid_cells = 0;
-  env->info.grid_cell_size = 0;
-  d.grid_n[0] = d.grid_n[1] = d.grid_n[2] = 0;
-  d.grid_inv_h = 0.f;
-  d.grid_o[0] = d.grid_o[1] = d.grid_o[2] = 0.f;
-  const char *grid_env = std::getenv("SFFG_CLEARANCE_GRID");
-  if (n_obst > 0 && !(grid_env && grid_env[0] == '0')) {
-    const double rho = d.rob_radius;
-    double h = rho / 4.0;
-    double ext[3], maxc = 0;
-    for (int k = 0; k < 3; ++k) {
-      ext[k] = (root_hi[k] - root_lo[k]) + 2.0 * rho;
-      maxc = std::max({maxc, std::fabs(root_lo[k]) + rho, std::fabs(root_hi[k]) + rho});
-    }
-    // cap the grid at 2^24 cells (2 MB of bits, L2-resident)
-    while ((ext[0] / h + 1) * (ext[1] / h + 1) * (ext[2] / h + 1) > double(1 << 24)) h *= 1.25;
-    int gn[3];
-    float go[3];
-    for (int k = 0; k < 3; ++k) {
-      go[k] = (float)(root_lo[k] - rho);
-      gn[k] = std::max(1, (int)std::ceil(ext[k] / h));
-    }
-    // reach = bounding radius + half cell diagonal + margins for float rounding of vertices, cell lookup and distances
-    const double reach = (rho + 0.8661 * h) * 1.002 + 1e-3 * h + maxc * 3.9e-6;
-    const size_t cells = (size_t)gn[0] * gn[1] * gn[2];
-    const size_t words = (cells + 31) / 32;
-    SFFG_CUDA(dev_alloc(env->d_clear, words * sizeof(unsigned)));
-    SFFG_CUDA(cudaMemset(env->d_clear.get(), 0, words * sizeof(unsigned)));
-    // one plane word per cell; the per-direction bounds of the build live in a temporary block of at most 512 MB (one
-    // pass over the triangles for grids up to 5.1 M cells, more passes above)
-    SFFG_CUDA(dev_alloc(env->d_planes, cells * sizeof(unsigned)));
-    // two contact witnesses per cell (8 bytes), unless SFFG_WITNESS=0; their build keys take 2 ints per cell of the block
-    const char *witness_env = std::getenv("SFFG_WITNESS");
-    const bool witness = !(witness_env && witness_env[0] == '0');
-    if (witness) SFFG_CUDA(dev_alloc(env->d_witness, cells * sizeof(int2)));
-    {
-      const size_t scratch_words = std::min<size_t>(26 * cells, std::max<size_t>(2 * cells, size_t(1) << 27));
-      DevPtr<int> d_scratch;
-      SFFG_CUDA(dev_alloc(d_scratch, scratch_words * sizeof(int)));
-      SFFG_CUDA(launch_build_clearance(env->d_tris32.get(), (int)n_obst, go, (float)h, gn, (float)reach, env->d_clear.get(),
-                                       env->d_planes.get(), env->d_witness.get(), d_scratch.get(), scratch_words,
-                                       env->streams[0].get()));
-      SFFG_CUDA(cudaStreamSynchronize(env->streams[0].get()));
-    }
-    bytes += words * sizeof(unsigned) + cells * sizeof(unsigned) + (witness ? cells * sizeof(int2) : 0);
-    d.clear_bits = env->d_clear.get();
-    d.planes = env->d_planes.get();
-    d.witness = env->d_witness.get();
-    // absolute part of the plane test's margin (see plane_says_free): the grid's slack and 2^-15 rho for the rotated robot
-    d.plane_pad = round_up_f32((1e-3 * h + maxc * 3.9e-6 + rho * std::ldexp(1.0, -15)) * 1.001);
-    for (int k = 0; k < 3; ++k) {
-      d.grid_o[k] = go[k];
-      d.grid_n[k] = gn[k];
-    }
-    d.grid_inv_h = (float)(1.0 / h);
-    env->info.grid_cells = (int64_t)gn[0] * gn[1] * gn[2];
-    env->info.grid_cell_size = h;
-  }
+  // the old grid goes before the new one is built, so that a set or refit never holds two
+  env->grid = ClearanceGrid();
+  const cudaError_t grid_err = build_clearance_grid(env->d_tris32.get(), n_obst, root_lo, root_hi, d.rob_radius, env->streams[0].get(),
+                                                    &env->grid);
+  d.grid = env->grid.view;   // no grid unless the build succeeded
+  env->info.grid_cells = env->grid.cells;
+  env->info.grid_cell_size = env->grid.h;
+  if (grid_err != cudaSuccess) return fail(SFFG_ERR_CUDA, std::string("clearance grid build: ") + cudaGetErrorString(grid_err));
+  bytes += env->grid.bytes;
   d.slots = reinterpret_cast<const float4 *>(env->d_slots.get());
   d.top = reinterpret_cast<const float4 *>(env->d_top.get());
   d.n_top = (int)top.size();

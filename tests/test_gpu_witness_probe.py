@@ -141,3 +141,24 @@ def test_probe_skips_most_of_the_walk(sff, orc, meshes, three_envs):
         per_pose.append(c["traversal_steps"] / c["poses_past_grid"])
     np.testing.assert_array_equal(verdicts[0], verdicts[1])
     assert per_pose[0] <= MAX_STEPS_RATIO * per_pose[1], per_pose
+
+
+# (grid_cells, grid_cell_size, device_bytes) of the bench environment and of the 2-D map under each switch setting, as
+# reported by the build before the grid's sizing moved into clearance_grid.cu: no test fixed the sizing before that.
+GRID_SIZING = {
+    ("B", None): (2798432, 0.6927118897438049, 39352620),
+    ("B", "SFFG_WITNESS"): (2798432, 0.6927118897438049, 16965164),
+    ("B", "SFFG_CLEARANCE_GRID"): (0, 0.0, 5421632),
+    ("2D", None): (8632224, 0.4128884789622589, 104695876),
+    ("2D", "SFFG_WITNESS"): (8632224, 0.4128884789622589, 35638084),
+    ("2D", "SFFG_CLEARANCE_GRID"): (0, 0.0, 30160),
+}
+
+
+@pytest.mark.parametrize("case,switch", list(GRID_SIZING))
+def test_grid_sizing(sff, meshes, monkeypatch, case, switch):
+    on, rn, _ = CASES[case]
+    if switch:
+        monkeypatch.setenv(switch, "0")
+    info = sff.Environment(meshes[on], meshes[rn]).info
+    assert (info["grid_cells"], info["grid_cell_size"], info["device_bytes"]) == GRID_SIZING[case, switch]

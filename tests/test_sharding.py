@@ -1,5 +1,4 @@
 """world_size-2 gloo test of the multi-GPU host logic (split -> local compute -> one all-gather)."""
-import os
 import sys
 from pathlib import Path
 
@@ -24,10 +23,14 @@ def test_shard_bounds_cover_everything():
             assert seen == n
 
 
-def _worker(rank, world, port, n, tmp):
+def _init_gloo(rank, world, tmp):
+    """rendezvous through a file in the test's own directory: no TCP port to pick, so no port another process may hold"""
     sys.path.insert(0, str(ROOT))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    dist.init_process_group("gloo", rank=rank, world_size=world)
+    dist.init_process_group("gloo", init_method=Path(tmp, "rendezvous").resolve().as_uri(), rank=rank, world_size=world)
+
+
+def _worker(rank, world, n, tmp):
+    _init_gloo(rank, world, tmp)
     from space_filling_forest_star_b200.sharding import shard_bounds, sharded_rows
     poses = torch.arange(n * 6, dtype=torch.float32).reshape(n, 6)
 
@@ -52,8 +55,7 @@ def _worker(rank, world, port, n, tmp):
 
 @pytest.mark.parametrize("n", [0, 5, 64, 1001])
 def test_sharded_rows_gloo_world2(tmp_path, n):
-    port = 29500 + (os.getpid() + n) % 2000
-    mp.spawn(_worker, args=(2, port, n, str(tmp_path)), nprocs=2, join=True)
+    mp.spawn(_worker, args=(2, n, str(tmp_path)), nprocs=2, join=True)
     assert (tmp_path / "ok0").read_text() == "True" and (tmp_path / "ok1").read_text() == "True"
 
 
@@ -66,10 +68,8 @@ class _FakeIndex:
         d2_out.copy_(queries[:, 1:2] + torch.arange(k, dtype=torch.float32)[None, :])
 
 
-def _knn_worker(rank, world, port, nq, k, tmp):
-    sys.path.insert(0, str(ROOT))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    dist.init_process_group("gloo", rank=rank, world_size=world)
+def _knn_worker(rank, world, nq, k, tmp):
+    _init_gloo(rank, world, tmp)
     from space_filling_forest_star_b200.sharding import sharded_knn
     q = torch.stack([torch.arange(nq, dtype=torch.float32), torch.arange(nq, dtype=torch.float32) * 0.5], 1).contiguous()
     ids, d2 = sharded_knn(_FakeIndex(), q, k)
@@ -83,8 +83,7 @@ def _knn_worker(rank, world, port, nq, k, tmp):
 @pytest.mark.parametrize("nq", [0, 1, 7, 64, 1001])
 def test_sharded_knn_in_place_gather_gloo_world2(tmp_path, nq):
     """the search writes its rows into its slice of the gathered buffers and the all-gathers run in place on them"""
-    port = 31500 + (os.getpid() + nq) % 2000
-    mp.spawn(_knn_worker, args=(2, port, nq, 5, str(tmp_path)), nprocs=2, join=True)
+    mp.spawn(_knn_worker, args=(2, nq, 5, str(tmp_path)), nprocs=2, join=True)
     assert (tmp_path / "ok0").read_text() == "True" and (tmp_path / "ok1").read_text() == "True"
 
 
@@ -101,11 +100,9 @@ class _FakeRadiusIndex:
         return cnt, off, ids, d2
 
 
-def _radius_worker(rank, world, port, nq, tmp):
+def _radius_worker(rank, world, nq, tmp):
     import numpy as np
-    sys.path.insert(0, str(ROOT))
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    dist.init_process_group("gloo", rank=rank, world_size=world)
+    _init_gloo(rank, world, tmp)
     from space_filling_forest_star_b200.sharding import sharded_radius
     q = np.stack([np.arange(nq, dtype=np.float32) * 3 + 1, np.zeros(nq, dtype=np.float32)], 1)
     counts, offsets, ids, d2 = sharded_radius(_FakeRadiusIndex(), q, 2.0)
@@ -119,6 +116,5 @@ def _radius_worker(rank, world, port, nq, tmp):
 @pytest.mark.parametrize("nq", [0, 1, 2, 9, 500])
 def test_sharded_radius_variable_rows_gloo_world2(tmp_path, nq):
     """counts first, then the packed rows padded to the largest per-rank total; every rank ends with the whole CSR result"""
-    port = 33500 + (os.getpid() + nq) % 2000
-    mp.spawn(_radius_worker, args=(2, port, nq, str(tmp_path)), nprocs=2, join=True)
+    mp.spawn(_radius_worker, args=(2, nq, str(tmp_path)), nprocs=2, join=True)
     assert (tmp_path / "ok0").read_text() == "True" and (tmp_path / "ok1").read_text() == "True"
