@@ -54,6 +54,8 @@ SIGNATURES = {
     "sffg_collide_poses_f64": (C.c_int, [_p, _p, C.c_int64, _p]),
     "sffg_collide_transforms_f64": (C.c_int, [_p, _p, C.c_int64, _p]),
     "sffg_collide_poses_device": (C.c_int, [_p, _p, C.c_int, C.c_int64, _p, _p]),
+    "sffg_distance_poses": (C.c_int, [_p, _p, C.c_int, C.c_int64, C.c_double, _p, _p]),
+    "sffg_distance_poses_device": (C.c_int, [_p, _p, C.c_int, C.c_int64, C.c_double, _p, _p, _p]),
     "sffg_peer_buffer_create": (C.c_int, [C.c_int64, C.POINTER(_p), _p]),
     "sffg_peer_buffer_open": (C.c_int, [_p, C.POINTER(_p)]),
     "sffg_peer_buffer_close": (C.c_int, [_p]),

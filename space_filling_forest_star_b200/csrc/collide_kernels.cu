@@ -26,6 +26,8 @@
 #include <cstdint>
 #include <mutex>
 
+#include <math_constants.h>
+
 #include "collide_kernels.cuh"
 
 namespace sffg {
@@ -1143,6 +1145,322 @@ __global__ void gen_poses_kernel(unsigned long long seed, unsigned long long fir
   o[5] = __fadd_rn(-3.14159274f, __fmul_rn(u01(b[2]), 6.28318548f));
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// separation distance per pose (sffg_distance_poses).  Contact is decided by check_32_poses, the verdict path itself; a
+// free pose then runs a branch-and-bound walk of the hierarchy whose bound `best` starts at max_dist and shrinks with every
+// triangle pair evaluated in FP64.  Every cull below is a rigorous lower bound on a distance, so nothing nearer than the
+// final `best` is ever dropped and the result is the minimum over all pairs, whatever the hierarchy.
+// ---------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ double ddiv(double a, double b) { return __ddiv_rn(a, b); }
+__device__ __forceinline__ double clamp01(double x) { return fmin(fmax(x, 0.0), 1.0); }
+__device__ __forceinline__ double dist2(const double *a, const double *b) {
+  const double d[3] = {dsub(a[0], b[0]), dsub(a[1], b[1]), dsub(a[2], b[2])};
+  return ddot(d, d);
+}
+
+// closest points a on [p0, p0 + d1] and b on [q0, q0 + d2] (Ericson, Real-Time Collision Detection 5.1.9, with exact
+// zero tests for degenerate segments); returns |a - b|^2
+__device__ double seg_seg(const double *p0, const double *d1, const double *q0, const double *d2, double *a, double *b) {
+  const double r[3] = {dsub(p0[0], q0[0]), dsub(p0[1], q0[1]), dsub(p0[2], q0[2])};
+  const double A = ddot(d1, d1), E = ddot(d2, d2), F = ddot(d2, r);
+  double s = 0.0, t = 0.0;
+  if (A == 0.0) {
+    if (E != 0.0) t = clamp01(ddiv(F, E));
+  } else {
+    const double C = ddot(d1, r);
+    if (E == 0.0) {
+      s = clamp01(ddiv(-C, A));
+    } else {
+      const double B = ddot(d1, d2);
+      const double den = dsub(dmul(A, E), dmul(B, B));
+      s = den != 0.0 ? clamp01(ddiv(dsub(dmul(B, F), dmul(C, E)), den)) : 0.0;
+      t = ddiv(dadd(dmul(B, s), F), E);
+      if (t < 0.0) {
+        t = 0.0;
+        s = clamp01(ddiv(-C, A));
+      } else if (t > 1.0) {
+        t = 1.0;
+        s = clamp01(ddiv(dsub(B, C), A));
+      }
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    a[k] = dadd(p0[k], dmul(d1[k], s));
+    b[k] = dadd(q0[k], dmul(d2[k], t));
+  }
+  return dist2(a, b);
+}
+
+// foot b of x on the plane of triangle c (9 doubles) when it lies inside the triangle; returns |x - b|^2, or +inf when the
+// foot lies outside or the triangle has no area (an edge term of the pair then bounds the distance from below)
+__device__ double point_face(const double *x, const double *c, double *b) {
+  double u[3], v[3], n[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) { u[k] = dsub(c[3 + k], c[k]); v[k] = dsub(c[6 + k], c[k]); b[k] = x[k]; }
+  dcross(n, u, v);
+  const double nn = ddot(n, n);
+  if (nn == 0.0) return CUDART_INF;
+#pragma unroll
+  for (int e = 0; e < 3; ++e) {
+    const double *c0 = c + 3 * e, *c1 = c + 3 * (e == 2 ? 0 : e + 1);
+    const double ed[3] = {dsub(c1[0], c0[0]), dsub(c1[1], c0[1]), dsub(c1[2], c0[2])};
+    const double w[3] = {dsub(x[0], c0[0]), dsub(x[1], c0[1]), dsub(x[2], c0[2])};
+    double m[3];
+    dcross(m, ed, w);
+    if (ddot(m, n) < 0.0) return CUDART_INF;
+  }
+  const double w[3] = {dsub(x[0], c[0]), dsub(x[1], c[1]), dsub(x[2], c[2])};
+  const double s = ddiv(ddot(n, w), nn);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) b[k] = dsub(x[k], dmul(n[k], s));
+  return dist2(x, b);
+}
+
+// Sub-problem k of a triangle pair, q = robot triangle and p = obstacle triangle (world frame): k < 9 robot edge k % 3
+// against obstacle edge k / 3, k = 9..11 robot vertex k - 9 against the obstacle face, k = 12..14 obstacle vertex k - 12
+// against the robot face.  For two disjoint triangles a nearest pair of points lies on an edge of each or is a vertex
+// facing the other's interior, so the minimum over the 15 is their distance.  a = robot point, b = obstacle point.
+__device__ __noinline__ double pair_subproblem(const double *q, const double *p, int k, double *a, double *b) {
+  if (k < 9) {
+    const int i = k / 3, j = k - 3 * i, i1 = i == 2 ? 0 : i + 1, j1 = j == 2 ? 0 : j + 1;
+    const double dq[3] = {dsub(q[3 * j1], q[3 * j]), dsub(q[3 * j1 + 1], q[3 * j + 1]), dsub(q[3 * j1 + 2], q[3 * j + 2])};
+    const double dp[3] = {dsub(p[3 * i1], p[3 * i]), dsub(p[3 * i1 + 1], p[3 * i + 1]), dsub(p[3 * i1 + 2], p[3 * i + 2])};
+    return seg_seg(q + 3 * j, dq, p + 3 * i, dp, a, b);
+  }
+  if (k < 12) {
+    const double *x = q + 3 * (k - 9);
+    a[0] = x[0]; a[1] = x[1]; a[2] = x[2];
+    return point_face(x, p, b);
+  }
+  const double *x = p + 3 * (k - 12);
+  b[0] = x[0]; b[1] = x[1]; b[2] = x[2];
+  return point_face(x, q, a);
+}
+
+// Lower bound on the distance between obstacle triangle x (robot frame, FP32) and the box [lo, hi]: the gap of the two
+// boxes less the position error of x (errpos per coordinate, sqrt(3) errpos in length, allotted 2 errpos; the FP32
+// subtractions and the square root are covered by the rest of the allowance and the factor).
+__device__ __forceinline__ float tri_box_distance_lb(const XTri &x, const float *lo, const float *hi, float errpos) {
+  float s = 0.f;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float g = fmaxf(fmaxf(min3f(x.v[c], x.v[3 + c], x.v[6 + c]) - hi[c], lo[c] - max3f(x.v[c], x.v[3 + c], x.v[6 + c])), 0.f);
+    s += g * g;
+  }
+  return sqrtf(s) * 0.99999f - 2.0f * errpos;
+}
+
+// Lower bound on the distance between a slot box and the robot's oriented box: the largest axis excess of slot_overlaps
+// less twice its pad (which covers the FP32 rotation against the pose's FP64 one), the robot-axis excess scaled down for
+// the rows of the FP32 R, which are unit only to within 2^-17.
+__device__ __forceinline__ float slot_distance_lb(const EnvDev &E, const PoseU &P, const BoxTest &bt, const float4 a, const float4 b) {
+  const float tx = (a.x - P.Thi[0]) - bt.o[0], ty = (a.y - P.Thi[1]) - bt.o[1], tz = (a.z - P.Thi[2]) - bt.o[2];
+  const float pad = kEpsBox * (fabsf(tx) + fabsf(ty) + fabsf(tz) + b.x + b.y + b.z + bt.rob_sz);
+  const float s0 = P.R[0] * tx + P.R[3] * ty + P.R[6] * tz, s1 = P.R[1] * tx + P.R[4] * ty + P.R[7] * tz,
+              s2 = P.R[2] * tx + P.R[5] * ty + P.R[8] * tz;
+  const float r0 = fabsf(P.R[0]) * b.x + fabsf(P.R[3]) * b.y + fabsf(P.R[6]) * b.z,
+              r1 = fabsf(P.R[1]) * b.x + fabsf(P.R[4]) * b.y + fabsf(P.R[7]) * b.z,
+              r2 = fabsf(P.R[2]) * b.x + fabsf(P.R[5]) * b.y + fabsf(P.R[8]) * b.z;
+  const float ex = fmaxf(fmaxf(fabsf(tx) - (b.x + bt.ra[0]), fabsf(ty) - (b.y + bt.ra[1])), fabsf(tz) - (b.z + bt.ra[2]));
+  const float eb = fmaxf(fmaxf(fabsf(s0) - (E.rob_h[0] + r0), fabsf(s1) - (E.rob_h[1] + r1)), fabsf(s2) - (E.rob_h[2] + r2));
+  return fmaxf(ex, eb * 0.99999f) - 2.0f * pad;
+}
+
+// Lower bound on the distance from the robot (inside its bounding sphere about T) to the obstacle AABB: the arithmetic of
+// sphere_hits_root, its pad and a relative allowance taken off.
+__device__ __forceinline__ float sphere_root_distance_lb(const EnvDev &E, const float *t, float tlo_mag) {
+  const float dx = fmaxf(fabsf(t[0] - E.root_c[0]) - E.root_h[0], 0.f);
+  const float dy = fmaxf(fabsf(t[1] - E.root_c[1]) - E.root_h[1], 0.f);
+  const float dz = fmaxf(fabsf(t[2] - E.root_c[2]) - E.root_h[2], 0.f);
+  const float pad = kEpsBox * (fabsf(t[0]) + fabsf(t[1]) + fabsf(t[2]) + fabsf(E.root_c[0]) + fabsf(E.root_c[1]) +
+                               fabsf(E.root_c[2]) + E.root_h[0] + E.root_h[1] + E.root_h[2] + E.rob_radius) + tlo_mag;
+  return sqrtf(dx * dx + dy * dy + dz * dz) * 0.99999f - (E.rob_radius + pad);
+}
+
+// the float that the slot and pair culls compare with: sqrt(best2) rounded up
+__device__ __forceinline__ float cull_bound(double best2) { return __double2float_ru(__dsqrt_ru(best2)); }
+
+// what the branch and bound of one pose has found: the squared distance bound and its two points (warp-uniform)
+struct DistBest {
+  double d2;
+  float cull;
+  double pts[6];   // robot point, obstacle point (world frame)
+};
+
+// Pair stage of one pose over the candidate triangles ws.tri[0, ntri): transform into the robot frame (FP32), drop those
+// whose box is farther than `best` from the robot's box, then lane-per-pair box bounds against each robot triangle; the
+// pairs they leave are evaluated in FP64, two pairs per pass on 15 lanes each (lanes 0..14 and 16..30).  The warp minimum
+// on (squared distance, lane) makes the outcome independent of timing.
+__device__ void distance_pair_stage(const EnvDev &E, WarpScratch &ws, const RobotTri *srob, const PoseU &P, const double *R2,
+                                    const double *T2, int lane, int ntri, DistBest &best) {
+  const unsigned lt = (1u << lane) - 1u;
+  const int half = lane >> 4, k = lane & 15;
+  const float inv_n_robot = 1.0f / (float)E.n_robot;
+  float rlo[3], rhi[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    rlo[c] = __fsub_rd(E.rob_c[c], E.rob_h[c]);
+    rhi[c] = __fadd_ru(E.rob_c[c], E.rob_h[c]);
+  }
+  for (int base = 0; base < ntri; base += 32) {
+    const int cnt = (ntri - base) < 32 ? (ntri - base) : 32;
+    bool keep = false;
+    XTri x;
+    if (lane < cnt) {
+      transform_triangle(E, P, ws.tri[base + lane], 0, x);   // (its overlap verdict is no use here)
+      keep = !(tri_box_distance_lb(x, rlo, rhi, 2.0f * x.err + kEpsSat * fmaxf(x.mabs, E.rob_radius)) > best.cull);
+    }
+    const unsigned km = __ballot_sync(kFull, keep);
+    if (keep) ws.xt[__popc(km & lt)] = x;
+    __syncwarp();
+    const int npairs = __popc(km) * E.n_robot;
+    for (int pb = 0; pb < npairs; pb += 32) {
+      const int pidx = pb + lane;
+      const int xi_l = (int)(((float)pidx + 0.5f) * inv_n_robot), r_l = pidx - xi_l * E.n_robot;
+      bool open = false;
+      if (pidx < npairs) {
+        const XTri &xp = ws.xt[xi_l];
+        const RobotTri &rt = srob[r_l];
+        open = !(tri_box_distance_lb(xp, rt.lo, rt.hi, 2.0f * xp.err + kEpsSat * fmaxf(xp.mabs, rt.qmax)) > best.cull);
+      }
+      unsigned um = __ballot_sync(kFull, open);
+      while (um) {
+        const int l0 = __ffs(um) - 1;
+        um &= um - 1;
+        const int l1 = um ? __ffs(um) - 1 : -1;
+        um &= um - 1;   // (0 stays 0)
+        const int lmine = half == 0 ? l0 : l1;
+        const int xim = __shfl_sync(kFull, xi_l, lmine & 31), rm = __shfl_sync(kFull, r_l, lmine & 31);
+        double d2 = CUDART_INF, a[3] = {0.0, 0.0, 0.0}, b[3] = {0.0, 0.0, 0.0};
+        if (lmine >= 0 && k < 15) {
+          const double *ot = E.tris64 + 9 * (size_t)ws.xt[xim].tri, *rq = E.robot64 + 9 * (size_t)rm;
+          double p[9], q[9];
+#pragma unroll
+          for (int j = 0; j < 9; ++j) p[j] = __ldg(ot + j);
+#pragma unroll
+          for (int v = 0; v < 3; ++v)   // robot vertex into the world frame: R2 r + T2
+#pragma unroll
+            for (int i = 0; i < 3; ++i)
+              q[3 * v + i] = dadd(dadd(dadd(dmul(R2[3 * i], __ldg(rq + 3 * v)), dmul(R2[3 * i + 1], __ldg(rq + 3 * v + 1))),
+                                       dmul(R2[3 * i + 2], __ldg(rq + 3 * v + 2))), T2[i]);
+          d2 = pair_subproblem(q, p, k, a, b);
+        }
+        int wl = lane;
+#pragma unroll
+        for (int s = 16; s > 0; s >>= 1) {
+          const double od = __shfl_xor_sync(kFull, d2, s);
+          const int ol = __shfl_xor_sync(kFull, wl, s);
+          if (od < d2 || (od == d2 && ol < wl)) { d2 = od; wl = ol; }
+        }
+        if (d2 < best.d2) {   // (warp-uniform)
+          best.d2 = d2;
+          best.cull = cull_bound(d2);
+#pragma unroll
+          for (int c = 0; c < 3; ++c) {
+            best.pts[c] = __shfl_sync(kFull, a[c], wl);
+            best.pts[3 + c] = __shfl_sync(kFull, b[c], wl);
+          }
+        }
+      }
+    }
+    __syncwarp();
+  }
+}
+
+// branch and bound of one free pose: walk_step with the distance cull, the pair stage after every step that found leaves
+template <int FMT>
+__device__ void warp_pose_distance(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const PoseU &P, const LanePose<FMT> &lp,
+                                   int src, int lane, DistBest &best) {
+  const BoxTest bt = make_box_test(E, P);
+  double R2[9], T2[3];
+  lp.exact(src, R2, T2, lane);
+  const auto near = [&](const float4 a, const float4 b) { return !(slot_distance_lb(E, P, bt, a, b) > best.cull); };
+  const unsigned lt = (1u << lane) - 1u;
+  Tally tally = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  int sp = 0;
+  bool first = true;
+  while (first || sp > 0) {
+    const StepLeaves lv = walk_step<false>(E, ws, cs, first, sp, lane, near, tally);
+    first = false;
+    if (lv.mine) ws.tri[__popc(lv.mask & lt)] = lv.tri;
+    if (sp > kStackCap) {     // never silently drop work: flag the launch as failed
+      if (lane == 0) *reinterpret_cast<volatile int *>(E.status) = 1;
+      sp = kStackCap;
+    }
+    __syncwarp();
+    if (lv.mask) distance_pair_stage(E, ws, cs.rob, P, R2, T2, lane, __popc(lv.mask), best);
+  }
+}
+
+template <int FMT>
+__global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) distance_poses_kernel(EnvDev E, const void *poses, long long n,
+                                                                                   double max_dist, double *dist_out,
+                                                                                   double *points_out, int chunk) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const CtaShared cs = stage_cta(E, smem, E.n_stage_max);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  WarpScratch &ws = warp_scratch(E, smem, warp);
+  const long long nchunks = (n + chunk - 1) / chunk;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  const double max2 = __dmul_ru(max_dist, max_dist);
+  Tally tally = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  while (true) {
+    unsigned c = 0;
+    if (lane == 0) c = atomicAdd(E.work_counter, 1u) - E.work_base;
+    c = __shfl_sync(kFull, c, 0);
+    if ((long long)c >= nchunks) break;
+    const long long i = (long long)c * chunk + lane;
+    const bool mine = lane < chunk && i < n;
+    LanePose<FMT> lp;
+    if (mine) lp.load(poses, i);
+    else lp.clear();
+    // contact: exactly the verdict of the pose kernel
+    const bool hit = (check_32_poses<FMT, false>(E, ws, cs, mine, lp, lane, false, tally) >> lane) & 1u;
+    float thi[3], tlo[3], R[9];
+    lp.split(thi, tlo);
+    const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
+    // lane-per-pose cap: a robot whose bounding sphere stays max_dist away from the obstacle box gets max_dist
+    const bool open = mine && !hit && E.n_obst > 0 && !((double)sphere_root_distance_lb(E, thi, tlo_mag) >= max_dist);
+    double d = hit ? 0.0 : max_dist, pt[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) pt[k] = nan;
+    if (open) lp.rot32(R);
+    unsigned todo = __ballot_sync(kFull, open);
+    while (todo) {
+      const int src = __ffs(todo) - 1;
+      todo &= todo - 1;
+      PoseU P;
+#pragma unroll
+      for (int k = 0; k < 9; ++k) P.R[k] = __shfl_sync(kFull, R[k], src);
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        P.Thi[k] = __shfl_sync(kFull, thi[k], src);
+        P.Tlo[k] = FMT == kFmtEulerF32 ? 0.f : __shfl_sync(kFull, tlo[k], src);
+      }
+      DistBest best;
+      best.d2 = max2;
+      best.cull = cull_bound(max2);
+      warp_pose_distance<FMT>(E, ws, cs, P, lp, src, lane, best);
+      if (lane == src && best.d2 < max2) {
+        const double dd = __dsqrt_rn(best.d2);
+        if (dd < max_dist) {
+          d = dd > 0.0 ? dd : 4.9406564584124654e-324;   // a free pose never reports contact
+#pragma unroll
+          for (int k = 0; k < 6; ++k) pt[k] = best.pts[k];
+        }
+      }
+    }
+    if (mine) {
+      dist_out[i] = d;
+      if (points_out) {
+#pragma unroll
+        for (int k = 0; k < 6; ++k) points_out[6 * i + k] = pt[k];
+      }
+    }
+  }
+}
+
 
 }  // namespace
 
@@ -1219,6 +1537,14 @@ cudaError_t launch_peer_barrier(const FlagSet &flags, unsigned epoch, bool signa
   return cudaGetLastError();
 }
 
+// poses per work unit of the pose kernels: enough units for ~2 per resident warp (at 2 CTAs/SM), capped at a full warp
+static int pose_chunk(int64_t n, const LaunchCfg &cfg) {
+  int chunk = 32;
+  const long long warps = (long long)cfg.sm_count * 2 * kWarpsPerBlock * 2;
+  while (chunk > 1 && (n + chunk - 1) / chunk < warps) chunk >>= 1;
+  return chunk;
+}
+
 // every warp of the grid leaves its loop through exactly one failing fetch, so a launch consumes
 // (units + grid * warps) values of the shared counter; the host advances the base instead of resetting the counter
 cudaError_t launch_collide_poses(const EnvDev &env_in, const void *d_poses, int pose_fmt, int64_t n, uint8_t *d_verdict,
@@ -1246,10 +1572,7 @@ cudaError_t launch_collide_poses_gather(const EnvDev &env_in, const void *d_pose
   EnvDev env = env_in;
   env.work_base = *work_base_io;
   int grid = 0;
-  // poses per work unit: enough units for ~2 per resident warp (at 2 CTAs/SM), capped at a full warp
-  int chunk = 32;
-  const long long warps = (long long)cfg.sm_count * 2 * kWarpsPerBlock * 2;
-  while (chunk > 1 && (n + chunk - 1) / chunk < warps) chunk >>= 1;
+  const int chunk = pose_chunk(n, cfg);
   cudaError_t e = cudaErrorInvalidValue;
   switch (pose_fmt) {
     case 0: e = launch_poses_fmt<kFmtEulerF32>(env, d_poses, n, d_verdict, gs, stream, cfg, count, chunk, &grid); break;
@@ -1257,6 +1580,28 @@ cudaError_t launch_collide_poses_gather(const EnvDev &env_in, const void *d_pose
     case 2: e = launch_poses_fmt<kFmtMatrixF64>(env, d_poses, n, d_verdict, gs, stream, cfg, count, chunk, &grid); break;
   }
   if (e == cudaSuccess) *work_base_io += (unsigned)((n + chunk - 1) / chunk) + (unsigned)grid * kWarpsPerBlock;
+  return e;
+}
+
+cudaError_t launch_distance_poses(const EnvDev &env_in, const void *d_poses, int pose_fmt, int64_t n, double max_dist,
+                                  double *d_dist, double *d_points, cudaStream_t stream, const LaunchCfg &cfg,
+                                  unsigned *work_base_io) {
+  if (n <= 0) return cudaSuccess;
+  EnvDev env = env_in;
+  env.work_base = *work_base_io;
+  const int chunk = pose_chunk(n, cfg);
+  const size_t smem = collide_smem_bytes(env.n_robot, env.n_stage_max);
+  const long long chunks = (n + chunk - 1) / chunk;
+  const long long want = (chunks + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  int grid = 0;
+  cudaError_t e = cudaErrorInvalidValue;
+  if (pose_fmt == kFmtEulerF32)
+    e = launch_resident<distance_poses_kernel<kFmtEulerF32>>(want, smem, stream, cfg, &grid, env, d_poses, (long long)n, max_dist,
+                                                             d_dist, d_points, chunk);
+  else if (pose_fmt == kFmtEulerF64)
+    e = launch_resident<distance_poses_kernel<kFmtEulerF64>>(want, smem, stream, cfg, &grid, env, d_poses, (long long)n, max_dist,
+                                                             d_dist, d_points, chunk);
+  if (e == cudaSuccess) *work_base_io += (unsigned)chunks + (unsigned)grid * kWarpsPerBlock;
   return e;
 }
 

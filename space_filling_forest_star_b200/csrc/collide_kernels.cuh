@@ -122,6 +122,13 @@ cudaError_t launch_collide_poses_gather(const EnvDev &env, const void *d_poses, 
 // by a 10 s timeout that raises the env status instead of hanging the GPU
 cudaError_t launch_peer_barrier(const FlagSet &flags, unsigned epoch, bool signal, int *d_status, cudaStream_t stream);
 
+// dist[i] = separation distance robot <-> obstacle soup of poses[i], capped at max_dist (0 exactly on contact); points
+// (optional, [n][6]) = nearest robot point then nearest obstacle point, world frame, NaN unless 0 < dist < max_dist.
+// pose_fmt 0 or 1 (the matrix form is not supported: cudaErrorInvalidValue)
+cudaError_t launch_distance_poses(const EnvDev &env, const void *d_poses, int pose_fmt, int64_t n, double max_dist,
+                                  double *d_dist, double *d_points, cudaStream_t stream, const LaunchCfg &cfg,
+                                  unsigned *work_base_io);
+
 cudaError_t launch_check_edges(const EnvDev &env, const double *d_starts, const double *d_ends, int64_t m,
                                double sample_dist, int rot_mode, uint8_t *d_free, int32_t *d_first_hit,
                                cudaStream_t stream, const LaunchCfg &cfg, bool count, unsigned *work_base_io,

@@ -36,8 +36,8 @@ namespace {
 constexpr size_t kSmallBytes = 1 << 20;   // pinned, device-mapped staging area of each object for planner-sized calls
 
 // The environment's staging area: inputs in the first 3/4, outputs in the last 1/4.  The outputs of a pose call are its
-// verdicts; those of an edge call are first hits [m] then free flags [m]; those of a move call are free flags [m] then
-// pose hits [m].
+// verdicts; those of a distance call are the distances [n] then (if asked for) the points [n][6]; those of an edge call
+// are first hits [m] then free flags [m]; those of a move call are free flags [m] then pose hits [m].
 struct EnvStaging {
   static constexpr size_t kInBytes = 768 << 10;
   static constexpr size_t kOutBytes = kSmallBytes - kInBytes;
@@ -822,24 +822,30 @@ int sffg_peer_barrier_device(sffg_env *env, uint32_t *const *d_flags, int n_rank
   return SFFG_OK;
 }
 
-static int collide_poses_host(sffg_env *env, const void *poses, int fmt, int64_t n, uint8_t *verdict_out) {
-  if (!env || n < 0 || (n > 0 && (!poses || !verdict_out))) return fail(SFFG_ERR_ARG, "sffg_collide_poses: bad arguments");
-  if (n == 0) return SFFG_OK;
-  const size_t psz = fmt == 0 ? 24 : (fmt == 1 ? 48 : 96);
+// Host-pointer pose calls (verdicts, distances) stage through one path: planner-sized batches through the pinned mapped
+// area (one kernel reading and writing it, one synchronisation, no DMA copies), larger ones in chunks of 2^20 poses on the
+// environment's two streams.  Pose i takes psz input bytes; output k (k < 2, null = not requested) takes osz[k] bytes per
+// pose.  launch(env view, d_in, cnt, d_out, stream, work base) enqueues the kernel for cnt poses.
+extern "C++" {   // (a template cannot have C linkage)
+template <class Launch>
+static int pose_call_host(sffg_env *env, const void *poses, size_t psz, int64_t n, void *const out[2], const size_t osz[2],
+                          const Launch &launch) {
+  const size_t ob[2] = {out[0] ? osz[0] : 0, out[1] ? osz[1] : 0};
   unsigned *base;
   {
     const int rc0 = env_enter_host(env);
     if (rc0 != SFFG_OK) return rc0;
   }
-  if ((size_t)n * psz <= EnvStaging::kInBytes && (size_t)n <= EnvStaging::kOutBytes) {
-    // planner-sized call: one kernel reading/writing pinned mapped memory, one synchronisation, no DMA copies
+  if ((size_t)n * psz <= EnvStaging::kInBytes && (size_t)n * (ob[0] + ob[1]) <= EnvStaging::kOutBytes) {
     cudaStream_t st = env->streams[0].get();
     const EnvStaging h = env->staging();
+    void *const d_out[2] = {out[0] ? h.out() : nullptr, out[1] ? h.out() + (size_t)n * ob[0] : nullptr};
     std::memcpy(h.in(), poses, (size_t)n * psz);
     EnvDev v = env_view(env, &base);
-    SFFG_CUDA(launch_collide_poses(v, h.in(), fmt, n, h.out(), st, env->cfg, env->count, base));
+    SFFG_CUDA(launch(v, h.in(), n, d_out, st, base));
     SFFG_CUDA(cudaStreamSynchronize(st));
-    std::memcpy(verdict_out, h.out(), (size_t)n);
+    for (int k = 0; k < 2; ++k)
+      if (out[k]) std::memcpy(out[k], d_out[k], (size_t)n * ob[k]);
     return check_status(env);
   }
   const int64_t chunk = 1 << 20;
@@ -848,16 +854,69 @@ static int collide_poses_host(sffg_env *env, const void *poses, int fmt, int64_t
     const int64_t cnt = std::min(chunk, n - off);
     cudaStream_t st = env->streams[s].get();
     SFFG_CUDA(cudaStreamSynchronize(st));   // buffers of this stream are free again
+    DevBuf *const bufs[2] = {&env->out[s], &env->aux[s]};
     int rc = env->in[s].reserve((size_t)cnt * psz);
-    if (rc == SFFG_OK) rc = env->out[s].reserve((size_t)cnt);
+    for (int k = 0; k < 2 && rc == SFFG_OK; ++k)
+      if (out[k]) rc = bufs[k]->reserve((size_t)cnt * ob[k]);
     if (rc != SFFG_OK) return rc;
+    void *const d_out[2] = {out[0] ? bufs[0]->p : nullptr, out[1] ? bufs[1]->p : nullptr};
     SFFG_CUDA(cudaMemcpyAsync(env->in[s].p, (const char *)poses + (size_t)off * psz, (size_t)cnt * psz, cudaMemcpyHostToDevice, st));
     EnvDev v = env_view(env, &base);
-    SFFG_CUDA(launch_collide_poses(v, env->in[s].p, fmt, cnt, (uint8_t *)env->out[s].p, st, env->cfg, env->count, base));
-    SFFG_CUDA(cudaMemcpyAsync(verdict_out + off, env->out[s].p, (size_t)cnt, cudaMemcpyDeviceToHost, st));
+    SFFG_CUDA(launch(v, env->in[s].p, cnt, d_out, st, base));
+    for (int k = 0; k < 2; ++k)
+      if (out[k])
+        SFFG_CUDA(cudaMemcpyAsync((char *)out[k] + (size_t)off * ob[k], d_out[k], (size_t)cnt * ob[k], cudaMemcpyDeviceToHost, st));
   }
   for (const Stream &st : env->streams) SFFG_CUDA(cudaStreamSynchronize(st.get()));
   return check_status(env);
+}
+}  // extern "C++"
+
+static int collide_poses_host(sffg_env *env, const void *poses, int fmt, int64_t n, uint8_t *verdict_out) {
+  if (!env || n < 0 || (n > 0 && (!poses || !verdict_out))) return fail(SFFG_ERR_ARG, "sffg_collide_poses: bad arguments");
+  if (n == 0) return SFFG_OK;
+  const size_t psz = fmt == 0 ? 24 : (fmt == 1 ? 48 : 96);
+  void *const out[2] = {verdict_out, nullptr};
+  const size_t osz[2] = {1, 0};
+  return pose_call_host(env, poses, psz, n, out, osz,
+                        [&](const EnvDev &v, const void *d_in, int64_t cnt, void *const *d_out, cudaStream_t st, unsigned *base) {
+                          return launch_collide_poses(v, d_in, fmt, cnt, (uint8_t *)d_out[0], st, env->cfg, env->count, base);
+                        });
+}
+
+// ---- separation distance per pose ------------------------------------------------------------------------------------
+static int distance_args(const sffg_env *env, const void *poses, int64_t n, double max_dist, const double *dist_out,
+                         const char *who) {
+  if (!env || n < 0 || (n > 0 && (!poses || !dist_out)) || !(max_dist > 0))
+    return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments (max_dist must be > 0)");
+  return SFFG_OK;
+}
+
+int sffg_distance_poses(sffg_env *env, const void *poses, int poses_are_f64, int64_t n, double max_dist, double *dist_out,
+                        double *points_out) {
+  const int rc = distance_args(env, poses, n, max_dist, dist_out, "sffg_distance_poses");
+  if (rc != SFFG_OK || n == 0) return rc;
+  const int fmt = poses_are_f64 ? 1 : 0;
+  void *const out[2] = {dist_out, points_out};
+  const size_t osz[2] = {8, 48};
+  return pose_call_host(env, poses, fmt ? 48 : 24, n, out, osz,
+                        [&](const EnvDev &v, const void *d_in, int64_t cnt, void *const *d_out, cudaStream_t st, unsigned *base) {
+                          return launch_distance_poses(v, d_in, fmt, cnt, max_dist, (double *)d_out[0], (double *)d_out[1], st,
+                                                       env->cfg, base);
+                        });
+}
+
+int sffg_distance_poses_device(sffg_env *env, const void *d_poses, int poses_are_f64, int64_t n, double max_dist,
+                               double *d_dist_out, double *d_points_out, void *stream) {
+  int rc = distance_args(env, d_poses, n, max_dist, d_dist_out, "sffg_distance_poses_device");
+  if (rc != SFFG_OK) return rc;
+  unsigned *base;
+  rc = env_enter(env, (cudaStream_t)stream);
+  if (rc != SFFG_OK) return rc;
+  EnvDev v = env_view(env, &base);
+  SFFG_CUDA(launch_distance_poses(v, d_poses, poses_are_f64 ? 1 : 0, n, max_dist, d_dist_out, d_points_out,
+                                  (cudaStream_t)stream, env->cfg, base));
+  return env_leave(env, (cudaStream_t)stream);
 }
 
 int sffg_collide_poses_f32(sffg_env *env, const float *poses, int64_t n, uint8_t *verdict_out) {

@@ -146,6 +146,38 @@ class Environment:
         check(self._L.sffg_collide_poses_device(self._h, poses.data_ptr(), int(poses.dtype == torch.float64), n, out.data_ptr(), st))
         return out
 
+    # ---- separation distance (sffg_distance_poses) -----------------------------------------------------------
+    def Distance(self, poses, max_dist: float = np.inf, points: bool = False):
+        """poses [n][6] float32 or float64 -> dist float64[n]: distance robot <-> obstacles capped at max_dist, 0 exactly
+        where Collide says 1; with ``points`` also float64 [n][6] (nearest robot point, nearest obstacle point, world
+        frame; NaN unless 0 < dist < max_dist)."""
+        p = np.asarray(poses)
+        if p.dtype != np.float32:
+            p = p.astype(np.float64, copy=False)
+        p = np.ascontiguousarray(p.reshape(-1, 6))
+        n = len(p)
+        dist = np.empty(n, dtype=np.float64)
+        pts = np.empty((n, 6), dtype=np.float64) if points else None
+        check(self._L.sffg_distance_poses(self._h, _ptr(p) if n else None, int(p.dtype == np.float64), n, float(max_dist),
+                                          _ptr(dist) if n else None, _ptr(pts) if (points and n) else None))
+        return (dist, pts) if points else dist
+
+    def distance_device(self, poses, max_dist: float = np.inf, out=None, points=None, stream: Optional[int] = None):
+        """poses: torch CUDA tensor [n][6] float32/float64 -> torch float64 [n] (enqueued, not synchronised); ``points``
+        (optional torch float64 [n][6] on the same device) receives the nearest points."""
+        import torch
+        assert poses.is_cuda and poses.is_contiguous() and poses.shape[-1] == 6
+        n = poses.numel() // 6
+        if out is None:
+            out = torch.empty(n, dtype=torch.float64, device=poses.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and out.numel() == n
+        if points is not None:
+            assert points.dtype == torch.float64 and points.is_contiguous() and points.numel() == 6 * n
+        st = torch.cuda.current_stream(poses.device).cuda_stream if stream is None else stream
+        check(self._L.sffg_distance_poses_device(self._h, poses.data_ptr(), int(poses.dtype == torch.float64), n, float(max_dist),
+                                                 out.data_ptr(), points.data_ptr() if points is not None else None, st))
+        return out
+
     # ---- Solver<T,R>::isPathFree ---------------------------------------------------------------------------
     def isPathFree(self, starts, ends, sample_dist: float = COLLISION_SAMPLE_SIZE, rot_mode: int = ROT_REFERENCE,
                    want_first_hit: bool = False):
