@@ -152,6 +152,28 @@ SFFG_API int sffg_distance_poses(sffg_env *env, const void *poses, int poses_are
 SFFG_API int sffg_distance_poses_device(sffg_env *env, const void *d_poses, int poses_are_f64, int64_t n, double max_dist,
                                         double *d_dist_out, double *d_points_out, void *stream);
 
+/* ---- separation distance per edge: the clearance of the segments isPathFree checks ---------------------------------
+ * The samples of edge e are exactly the poses sffg_check_edges tests for the same (start, end, sample_dist, rot_mode);
+ * D(e, k) is what sffg_distance_poses returns for sample k as a double pose at the same max_dist (in reference mode the
+ * sample's angles are 0).
+ *   - dist_out[e] = minimum of D(e, k) over the samples of e, bit for bit.  So dist_out[e] == 0 exactly where
+ *     sffg_check_edges reports free == 0; an edge without samples, and every edge when there are no obstacles, gets
+ *     max_dist.  The end points are not samples (as in isPathFree): a path's clearance is the minimum of its edges'
+ *     distances and sffg_distance_poses of its nodes
+ *   - index_out (optional, NULL allowed): the first colliding sample (first_hit_out of sffg_check_edges) when dist == 0;
+ *     the lowest k with D(e, k) == dist_out[e] when 0 < dist < max_dist; 0 otherwise
+ *   - points_out (optional, NULL allowed) [m][6]: a nearest point on the robot at sample index_out[e], then a nearest
+ *     point on the obstacles, world frame, as sffg_distance_poses gives them for that sample; NaN unless 0 < dist <
+ *     max_dist.  Where pairs tie, any of the tied points may be reported
+ *   - the argument errors of sffg_check_edges, and max_dist <= 0 or NaN: SFFG_ERR_ARG.  A traversal stack overflow raises
+ *     SFFG_ERR_INTERNAL (at once for the host call, at sffg_env_sync_check for the _device call)
+ *   - streams and threads as for every other call; no begin / end form and no counters */
+SFFG_API int sffg_distance_edges(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist,
+                                 int rot_mode, double max_dist, double *dist_out, int32_t *index_out, double *points_out);
+SFFG_API int sffg_distance_edges_device(sffg_env *env, const double *d_starts, const double *d_ends, int64_t m,
+                                        double sample_dist, int rot_mode, double max_dist, double *d_dist_out,
+                                        int32_t *d_index_out, double *d_points_out, void *stream);
+
 /* ---- multi-GPU (SURVEY 8e): pose batches are split over ranks, every rank needs all verdicts.  Instead of a separate
  * all-gather, the kernel stores verdict i to d_outs[r][i] for EVERY destination r: the local result buffer and the same
  * slice of every peer's buffer, mapped into this process through CUDA IPC -- the exchange rides on the kernel's own stores

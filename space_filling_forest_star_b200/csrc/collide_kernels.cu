@@ -1002,6 +1002,58 @@ constexpr int kNoHit = 0x7f7f7f7f;   // what cudaMemsetAsync(..., 0x7f, ...) pro
 // against 44.9 / 50.9 / 69.6), long edges lose a little (length 12: 68 against 62 us at 4).
 constexpr int kEdgeUnitsPerWarp = 1;
 
+// The samples of one edge as Solver<T,R>::isPathFree visits them: indices 1 .. S with (double)index < parts.  The edge
+// verdict and the edge distance kernels both take their poses from here, so the two see the same samples.
+struct EdgeSamples {
+  double s[6], dir[3], adir[3];
+  double parts;
+  long long S;
+};
+__device__ __forceinline__ EdgeSamples edge_samples(const double *starts, const double *ends, unsigned eidx, double sample) {
+  EdgeSamples es;
+  double f[6];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) {
+    es.s[k] = __ldg(starts + 6 * (size_t)eidx + k);
+    f[k] = __ldg(ends + 6 * (size_t)eidx + k);
+  }
+  // Point<T>::distance, src/primitives.h:224-235
+  double sum = 0.0;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const double d = dsub(es.s[k], f[k]);
+    sum = dadd(sum, dmul(d, d));
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    es.adir[k] = wrap_pi(dsub(f[3 + k], es.s[3 + k]));
+    sum = dadd(sum, dmul(es.adir[k], es.adir[k]));
+  }
+  const double total = sqrt(sum);
+  es.parts = __ddiv_rn(total, sample);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) es.dir[k] = dsub(f[k], es.s[k]);
+  es.S = 0;
+  if (es.parts > 1.0) {
+    const double cl = ceil(es.parts);
+    es.S = (cl > 2.0e9 ? 2000000000LL : (long long)cl) - 1;
+  }
+  return es;
+}
+// sample `idx` of the edge: start + (idx * dir) / parts, the angles interpolated the same way or (reference mode) the
+// identity rotation
+__device__ __forceinline__ void edge_sample_pose(const EdgeSamples &es, long long idx, int rot_mode, LanePose<kFmtEulerF64> &lp) {
+  const double di = (double)idx;
+  lp.clear();
+  lp.identity = rot_mode != SFFG_ROT_INTERPOLATE;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) lp.t[k] = dadd(es.s[k], __ddiv_rn(dmul(di, es.dir[k]), es.parts));
+  if (rot_mode == SFFG_ROT_INTERPOLATE) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) lp.a[k] = dadd(es.s[3 + k], __ddiv_rn(dmul(di, es.adir[k]), es.parts));
+  }
+}
+
 template <bool COUNT>
 __global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) check_edges_kernel(EnvDev E, const double *starts,
                                                                            const double *ends, long long m, double sample,
@@ -1021,52 +1073,18 @@ __global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) check_edges_kernel(
     if ((long long)u >= units) break;
     const unsigned eidx = u / (unsigned)split;
     const int part = (int)(u - eidx * (unsigned)split);
-    double s[6], f[6];
-#pragma unroll
-    for (int k = 0; k < 6; ++k) {
-      s[k] = __ldg(starts + 6 * (size_t)eidx + k);
-      f[k] = __ldg(ends + 6 * (size_t)eidx + k);
-    }
-    // Point<T>::distance, src/primitives.h:224-235
-    double sum = 0.0, adir[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      const double d = dsub(s[k], f[k]);
-      sum = dadd(sum, dmul(d, d));
-    }
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      adir[k] = wrap_pi(dsub(f[3 + k], s[3 + k]));
-      sum = dadd(sum, dmul(adir[k], adir[k]));
-    }
-    const double total = sqrt(sum);
-    const double parts = __ddiv_rn(total, sample);
-    const double dir[3] = {dsub(f[0], s[0]), dsub(f[1], s[1]), dsub(f[2], s[2])};
-    // indices 1 .. S with (double)index < parts
-    long long S = 0;
-    if (parts > 1.0) {
-      const double cl = ceil(parts);
-      S = (cl > 2.0e9 ? 2000000000LL : (long long)cl) - 1;
-    }
+    const EdgeSamples es = edge_samples(starts, ends, eidx, sample);
     int hit_index = 0;
     // warp `part` of the edge takes a CONTIGUOUS range of the sample indices (neighbouring samples share one swept box)
-    const long long range_len = (S + split - 1) / split;
+    const long long range_len = (es.S + split - 1) / split;
     const long long first_idx = 1 + (long long)part * range_len;
-    const long long last_idx = first_idx + range_len - 1 < S ? first_idx + range_len - 1 : S;
+    const long long last_idx = first_idx + range_len - 1 < es.S ? first_idx + range_len - 1 : es.S;
     for (long long base = first_idx; base <= last_idx && hit_index == 0; base += 32) {
       if (split > 1 && *reinterpret_cast<volatile int *>(fh + eidx) < base) break;   // an earlier hit is already known
       const long long idx = base + lane;
       const bool valid = idx <= last_idx;
-      const double di = (double)idx;
       LanePose<kFmtEulerF64> lp;
-      lp.clear();
-      lp.identity = rot_mode != SFFG_ROT_INTERPOLATE;
-#pragma unroll
-      for (int k = 0; k < 3; ++k) lp.t[k] = dadd(s[k], __ddiv_rn(dmul(di, dir[k]), parts));
-      if (rot_mode == SFFG_ROT_INTERPOLATE) {
-#pragma unroll
-        for (int k = 0; k < 3; ++k) lp.a[k] = dadd(s[3 + k], __ddiv_rn(dmul(di, adir[k]), parts));
-      }
+      edge_sample_pose(es, idx, rot_mode, lp);
       if (COUNT) nposes += valid ? 1 : 0;
       const unsigned hm = check_32_poses<kFmtEulerF64, COUNT, true>(E, ws, cs, valid, lp, lane, true, tally, true,
                                                                     rot_mode != SFFG_ROT_INTERPOLATE);
@@ -1461,6 +1479,155 @@ __global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) distance_poses_kern
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// separation distance per edge (sffg_distance_edges): the minimum of the pose distance over the samples isPathFree
+// checks.  Contact comes from the verdict launch that runs first (free flags and first hits), so this kernel does distance
+// work for free edges only.  A warp visits its range of an edge in index order; each sample's branch and bound starts
+// from the smallest squared distance found so far on that range, and a sample replaces the record only when its
+// reported (rounded) distance is strictly smaller.  A sample that finds nothing below the seed cannot lower the minimum,
+// so the record is the minimum over the samples and the lowest index that reports it.
+// ---------------------------------------------------------------------------------------------------------
+// one warp's result for its range of an edge (split > 1: finalize_distance_edges_kernel reduces them)
+struct EdgeDistRec {
+  double d;
+  int idx;
+  int pad;
+  double pts[6];
+};
+
+__device__ __forceinline__ void store_edge_distance(long long e, double d, int idx, const double *pts, int lane, double *dist_out,
+                                                    int32_t *index_out, double *points_out) {
+  if (lane == 0) {
+    dist_out[e] = d;
+    if (index_out) index_out[e] = idx;
+  }
+  if (points_out) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+      if (lane == k) points_out[6 * e + k] = pts[k];
+  }
+}
+
+__global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) distance_edges_kernel(EnvDev E, const double *starts,
+                                                                                   const double *ends, long long m, double sample,
+                                                                                   int rot_mode, double max_dist,
+                                                                                   const uint8_t *free_in, const int32_t *first_hit,
+                                                                                   double *dist_out, int32_t *index_out,
+                                                                                   double *points_out, int split, EdgeDistRec *recs) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const CtaShared cs = stage_cta(E, smem, E.n_stage_max);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  WarpScratch &ws = warp_scratch(E, smem, warp);
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  const double max2 = __dmul_ru(max_dist, max_dist);
+  const long long units = m * split;
+  while (true) {
+    unsigned u = 0;
+    if (lane == 0) u = atomicAdd(E.work_counter, 1u) - E.work_base;
+    u = __shfl_sync(kFull, u, 0);
+    if ((long long)u >= units) break;
+    const unsigned eidx = u / (unsigned)split;
+    const int part = (int)(u - eidx * (unsigned)split);
+    double pts[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) pts[k] = nan;
+    if (!__ldg(free_in + eidx)) {   // contact: 0 and the first colliding sample (split > 1: the finalize kernel writes it)
+      if (split == 1) store_edge_distance(eidx, 0.0, __ldg(first_hit + eidx), pts, lane, dist_out, index_out, points_out);
+      continue;
+    }
+    const EdgeSamples es = edge_samples(starts, ends, eidx, sample);
+    // the range of check_edges_kernel's warp `part`
+    const long long range_len = (es.S + split - 1) / split;
+    const long long first_idx = 1 + (long long)part * range_len;
+    const long long last_idx = first_idx + range_len - 1 < es.S ? first_idx + range_len - 1 : es.S;
+    double rd = max_dist, seed2 = max2;   // the record's distance and the bound the next sample starts from
+    int ri = 0;
+    for (long long base = first_idx; base <= last_idx; base += 32) {
+      const long long idx = base + lane;
+      LanePose<kFmtEulerF64> lp;
+      edge_sample_pose(es, idx, rot_mode, lp);
+      float thi[3], tlo[3], R[9];
+      lp.split(thi, tlo);
+      const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
+      // lane-per-sample cap: a robot whose bounding sphere stays the record's distance away from the obstacle box cannot
+      // lower it (re-checked against the record as it shrinks)
+      const double lb = idx <= last_idx && E.n_obst > 0 ? (double)sphere_root_distance_lb(E, thi, tlo_mag) : CUDART_INF;
+      const bool open = !(lb >= rd);
+      if (open) lp.rot32(R);
+      unsigned todo = __ballot_sync(kFull, open);
+      while (todo) {
+        const int src = __ffs(todo) - 1;
+        todo &= todo - 1;
+        if (__shfl_sync(kFull, lb, src) >= rd) continue;
+        PoseU P;
+#pragma unroll
+        for (int k = 0; k < 9; ++k) P.R[k] = __shfl_sync(kFull, R[k], src);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          P.Thi[k] = __shfl_sync(kFull, thi[k], src);
+          P.Tlo[k] = __shfl_sync(kFull, tlo[k], src);
+        }
+        DistBest best;
+        best.d2 = seed2;
+        best.cull = cull_bound(seed2);
+        warp_pose_distance<kFmtEulerF64>(E, ws, cs, P, lp, src, lane, best);
+        if (best.d2 < seed2) {   // (warp-uniform)
+          seed2 = best.d2;
+          const double dd = __dsqrt_rn(best.d2);
+          const double dr = dd > 0.0 ? dd : 4.9406564584124654e-324;   // what the pose query reports for this sample
+          if (dd < max_dist && dr < rd) {
+            rd = dr;
+            ri = (int)(base + src);
+#pragma unroll
+            for (int k = 0; k < 6; ++k) pts[k] = best.pts[k];
+          }
+        }
+      }
+    }
+    if (split == 1) {
+      store_edge_distance(eidx, rd, ri, pts, lane, dist_out, index_out, points_out);
+    } else {
+      EdgeDistRec *r = recs + u;
+      if (lane == 0) {
+        r->d = rd;
+        r->idx = ri;
+      }
+#pragma unroll
+      for (int k = 0; k < 6; ++k)
+        if (lane == k) r->pts[k] = pts[k];
+    }
+  }
+}
+
+// split > 1: the records of an edge's warps, in index order; the first one with the smallest distance holds the lowest
+// index that reports it
+__global__ void finalize_distance_edges_kernel(const EdgeDistRec *recs, int split, long long m, double max_dist,
+                                               const uint8_t *free_in, const int32_t *first_hit, double *dist_out,
+                                               int32_t *index_out, double *points_out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  double d = 0.0;
+  int idx = first_hit[i];
+  const double *pts = nullptr;
+  if (free_in[i]) {
+    d = max_dist;
+    idx = 0;
+    for (int p = 0; p < split; ++p) {
+      const EdgeDistRec &r = recs[i * split + p];
+      if (r.d < d) {
+        d = r.d;
+        idx = r.idx;
+        pts = r.pts;
+      }
+    }
+  }
+  dist_out[i] = d;
+  if (index_out) index_out[i] = idx;
+  if (points_out)
+    for (int k = 0; k < 6; ++k) points_out[6 * i + k] = pts ? pts[k] : nan;
+}
+
 
 }  // namespace
 
@@ -1632,6 +1799,48 @@ cudaError_t launch_check_edges(const EnvDev &env_in, const double *d_starts, con
   *work_base_io += (unsigned)units + (unsigned)grid * kWarpsPerBlock;
   if (split > 1) {
     finalize_edges_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>(d_fh_scratch, (long long)m, d_free, d_first_hit);
+    e = cudaGetLastError();
+  }
+  return e;
+}
+
+// warps per edge of the edge distance kernel: the rule of launch_check_edges, several only with a record slot each
+static int distance_edges_split(int64_t m, const LaunchCfg &cfg, bool have_recs) {
+  int split = 1;
+  const long long warps = (long long)cfg.sm_count * kWarpsPerBlock * kEdgeUnitsPerWarp;
+  if (have_recs)
+    while (split < 32 && m * split < warps) split <<= 1;
+  return split;
+}
+
+size_t distance_edges_rec_bytes(int64_t m, const LaunchCfg &cfg) {
+  const int split = distance_edges_split(m, cfg, true);
+  return split > 1 ? (size_t)m * split * sizeof(EdgeDistRec) : 0;
+}
+
+cudaError_t launch_distance_edges(const EnvDev &env, const double *d_starts, const double *d_ends, int64_t m, double sample_dist,
+                                  int rot_mode, double max_dist, double *d_dist, int32_t *d_index, double *d_points,
+                                  cudaStream_t stream, const LaunchCfg &cfg, unsigned *work_base_io,
+                                  const EdgeDistScratch &scr) {
+  if (m <= 0) return cudaSuccess;
+  cudaError_t e = launch_check_edges(env, d_starts, d_ends, m, sample_dist, rot_mode, scr.free, scr.first_hit, stream, cfg, false,
+                                     work_base_io, scr.fh);
+  if (e != cudaSuccess) return e;
+  EnvDev v = env;
+  v.work_base = *work_base_io;
+  const int split = distance_edges_split(m, cfg, scr.recs != nullptr);
+  const long long units = m * split;
+  const long long want = (units + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  int grid = 0;
+  e = launch_resident<distance_edges_kernel>(want, collide_smem_bytes(v.n_robot, v.n_stage_max), stream, cfg, &grid, v, d_starts,
+                                             d_ends, (long long)m, sample_dist, rot_mode, max_dist, (const uint8_t *)scr.free,
+                                             (const int32_t *)scr.first_hit, d_dist, d_index, d_points, split,
+                                             (EdgeDistRec *)scr.recs);
+  if (e != cudaSuccess) return e;
+  *work_base_io += (unsigned)units + (unsigned)grid * kWarpsPerBlock;
+  if (split > 1) {
+    finalize_distance_edges_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>(
+        (const EdgeDistRec *)scr.recs, split, (long long)m, max_dist, scr.free, scr.first_hit, d_dist, d_index, d_points);
     e = cudaGetLastError();
   }
   return e;

@@ -134,6 +134,21 @@ cudaError_t launch_check_edges(const EnvDev &env, const double *d_starts, const 
                                cudaStream_t stream, const LaunchCfg &cfg, bool count, unsigned *work_base_io,
                                int *d_fh_scratch /* m ints, or null to force one warp per edge */);
 
+// dist[e] = minimum over the samples of edge e (those launch_check_edges tests) of the pose distance capped at max_dist,
+// index[e] (optional) = the lowest sample reporting it (the first hit on contact, 0 when dist == max_dist), points
+// (optional, [m][6]) as for launch_distance_poses at that sample.  Enqueues launch_check_edges into the scratch first.
+struct EdgeDistScratch {
+  uint8_t *free;        // m free flags of the verdict launch
+  int32_t *first_hit;   // m first hits of the verdict launch
+  int *fh;              // m ints for the verdict launch's split edges, or null (one warp per edge)
+  void *recs;           // distance_edges_rec_bytes(m, cfg) bytes for the distance kernel's split edges, or null
+};
+size_t distance_edges_rec_bytes(int64_t m, const LaunchCfg &cfg);
+cudaError_t launch_distance_edges(const EnvDev &env, const double *d_starts, const double *d_ends, int64_t m, double sample_dist,
+                                  int rot_mode, double max_dist, double *d_dist, int32_t *d_index, double *d_points,
+                                  cudaStream_t stream, const LaunchCfg &cfg, unsigned *work_base_io,
+                                  const EdgeDistScratch &scr);
+
 cudaError_t launch_gen_poses(uint64_t seed, uint64_t first, int64_t n, const float range[6], float *d_out,
                              cudaStream_t stream);
 

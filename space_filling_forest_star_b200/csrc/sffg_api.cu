@@ -37,7 +37,8 @@ constexpr size_t kSmallBytes = 1 << 20;   // pinned, device-mapped staging area 
 
 // The environment's staging area: inputs in the first 3/4, outputs in the last 1/4.  The outputs of a pose call are its
 // verdicts; those of a distance call are the distances [n] then (if asked for) the points [n][6]; those of an edge call
-// are first hits [m] then free flags [m]; those of a move call are free flags [m] then pose hits [m].
+// are first hits [m] then free flags [m]; those of a move call are free flags [m] then pose hits [m]; those of an edge
+// distance call are the distances [m], the points [m][6], then the sample indices [m].
 struct EnvStaging {
   static constexpr size_t kInBytes = 768 << 10;
   static constexpr size_t kOutBytes = kSmallBytes - kInBytes;
@@ -48,6 +49,9 @@ struct EnvStaging {
   uint8_t *edge_free(int64_t m) const { return out() + (size_t)m * 4; }
   uint8_t *move_free() const { return out(); }
   uint8_t *move_hit(int64_t m) const { return out() + (size_t)m; }
+  double *edge_dist() const { return reinterpret_cast<double *>(out()); }
+  double *edge_points(int64_t m) const { return reinterpret_cast<double *>(out() + (size_t)m * 8); }
+  int32_t *edge_index(int64_t m) const { return reinterpret_cast<int32_t *>(out() + (size_t)m * 56); }
 };
 
 // The index's staging area.  The first 64 KiB hold the queries; the one-kernel radius search keeps its fallback flag in
@@ -170,6 +174,7 @@ struct sffg_env {
   cudaStream_t last_stream = nullptr;
   bool order_pending = false;
   DevBuf in[2], out[2], aux[2], fh;   // fh: per-edge first-hit scratch of small edge batches
+  DevBuf edge_scr, edge_rec;          // edge distance calls: the verdict launch's results, the per-warp records
   bool count = false;
   int64_t robot_bytes = 0;
   sffg_env_info_t info{};
@@ -931,7 +936,7 @@ int sffg_collide_transforms_f64(sffg_env *env, const double *rt, int64_t n, uint
 
 // arguments of the edge and move calls
 static int check_segment_args(const sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist,
-                              int rot_mode, const uint8_t *out, const char *who) {
+                              int rot_mode, const void *out, const char *who) {
   if (!env || m < 0 || (m > 0 && (!starts || !ends || !out)) || !(sample_dist > 0) ||
       (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
     return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments");
@@ -1014,6 +1019,30 @@ static int env_commit(sffg_env *env, const sffg_env::Pending &p, bool async) {
   return async ? SFFG_OK : sffg_env_end(env);
 }
 
+// Host-pointer edge calls too large for the staging area run in chunks of 2^18 edges on the environment's two streams in
+// turn.  run(s, off, cnt, ds, de, st) enqueues the kernels of one chunk, whose end points are at ds / de in device memory,
+// and the copies of its results on st (the buffers of stream s are free again when it is called).
+extern "C++" {   // (a template cannot have C linkage)
+template <class Run>
+static int edge_call_chunks(sffg_env *env, const double *starts, const double *ends, int64_t m, const Run &run) {
+  const int64_t chunk = 1 << 18;
+  int s = 0;
+  for (int64_t off = 0; off < m; off += chunk, s ^= 1) {
+    const int64_t cnt = std::min(chunk, m - off);
+    cudaStream_t st = env->streams[s].get();
+    SFFG_CUDA(cudaStreamSynchronize(st));
+    int rc = env->in[s].reserve((size_t)cnt * 96);
+    if (rc != SFFG_OK) return rc;
+    double *ds = (double *)env->in[s].p, *de = ds + 6 * cnt;
+    SFFG_CUDA(cudaMemcpyAsync(ds, starts + 6 * off, (size_t)cnt * 48, cudaMemcpyHostToDevice, st));
+    SFFG_CUDA(cudaMemcpyAsync(de, ends + 6 * off, (size_t)cnt * 48, cudaMemcpyHostToDevice, st));
+    if ((rc = run(s, off, cnt, ds, de, st)) != SFFG_OK) return rc;
+  }
+  for (const Stream &st : env->streams) SFFG_CUDA(cudaStreamSynchronize(st.get()));
+  return check_status(env);
+}
+}  // extern "C++"
+
 static int check_edges_impl(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist, int rot_mode,
                             uint8_t *free_out, int32_t *first_hit_out, bool async) {
   int rc = check_segment_args(env, starts, ends, m, sample_dist, rot_mode, free_out, "sffg_check_edges");
@@ -1030,28 +1059,103 @@ static int check_edges_impl(sffg_env *env, const double *starts, const double *e
                                  env->cfg, env->count, base, (int *)env->fh.p));
     return env_commit(env, sffg_env::Pending{1, m, free_out, first_hit_out}, async);
   }
-  const int64_t chunk = 1 << 18;
-  int s = 0;
-  for (int64_t off = 0; off < m; off += chunk, s ^= 1) {
-    const int64_t cnt = std::min(chunk, m - off);
-    cudaStream_t st = env->streams[s].get();
-    SFFG_CUDA(cudaStreamSynchronize(st));
-    rc = env->in[s].reserve((size_t)cnt * 96);
-    if (rc == SFFG_OK) rc = env->out[s].reserve((size_t)cnt);
-    if (rc == SFFG_OK) rc = env->aux[s].reserve((size_t)cnt * 4);
-    if (rc != SFFG_OK) return rc;
-    double *ds = (double *)env->in[s].p, *de = ds + 6 * cnt;
-    SFFG_CUDA(cudaMemcpyAsync(ds, starts + 6 * off, (size_t)cnt * 48, cudaMemcpyHostToDevice, st));
-    SFFG_CUDA(cudaMemcpyAsync(de, ends + 6 * off, (size_t)cnt * 48, cudaMemcpyHostToDevice, st));
+  return edge_call_chunks(env, starts, ends, m, [&](int s, int64_t off, int64_t cnt, double *ds, double *de, cudaStream_t st) {
+    int rc2 = env->out[s].reserve((size_t)cnt);
+    if (rc2 == SFFG_OK) rc2 = env->aux[s].reserve((size_t)cnt * 4);
+    if (rc2 != SFFG_OK) return rc2;
     EnvDev v = env_view(env, &base);
     SFFG_CUDA(launch_check_edges(v, ds, de, cnt, sample_dist, rot_mode, (uint8_t *)env->out[s].p,
                                  (int32_t *)env->aux[s].p, st, env->cfg, env->count, base, nullptr));
     SFFG_CUDA(cudaMemcpyAsync(free_out + off, env->out[s].p, (size_t)cnt, cudaMemcpyDeviceToHost, st));
     if (first_hit_out)
       SFFG_CUDA(cudaMemcpyAsync(first_hit_out + off, env->aux[s].p, (size_t)cnt * 4, cudaMemcpyDeviceToHost, st));
+    return SFFG_OK;
+  });
+}
+
+// ---- separation distance per edge --------------------------------------------------------------------------------
+static int distance_edges_args(const sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist,
+                               int rot_mode, double max_dist, const double *dist_out, const char *who) {
+  const int rc = check_segment_args(env, starts, ends, m, sample_dist, rot_mode, dist_out, who);
+  if (rc != SFFG_OK) return rc;
+  if (!(max_dist > 0)) return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments (max_dist must be > 0)");
+  return SFFG_OK;
+}
+
+// scratch of an edge distance call in environment memory: the verdict launch's first hits and free flags and, when its
+// edges may be split over several warps (`split`), the verdict launch's per-edge word and the distance kernel's records.
+// Growing frees the old block, so `st` (ordered behind every earlier launch of the environment) is drained first.
+static int edge_distance_scratch(sffg_env *env, int64_t m, bool split, cudaStream_t st, EdgeDistScratch *scr) {
+  const size_t rec = split ? distance_edges_rec_bytes(m, env->cfg) : 0;
+  const size_t fh = split ? (size_t)m * sizeof(int) : 0;
+  if ((size_t)m * 5 > env->edge_scr.cap || rec > env->edge_rec.cap || fh > env->fh.cap) SFFG_CUDA(cudaStreamSynchronize(st));
+  int rc = env->edge_scr.reserve((size_t)m * 5);
+  if (rc == SFFG_OK) rc = env->fh.reserve(fh);
+  if (rc == SFFG_OK) rc = env->edge_rec.reserve(rec);
+  if (rc != SFFG_OK) return rc;
+  scr->first_hit = (int32_t *)env->edge_scr.p;
+  scr->free = (uint8_t *)env->edge_scr.p + (size_t)m * 4;
+  scr->fh = split ? (int *)env->fh.p : nullptr;
+  scr->recs = rec ? env->edge_rec.p : nullptr;
+  return SFFG_OK;
+}
+
+int sffg_distance_edges(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist, int rot_mode,
+                        double max_dist, double *dist_out, int32_t *index_out, double *points_out) {
+  int rc = distance_edges_args(env, starts, ends, m, sample_dist, rot_mode, max_dist, dist_out, "sffg_distance_edges");
+  if (rc != SFFG_OK || m == 0) return rc;
+  if ((rc = env_enter_host(env)) != SFFG_OK) return rc;
+  unsigned *base;
+  if ((size_t)m * 96 <= EnvStaging::kInBytes && (size_t)m * 60 <= EnvStaging::kOutBytes) {
+    // planner-sized call: both kernels on one stream, results straight into pinned mapped memory, one synchronisation
+    cudaStream_t st = env->streams[0].get();
+    const EnvStaging h = env->staging();
+    EdgeDistScratch scr;
+    double *ds, *de;
+    if ((rc = edge_distance_scratch(env, m, true, st, &scr)) != SFFG_OK) return rc;
+    if ((rc = stage_segments(env, starts, ends, m, &ds, &de)) != SFFG_OK) return rc;
+    EnvDev v = env_view(env, &base);
+    SFFG_CUDA(launch_distance_edges(v, ds, de, m, sample_dist, rot_mode, max_dist, h.edge_dist(), index_out ? h.edge_index(m) : nullptr,
+                                    points_out ? h.edge_points(m) : nullptr, st, env->cfg, base, scr));
+    SFFG_CUDA(cudaStreamSynchronize(st));
+    std::memcpy(dist_out, h.edge_dist(), (size_t)m * 8);
+    if (index_out) std::memcpy(index_out, h.edge_index(m), (size_t)m * 4);
+    if (points_out) std::memcpy(points_out, h.edge_points(m), (size_t)m * 48);
+    return check_status(env);
   }
-  for (const Stream &st : env->streams) SFFG_CUDA(cudaStreamSynchronize(st.get()));
-  return check_status(env);
+  return edge_call_chunks(env, starts, ends, m, [&](int s, int64_t off, int64_t cnt, double *ds, double *de, cudaStream_t st) {
+    // out[s]: distances [cnt], points [cnt][6], indices [cnt]; aux[s]: the verdict launch's first hits and free flags
+    int rc2 = env->out[s].reserve((size_t)cnt * 60);
+    if (rc2 == SFFG_OK) rc2 = env->aux[s].reserve((size_t)cnt * 5);
+    if (rc2 != SFFG_OK) return rc2;
+    double *d_dist = (double *)env->out[s].p, *d_points = d_dist + cnt;
+    int32_t *d_index = (int32_t *)(d_points + 6 * cnt);
+    const EdgeDistScratch scr{(uint8_t *)env->aux[s].p + (size_t)cnt * 4, (int32_t *)env->aux[s].p, nullptr, nullptr};
+    EnvDev v = env_view(env, &base);
+    SFFG_CUDA(launch_distance_edges(v, ds, de, cnt, sample_dist, rot_mode, max_dist, d_dist, index_out ? d_index : nullptr,
+                                    points_out ? d_points : nullptr, st, env->cfg, base, scr));
+    SFFG_CUDA(cudaMemcpyAsync(dist_out + off, d_dist, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+    if (index_out) SFFG_CUDA(cudaMemcpyAsync(index_out + off, d_index, (size_t)cnt * 4, cudaMemcpyDeviceToHost, st));
+    if (points_out) SFFG_CUDA(cudaMemcpyAsync(points_out + 6 * off, d_points, (size_t)cnt * 48, cudaMemcpyDeviceToHost, st));
+    return SFFG_OK;
+  });
+}
+
+int sffg_distance_edges_device(sffg_env *env, const double *d_starts, const double *d_ends, int64_t m, double sample_dist,
+                               int rot_mode, double max_dist, double *d_dist_out, int32_t *d_index_out, double *d_points_out,
+                               void *stream) {
+  int rc = distance_edges_args(env, d_starts, d_ends, m, sample_dist, rot_mode, max_dist, d_dist_out, "sffg_distance_edges_device");
+  if (rc != SFFG_OK) return rc;
+  unsigned *base;
+  rc = env_enter(env, (cudaStream_t)stream);
+  if (rc != SFFG_OK) return rc;
+  // small batches: several warps per edge, as sffg_check_edges_device
+  EdgeDistScratch scr;
+  if ((rc = edge_distance_scratch(env, m, m < 8192, (cudaStream_t)stream, &scr)) != SFFG_OK) return rc;
+  EnvDev v = env_view(env, &base);
+  SFFG_CUDA(launch_distance_edges(v, d_starts, d_ends, m, sample_dist, rot_mode, max_dist, d_dist_out, d_index_out, d_points_out,
+                                  (cudaStream_t)stream, env->cfg, base, scr));
+  return env_leave(env, (cudaStream_t)stream);
 }
 
 static int check_moves_impl(sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist, int rot_mode,

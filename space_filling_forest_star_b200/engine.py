@@ -178,6 +178,46 @@ class Environment:
                                                  out.data_ptr(), points.data_ptr() if points is not None else None, st))
         return out
 
+    def EdgeDistance(self, starts, ends, max_dist: float = np.inf, sample_dist: float = COLLISION_SAMPLE_SIZE,
+                     rot_mode: int = ROT_REFERENCE, points: bool = False):
+        """edges start -> end ([m][6] float64) -> (dist float64[m], index int32[m]): the minimum over the samples isPathFree
+        checks of the pose distance capped at max_dist (0 exactly where isPathFree says 0) and the lowest sample reporting
+        it (the first hit on contact, 0 when dist == max_dist); with ``points`` also float64 [m][6] (nearest robot point at
+        that sample, nearest obstacle point; NaN unless 0 < dist < max_dist).  The end points are not samples."""
+        s = np.ascontiguousarray(np.asarray(starts, dtype=np.float64).reshape(-1, 6))
+        e = np.ascontiguousarray(np.asarray(ends, dtype=np.float64).reshape(-1, 6))
+        assert len(s) == len(e)
+        m = len(s)
+        dist = np.empty(m, dtype=np.float64)
+        index = np.empty(m, dtype=np.int32)
+        pts = np.empty((m, 6), dtype=np.float64) if points else None
+        check(self._L.sffg_distance_edges(self._h, _ptr(s) if m else None, _ptr(e) if m else None, m, float(sample_dist), rot_mode,
+                                          float(max_dist), _ptr(dist) if m else None, _ptr(index) if m else None,
+                                          _ptr(pts) if (points and m) else None))
+        return (dist, index, pts) if points else (dist, index)
+
+    def edge_distance_device(self, starts, ends, max_dist: float = np.inf, sample_dist: float = COLLISION_SAMPLE_SIZE,
+                             rot_mode: int = ROT_REFERENCE, out=None, index_out=None, points=None, stream: Optional[int] = None):
+        """starts, ends: torch CUDA float64 [m][6] -> torch float64 [m] (enqueued, not synchronised); ``index_out`` (int32
+        [m]) and ``points`` (float64 [m][6]) on the same device are optional."""
+        import torch
+        assert starts.is_cuda and starts.dtype == torch.float64 and ends.dtype == torch.float64
+        assert starts.is_contiguous() and ends.is_contiguous() and starts.shape == ends.shape
+        m = starts.numel() // 6
+        if out is None:
+            out = torch.empty(m, dtype=torch.float64, device=starts.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and out.numel() == m
+        if index_out is not None:
+            assert index_out.dtype == torch.int32 and index_out.is_contiguous() and index_out.numel() == m
+        if points is not None:
+            assert points.dtype == torch.float64 and points.is_contiguous() and points.numel() == 6 * m
+        st = torch.cuda.current_stream(starts.device).cuda_stream if stream is None else stream
+        check(self._L.sffg_distance_edges_device(self._h, starts.data_ptr(), ends.data_ptr(), m, float(sample_dist), rot_mode,
+                                                 float(max_dist), out.data_ptr(),
+                                                 index_out.data_ptr() if index_out is not None else None,
+                                                 points.data_ptr() if points is not None else None, st))
+        return out
+
     # ---- Solver<T,R>::isPathFree ---------------------------------------------------------------------------
     def isPathFree(self, starts, ends, sample_dist: float = COLLISION_SAMPLE_SIZE, rot_mode: int = ROT_REFERENCE,
                    want_first_hit: bool = False):
