@@ -174,6 +174,37 @@ SFFG_API int sffg_distance_edges_device(sffg_env *env, const double *d_starts, c
                                         double sample_dist, int rot_mode, double max_dist, double *d_dist_out,
                                         int32_t *d_index_out, double *d_points_out, void *stream);
 
+/* ---- continuous edge check: a certificate for the whole motion, not only for the samples isPathFree checks -----------
+ * sffg_check_edges tests poses sample_dist apart and says nothing between them: a thin wall or a pole crossed between two
+ * samples is missed.  This call certifies the motion itself by conservative advancement on the pose distance.
+ *   - the motion of edge e, tau in [0, 1]: position x_k(tau) = s_k + tau * (f_k - s_k) (s = starts[e], f = ends[e]), each
+ *     operation rounded to nearest, no FMA.  SFFG_ROT_REFERENCE: identity rotation for every tau, end points included (how
+ *     isPathFree places its samples).  SFFG_ROT_INTERPOLATE: angles s_{3+k} + tau * wrap(f_{3+k} - s_{3+k}), wrap as in
+ *     sffg_check_edges.  Every sample sffg_check_edges tests lies on this curve, up to rounding, for any sample_dist
+ *   - margin = m > 0.  clear_out[e] = 1: every pose of the motion is at distance >= m / 2 from the obstacles, up to the
+ *     accuracy of sffg_distance_poses (1e-9 S); in particular the whole motion is collision free.  t_out[e] = 1.0 and
+ *     dist_out[e] = m then
+ *   - clear_out[e] = 0: t_out[e] = tau* in [0, 1) where the distance of pose(tau*) is < m, every pose with tau < tau* is at
+ *     distance >= m / 2 (same accuracy), and dist_out[e] is, bit for bit, what sffg_distance_poses returns for pose(tau*)
+ *     as a double pose at max_dist = m (in reference mode its angles are 0).  So dist_out[e] == 0 exactly when
+ *     sffg_collide_poses_f64 reports contact at pose(tau*)
+ *   - a motion that comes within m / 2 of the obstacles is never clear, one that stays >= m away is always clear; in
+ *     between either answer can come back, each certified as stated.  An edge with a non-finite coordinate (that the
+ *     motion uses) is never clear: t = 0, dist = NaN.  With no obstacles every edge is clear
+ *   - t_out and dist_out are optional (NULL allowed).  No points, no begin / end form, no counters
+ *   - clear, t and dist do not depend on the batch size, the split of edges over warps, host chunking, the host or device
+ *     form, the hierarchy builder or timing
+ *   - work: at most 32 + 2 mu / m pose distance evaluations per edge, mu = |f_xyz - s_xyz| (reference mode) plus
+ *     rho (|dyaw| + |dpitch| + |droll|) with wrapped differences (interpolate mode), rho = the robot's bounding radius
+ *   - SFFG_ERR_ARG: the argument errors of sffg_check_edges (sample_dist aside); margin <= 0, NaN or infinite; margin <
+ *     1e-6 max(1, max |obstacle coordinate|) (the coordinate rounded up to float).  A traversal stack overflow raises
+ *     SFFG_ERR_INTERNAL (at once for the host call, at sffg_env_sync_check for the _device call), never a wrong answer
+ *   - streams and threads as for every other call */
+SFFG_API int sffg_sweep_edges(sffg_env *env, const double *starts, const double *ends, int64_t m, int rot_mode,
+                              double margin, uint8_t *clear_out, double *t_out, double *dist_out);
+SFFG_API int sffg_sweep_edges_device(sffg_env *env, const double *d_starts, const double *d_ends, int64_t m, int rot_mode,
+                                     double margin, uint8_t *d_clear_out, double *d_t_out, double *d_dist_out, void *stream);
+
 /* ---- multi-GPU (SURVEY 8e): pose batches are split over ranks, every rank needs all verdicts.  Instead of a separate
  * all-gather, the kernel stores verdict i to d_outs[r][i] for EVERY destination r: the local result buffer and the same
  * slice of every peer's buffer, mapped into this process through CUDA IPC -- the exchange rides on the kernel's own stores

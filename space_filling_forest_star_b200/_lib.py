@@ -58,6 +58,8 @@ SIGNATURES = {
     "sffg_distance_poses_device": (C.c_int, [_p, _p, C.c_int, C.c_int64, C.c_double, _p, _p, _p]),
     "sffg_distance_edges": (C.c_int, [_p, _p, _p, C.c_int64, C.c_double, C.c_int, C.c_double, _p, _p, _p]),
     "sffg_distance_edges_device": (C.c_int, [_p, _p, _p, C.c_int64, C.c_double, C.c_int, C.c_double, _p, _p, _p, _p]),
+    "sffg_sweep_edges": (C.c_int, [_p, _p, _p, C.c_int64, C.c_int, C.c_double, _p, _p, _p]),
+    "sffg_sweep_edges_device": (C.c_int, [_p, _p, _p, C.c_int64, C.c_int, C.c_double, _p, _p, _p, _p]),
     "sffg_peer_buffer_create": (C.c_int, [C.c_int64, C.POINTER(_p), _p]),
     "sffg_peer_buffer_open": (C.c_int, [_p, C.POINTER(_p)]),
     "sffg_peer_buffer_close": (C.c_int, [_p]),

@@ -1628,6 +1628,194 @@ __global__ void finalize_distance_edges_kernel(const EdgeDistRec *recs, int spli
     for (int k = 0; k < 6; ++k) points_out[6 * i + k] = pts ? pts[k] : nan;
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// continuous edge check (sffg_sweep_edges): conservative advancement on the pose distance over the motion
+// pose(tau) = start + tau (end - start), tau in [0, 1].  No robot point moves faster than mu per unit tau, so a pose at
+// distance D >= margin certifies every pose up to tau + (D - margin / 2) / mu at distance >= margin / 2.  [0, 1] is cut into
+// kSweepPieces fixed pieces, one lane each; a piece advances from its own start, so its outcome does not depend on which
+// warp runs it.  A step's D is 0 on contact (check_32_poses, the verdict path), else min(d, C) with the cap
+// C = mu (b - tau) + margin: the FP64 branch-and-bound minimum seeded at C^2, or C itself when the lane's bounding-sphere
+// bound already proves d >= C.  Both ways D is C or the cap-independent minimum, so it is deterministic.
+// ---------------------------------------------------------------------------------------------------------
+constexpr int kSweepPieces = 32;
+
+// one warp's lowest stopped piece of an edge (split > 1: finalize_sweep_edges_kernel reduces them), kSweepPieces for none
+struct SweepRec {
+  double t, d;
+  int piece;
+  int pad;
+};
+
+// the motion of one edge and mu, its motion bound rounded up: |f_xyz - s_xyz|, plus rho times the sum of the wrapped angle
+// differences when the angles are interpolated (|omega| <= the sum of the Euler angle rates, |robot point| <= rho)
+struct SweepEdge {
+  double s[6], dir[3], adir[3];
+  double mu;
+};
+__device__ __forceinline__ SweepEdge sweep_edge(const EnvDev &E, const double *starts, const double *ends, unsigned eidx,
+                                                int rot_mode) {
+  SweepEdge ed;
+  double l2 = 0.0, turn = 0.0;
+#pragma unroll
+  for (int k = 0; k < 6; ++k) ed.s[k] = __ldg(starts + 6 * (size_t)eidx + k);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    ed.dir[k] = dsub(__ldg(ends + 6 * (size_t)eidx + k), ed.s[k]);
+    ed.adir[k] = wrap_pi(dsub(__ldg(ends + 6 * (size_t)eidx + 3 + k), ed.s[3 + k]));
+    l2 = __dadd_ru(l2, __dmul_ru(ed.dir[k], ed.dir[k]));
+    turn = __dadd_ru(turn, fabs(ed.adir[k]));
+  }
+  ed.mu = __dsqrt_ru(l2);
+  if (rot_mode == SFFG_ROT_INTERPOLATE) ed.mu = __dadd_ru(ed.mu, __dmul_ru((double)E.rob_radius, turn));
+  return ed;
+}
+// pose(tau): each operation rounded to nearest, no FMA; reference mode keeps the identity rotation
+__device__ __forceinline__ void sweep_pose(const SweepEdge &ed, double tau, int rot_mode, LanePose<kFmtEulerF64> &lp) {
+  lp.clear();
+  lp.identity = rot_mode != SFFG_ROT_INTERPOLATE;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) lp.t[k] = dadd(ed.s[k], dmul(tau, ed.dir[k]));
+  if (rot_mode == SFFG_ROT_INTERPOLATE) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) lp.a[k] = dadd(ed.s[3 + k], dmul(tau, ed.adir[k]));
+  }
+}
+
+__device__ __forceinline__ void store_sweep(long long e, int piece, double t, double d, uint8_t *clear_out, double *t_out,
+                                            double *dist_out) {
+  clear_out[e] = piece == kSweepPieces ? 1 : 0;
+  if (t_out) t_out[e] = t;
+  if (dist_out) dist_out[e] = d;
+}
+
+// Units are (edge, part): warp `part` of an edge takes pieces part * (kSweepPieces / split) .. + kSweepPieces / split - 1,
+// piece = first + lane.  Every round builds the current pose of each live piece, decides contact for all of them in one
+// check_32_poses call, runs the branch and bound warp-cooperatively for the lanes the sphere bound leaves open, then
+// advances each piece.  A piece above a known stop (this warp's, or with split > 1 another warp's, published in `stop`)
+// cannot change the result and is dropped.
+__global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) sweep_edges_kernel(EnvDev E, const double *starts, const double *ends,
+                                                                                long long m, int rot_mode, double margin,
+                                                                                uint8_t *clear_out, double *t_out, double *dist_out,
+                                                                                int split, int *stop, SweepRec *recs) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const CtaShared cs = stage_cta(E, smem, E.n_stage_max);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  WarpScratch &ws = warp_scratch(E, smem, warp);
+  const double half = 0.5 * margin;
+  const int per = kSweepPieces / split;
+  const long long units = m * split;
+  Tally tally = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  while (true) {
+    unsigned u = 0;
+    if (lane == 0) u = atomicAdd(E.work_counter, 1u) - E.work_base;
+    u = __shfl_sync(kFull, u, 0);
+    if ((long long)u >= units) break;
+    const unsigned eidx = u / (unsigned)split;
+    const int part = (int)(u - eidx * (unsigned)split);
+    const SweepEdge ed = sweep_edge(E, starts, ends, eidx, rot_mode);
+    // a motionless edge is one pose (every piece would repeat piece 0); a non-finite one is never clear
+    const bool finite = ed.mu <= DBL_MAX;
+    const int npieces = ed.mu > 0.0 ? kSweepPieces : 1;
+    const int piece = part * per + lane;
+    bool live = finite && lane < per && piece < npieces;
+    double tau = (double)piece * (1.0 / kSweepPieces);
+    const double b = (double)(piece + 1) * (1.0 / kSweepPieces);
+    int rp = finite ? kSweepPieces : 0;   // this warp's lowest stopped piece, its tau and its D
+    double rt = finite ? 1.0 : 0.0, rd = finite ? margin : __longlong_as_double(0x7ff8000000000000ll);
+    while (true) {
+      int lowest = rp;
+      if (split > 1) lowest = min(lowest, *reinterpret_cast<volatile int *>(stop + eidx));
+      live = live && piece < lowest;
+      if (!__any_sync(kFull, live)) break;
+      LanePose<kFmtEulerF64> lp;
+      sweep_pose(ed, tau, rot_mode, lp);
+      float thi[3], tlo[3], R[9];
+      lp.split(thi, tlo);
+      const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
+      const double cap = __dadd_ru(__dmul_ru(ed.mu, __dsub_ru(b, tau)), margin);
+      // the sphere bound proves d >= cap (so no contact either): D = cap without the walk
+      const bool near = live && E.n_obst > 0 && !((double)sphere_root_distance_lb(E, thi, tlo_mag) >= cap);
+      const bool hit = (check_32_poses<kFmtEulerF64, false>(E, ws, cs, near, lp, lane, false, tally) >> lane) & 1u;
+      double D = hit ? 0.0 : cap;
+      const bool open = near && !hit;
+      if (open) lp.rot32(R);
+      unsigned todo = __ballot_sync(kFull, open);
+      while (todo) {
+        const int src = __ffs(todo) - 1;
+        todo &= todo - 1;
+        PoseU P;
+#pragma unroll
+        for (int k = 0; k < 9; ++k) P.R[k] = __shfl_sync(kFull, R[k], src);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          P.Thi[k] = __shfl_sync(kFull, thi[k], src);
+          P.Tlo[k] = __shfl_sync(kFull, tlo[k], src);
+        }
+        const double c = __shfl_sync(kFull, cap, src), c2 = __dmul_ru(c, c);
+        DistBest best;
+        best.d2 = c2;
+        best.cull = cull_bound(c2);
+        warp_pose_distance<kFmtEulerF64>(E, ws, cs, P, lp, src, lane, best);
+        if (lane == src && best.d2 < c2) {
+          const double dd = __dsqrt_rn(best.d2);
+          if (dd < c) D = dd > 0.0 ? dd : 4.9406564584124654e-324;   // what the pose query reports for this pose
+        }
+      }
+      const bool stopped = live && D < margin;
+      if (live && !stopped) {
+        if (ed.mu == 0.0) {
+          live = false;   // clear: the whole motion is this pose
+        } else {
+          // the step rounds down (mu is rounded up); when mu > 2^51 margin it can fall below one ulp of tau, and the piece
+          // moves to the next double
+          double next = __dadd_rd(tau, __ddiv_rd(__dsub_rd(D, half), ed.mu));
+          if (next == tau) next = nextafter(tau, 2.0);
+          tau = next;
+          live = tau < b;
+        }
+      }
+      const unsigned sm = __ballot_sync(kFull, stopped);
+      if (sm) {
+        const int l = __ffs(sm) - 1;   // lanes hold increasing pieces: the lowest stopped piece of this round
+        const int p = __shfl_sync(kFull, piece, l);
+        const double t = __shfl_sync(kFull, tau, l), d = __shfl_sync(kFull, D, l);
+        if (p < rp) {
+          rp = p;
+          rt = t;
+          rd = d;
+          if (split > 1 && lane == 0) atomicMin(stop + eidx, p);
+        }
+      }
+      live = live && !stopped;
+    }
+    if (split == 1) {
+      if (lane == 0) store_sweep(eidx, rp, rt, rd, clear_out, t_out, dist_out);
+    } else if (lane == 0) {
+      recs[u].t = rt;
+      recs[u].d = rd;
+      recs[u].piece = rp;
+    }
+  }
+}
+
+// split > 1: the lowest stopped piece over an edge's warps decides; none stopped = clear
+__global__ void finalize_sweep_edges_kernel(const SweepRec *recs, int split, long long m, double margin, uint8_t *clear_out,
+                                            double *t_out, double *dist_out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  int piece = kSweepPieces;
+  double t = 1.0, d = margin;
+  for (int p = 0; p < split; ++p) {
+    const SweepRec &r = recs[i * split + p];
+    if (r.piece < piece) {
+      piece = r.piece;
+      t = r.t;
+      d = r.d;
+    }
+  }
+  store_sweep(i, piece, t, d, clear_out, t_out, dist_out);
+}
+
 
 }  // namespace
 
@@ -1841,6 +2029,36 @@ cudaError_t launch_distance_edges(const EnvDev &env, const double *d_starts, con
   if (split > 1) {
     finalize_distance_edges_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>(
         (const EdgeDistRec *)scr.recs, split, (long long)m, max_dist, scr.free, scr.first_hit, d_dist, d_index, d_points);
+    e = cudaGetLastError();
+  }
+  return e;
+}
+
+size_t sweep_edges_rec_bytes(int64_t m, const LaunchCfg &cfg) {
+  const int split = distance_edges_split(m, cfg, true);
+  return split > 1 ? (size_t)m * split * sizeof(SweepRec) : 0;
+}
+
+cudaError_t launch_sweep_edges(const EnvDev &env_in, const double *d_starts, const double *d_ends, int64_t m, int rot_mode,
+                               double margin, uint8_t *d_clear, double *d_t, double *d_dist, cudaStream_t stream,
+                               const LaunchCfg &cfg, unsigned *work_base_io, const SweepScratch &scr) {
+  if (m <= 0) return cudaSuccess;
+  EnvDev env = env_in;
+  env.work_base = *work_base_io;
+  const int split = distance_edges_split(m, cfg, scr.stop != nullptr && scr.recs != nullptr);
+  const long long units = m * split;
+  const long long want = (units + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  cudaError_t e;
+  if (split > 1 && (e = cudaMemsetAsync(scr.stop, 0x7f, (size_t)m * sizeof(int), stream)) != cudaSuccess) return e;
+  int grid = 0;
+  e = launch_resident<sweep_edges_kernel>(want, collide_smem_bytes(env.n_robot, env.n_stage_max), stream, cfg, &grid, env, d_starts,
+                                          d_ends, (long long)m, rot_mode, margin, d_clear, d_t, d_dist, split, scr.stop,
+                                          (SweepRec *)scr.recs);
+  if (e != cudaSuccess) return e;
+  *work_base_io += (unsigned)units + (unsigned)grid * kWarpsPerBlock;
+  if (split > 1) {
+    finalize_sweep_edges_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>((const SweepRec *)scr.recs, split, (long long)m,
+                                                                                  margin, d_clear, d_t, d_dist);
     e = cudaGetLastError();
   }
   return e;

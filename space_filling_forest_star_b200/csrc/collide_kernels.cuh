@@ -149,6 +149,18 @@ cudaError_t launch_distance_edges(const EnvDev &env, const double *d_starts, con
                                   cudaStream_t stream, const LaunchCfg &cfg, unsigned *work_base_io,
                                   const EdgeDistScratch &scr);
 
+// continuous check of the motion start -> end of every edge by conservative advancement on the pose distance
+// (include/sffg.h): clear[e] = 1 when every pose of the motion is certified at distance >= margin / 2; otherwise t[e] is
+// where the lowest stopped piece stopped and dist[e] the pose distance there (< margin).  t and dist may be null.
+struct SweepScratch {
+  int *stop;    // m ints for the edges split over several warps, or null (one warp per edge)
+  void *recs;   // sweep_edges_rec_bytes(m, cfg) bytes for the split edges' per-warp records, or null
+};
+size_t sweep_edges_rec_bytes(int64_t m, const LaunchCfg &cfg);
+cudaError_t launch_sweep_edges(const EnvDev &env, const double *d_starts, const double *d_ends, int64_t m, int rot_mode,
+                               double margin, uint8_t *d_clear, double *d_t, double *d_dist, cudaStream_t stream,
+                               const LaunchCfg &cfg, unsigned *work_base_io, const SweepScratch &scr);
+
 cudaError_t launch_gen_poses(uint64_t seed, uint64_t first, int64_t n, const float range[6], float *d_out,
                              cudaStream_t stream);
 

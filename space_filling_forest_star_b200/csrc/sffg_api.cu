@@ -38,7 +38,8 @@ constexpr size_t kSmallBytes = 1 << 20;   // pinned, device-mapped staging area 
 // The environment's staging area: inputs in the first 3/4, outputs in the last 1/4.  The outputs of a pose call are its
 // verdicts; those of a distance call are the distances [n] then (if asked for) the points [n][6]; those of an edge call
 // are first hits [m] then free flags [m]; those of a move call are free flags [m] then pose hits [m]; those of an edge
-// distance call are the distances [m], the points [m][6], then the sample indices [m].
+// distance call are the distances [m], the points [m][6], then the sample indices [m]; those of a sweep call are the
+// stop parameters [m], the distances [m], then the clear flags [m].
 struct EnvStaging {
   static constexpr size_t kInBytes = 768 << 10;
   static constexpr size_t kOutBytes = kSmallBytes - kInBytes;
@@ -52,6 +53,9 @@ struct EnvStaging {
   double *edge_dist() const { return reinterpret_cast<double *>(out()); }
   double *edge_points(int64_t m) const { return reinterpret_cast<double *>(out() + (size_t)m * 8); }
   int32_t *edge_index(int64_t m) const { return reinterpret_cast<int32_t *>(out() + (size_t)m * 56); }
+  double *sweep_t() const { return reinterpret_cast<double *>(out()); }
+  double *sweep_dist(int64_t m) const { return reinterpret_cast<double *>(out() + (size_t)m * 8); }
+  uint8_t *sweep_clear(int64_t m) const { return out() + (size_t)m * 16; }
 };
 
 // The index's staging area.  The first 64 KiB hold the queries; the one-kernel radius search keeps its fallback flag in
@@ -159,6 +163,7 @@ struct sffg_env {
   DevPtr<int> d_order;                           // leaf position -> caller's triangle index (refit)
   std::vector<int> level_base, level_count;      // breadth-first level table of the hierarchy (refit)
   int64_t obst_bytes = 0;
+  double obst_max_abs = 0;                       // max |obstacle coordinate| (root box), 0 without obstacles
   DevPtr<unsigned long long> d_counters;
   PinnedPtr<int> h_status;      // the kernels raise it, the host reads it without a copy
   DevPtr<unsigned> d_work;      // ring of 8 work counters (never reset; see launch_collide_poses)
@@ -359,7 +364,11 @@ static int finish_obstacles(sffg_env *env, const std::vector<ChildSlot> &top, co
   env->d_top.reset();
   SFFG_CUDA(upload(env->d_top, top.data(), top.size() * sizeof(ChildSlot), &bytes));
   d.n_obst = (int)n_obst;
+  env->obst_max_abs = 0;
   for (int k = 0; k < 3; ++k) {
+    // rounded up to float: the device builder's root box is outward rounded to float, the host builder's is exact
+    if (n_obst) env->obst_max_abs = std::max({env->obst_max_abs, (double)round_up_f32(std::fabs(root_lo[k])),
+                                              (double)round_up_f32(std::fabs(root_hi[k]))});
     const double oc = 0.5 * (root_lo[k] + root_hi[k]);
     d.root_c[k] = (float)oc;
     d.root_h[k] = n_obst ? round_up_f32(std::max(root_hi[k] - (double)d.root_c[k], (double)d.root_c[k] - root_lo[k]) * 1.0000001) : 0.f;
@@ -934,10 +943,10 @@ int sffg_collide_transforms_f64(sffg_env *env, const double *rt, int64_t n, uint
   return collide_poses_host(env, rt, 2, n, verdict_out);
 }
 
-// arguments of the edge and move calls
+// arguments of the edge and move calls; the sweep call has no sample spacing and passes check_sample = false
 static int check_segment_args(const sffg_env *env, const double *starts, const double *ends, int64_t m, double sample_dist,
-                              int rot_mode, const void *out, const char *who) {
-  if (!env || m < 0 || (m > 0 && (!starts || !ends || !out)) || !(sample_dist > 0) ||
+                              int rot_mode, const void *out, const char *who, bool check_sample = true) {
+  if (!env || m < 0 || (m > 0 && (!starts || !ends || !out)) || (check_sample && !(sample_dist > 0)) ||
       (rot_mode != SFFG_ROT_REFERENCE && rot_mode != SFFG_ROT_INTERPOLATE))
     return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments");
   return SFFG_OK;
@@ -1155,6 +1164,87 @@ int sffg_distance_edges_device(sffg_env *env, const double *d_starts, const doub
   EnvDev v = env_view(env, &base);
   SFFG_CUDA(launch_distance_edges(v, d_starts, d_ends, m, sample_dist, rot_mode, max_dist, d_dist_out, d_index_out, d_points_out,
                                   (cudaStream_t)stream, env->cfg, base, scr));
+  return env_leave(env, (cudaStream_t)stream);
+}
+
+// ---- continuous edge check -----------------------------------------------------------------------------------------
+// margin: positive, finite and at least 1e-6 max(1, max |obstacle coordinate|), which bounds the steps per edge
+static int sweep_args(const sffg_env *env, const double *starts, const double *ends, int64_t m, int rot_mode, double margin,
+                      const uint8_t *clear_out, const char *who) {
+  const int rc = check_segment_args(env, starts, ends, m, 0.0, rot_mode, clear_out, who, false);
+  if (rc != SFFG_OK) return rc;
+  if (!(margin > 0) || !std::isfinite(margin) || margin < 1e-6 * std::max(1.0, env->obst_max_abs))
+    return fail(SFFG_ERR_ARG, std::string(who) + ": bad arguments (margin must be finite and >= 1e-6 max(1, max |obstacle "
+                              "coordinate|) = " + std::to_string(1e-6 * std::max(1.0, env->obst_max_abs)) + ")");
+  return SFFG_OK;
+}
+
+// scratch of a sweep call whose edges may be split over several warps: the per-edge stop word and the per-warp records.
+// Growing frees the old block, so `st` (ordered behind every earlier launch of the environment) is drained first.
+static int sweep_scratch(sffg_env *env, int64_t m, bool split, cudaStream_t st, SweepScratch *scr) {
+  const size_t rec = split ? sweep_edges_rec_bytes(m, env->cfg) : 0;
+  const size_t fh = split ? (size_t)m * sizeof(int) : 0;
+  if (rec > env->edge_rec.cap || fh > env->fh.cap) SFFG_CUDA(cudaStreamSynchronize(st));
+  int rc = env->fh.reserve(fh);
+  if (rc == SFFG_OK) rc = env->edge_rec.reserve(rec);
+  if (rc != SFFG_OK) return rc;
+  scr->stop = rec ? (int *)env->fh.p : nullptr;
+  scr->recs = rec ? env->edge_rec.p : nullptr;
+  return SFFG_OK;
+}
+
+int sffg_sweep_edges(sffg_env *env, const double *starts, const double *ends, int64_t m, int rot_mode, double margin,
+                     uint8_t *clear_out, double *t_out, double *dist_out) {
+  int rc = sweep_args(env, starts, ends, m, rot_mode, margin, clear_out, "sffg_sweep_edges");
+  if (rc != SFFG_OK || m == 0) return rc;
+  if ((rc = env_enter_host(env)) != SFFG_OK) return rc;
+  unsigned *base;
+  if ((size_t)m * 96 <= EnvStaging::kInBytes && (size_t)m * 17 <= EnvStaging::kOutBytes) {
+    // planner-sized call: results straight into pinned mapped memory, one synchronisation
+    cudaStream_t st = env->streams[0].get();
+    const EnvStaging h = env->staging();
+    SweepScratch scr;
+    double *ds, *de;
+    if ((rc = sweep_scratch(env, m, true, st, &scr)) != SFFG_OK) return rc;
+    if ((rc = stage_segments(env, starts, ends, m, &ds, &de)) != SFFG_OK) return rc;
+    EnvDev v = env_view(env, &base);
+    SFFG_CUDA(launch_sweep_edges(v, ds, de, m, rot_mode, margin, h.sweep_clear(m), t_out ? h.sweep_t() : nullptr,
+                                 dist_out ? h.sweep_dist(m) : nullptr, st, env->cfg, base, scr));
+    SFFG_CUDA(cudaStreamSynchronize(st));
+    std::memcpy(clear_out, h.sweep_clear(m), (size_t)m);
+    if (t_out) std::memcpy(t_out, h.sweep_t(), (size_t)m * 8);
+    if (dist_out) std::memcpy(dist_out, h.sweep_dist(m), (size_t)m * 8);
+    return check_status(env);
+  }
+  return edge_call_chunks(env, starts, ends, m, [&](int s, int64_t off, int64_t cnt, double *ds, double *de, cudaStream_t st) {
+    // out[s]: stop parameters [cnt], distances [cnt], clear flags [cnt]; one warp per edge (no scratch)
+    const int rc2 = env->out[s].reserve((size_t)cnt * 17);
+    if (rc2 != SFFG_OK) return rc2;
+    double *d_t = (double *)env->out[s].p, *d_dist = d_t + cnt;
+    uint8_t *d_clear = (uint8_t *)(d_dist + cnt);
+    EnvDev v = env_view(env, &base);
+    SFFG_CUDA(launch_sweep_edges(v, ds, de, cnt, rot_mode, margin, d_clear, t_out ? d_t : nullptr, dist_out ? d_dist : nullptr, st,
+                                 env->cfg, base, SweepScratch{nullptr, nullptr}));
+    SFFG_CUDA(cudaMemcpyAsync(clear_out + off, d_clear, (size_t)cnt, cudaMemcpyDeviceToHost, st));
+    if (t_out) SFFG_CUDA(cudaMemcpyAsync(t_out + off, d_t, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+    if (dist_out) SFFG_CUDA(cudaMemcpyAsync(dist_out + off, d_dist, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+    return SFFG_OK;
+  });
+}
+
+int sffg_sweep_edges_device(sffg_env *env, const double *d_starts, const double *d_ends, int64_t m, int rot_mode, double margin,
+                            uint8_t *d_clear_out, double *d_t_out, double *d_dist_out, void *stream) {
+  int rc = sweep_args(env, d_starts, d_ends, m, rot_mode, margin, d_clear_out, "sffg_sweep_edges_device");
+  if (rc != SFFG_OK) return rc;
+  unsigned *base;
+  rc = env_enter(env, (cudaStream_t)stream);
+  if (rc != SFFG_OK) return rc;
+  // small batches: several warps per edge, as sffg_check_edges_device
+  SweepScratch scr;
+  if ((rc = sweep_scratch(env, m, m < 8192, (cudaStream_t)stream, &scr)) != SFFG_OK) return rc;
+  EnvDev v = env_view(env, &base);
+  SFFG_CUDA(launch_sweep_edges(v, d_starts, d_ends, m, rot_mode, margin, d_clear_out, d_t_out, d_dist_out, (cudaStream_t)stream,
+                               env->cfg, base, scr));
   return env_leave(env, (cudaStream_t)stream);
 }
 

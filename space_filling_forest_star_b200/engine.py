@@ -218,6 +218,42 @@ class Environment:
                                                  points.data_ptr() if points is not None else None, st))
         return out
 
+    # ---- continuous edge check (sffg_sweep_edges) ------------------------------------------------------------
+    def SweepEdges(self, starts, ends, margin: float, rot_mode: int = ROT_REFERENCE):
+        """edges start -> end ([m][6] float64) -> (clear uint8[m], t float64[m], dist float64[m]): clear = 1 certifies every
+        pose of the motion start + t (end - start), t in [0, 1], at distance >= margin / 2 (t = 1, dist = margin);
+        otherwise the motion is certified on [0, t) and dist < margin is the pose distance at t (0 on contact)."""
+        s = np.ascontiguousarray(np.asarray(starts, dtype=np.float64).reshape(-1, 6))
+        e = np.ascontiguousarray(np.asarray(ends, dtype=np.float64).reshape(-1, 6))
+        assert len(s) == len(e)
+        m = len(s)
+        clear = np.empty(m, dtype=np.uint8)
+        t = np.empty(m, dtype=np.float64)
+        dist = np.empty(m, dtype=np.float64)
+        check(self._L.sffg_sweep_edges(self._h, _ptr(s) if m else None, _ptr(e) if m else None, m, rot_mode, float(margin),
+                                       _ptr(clear) if m else None, _ptr(t) if m else None, _ptr(dist) if m else None))
+        return clear, t, dist
+
+    def sweep_edges_device(self, starts, ends, margin: float, rot_mode: int = ROT_REFERENCE, clear_out=None, t_out=None,
+                           dist_out=None, stream: Optional[int] = None):
+        """starts, ends: torch CUDA float64 [m][6] -> torch uint8 [m] clear flags (enqueued, not synchronised); ``t_out`` and
+        ``dist_out`` (float64 [m] on the same device) are optional."""
+        import torch
+        assert starts.is_cuda and starts.dtype == torch.float64 and ends.dtype == torch.float64
+        assert starts.is_contiguous() and ends.is_contiguous() and starts.shape == ends.shape
+        m = starts.numel() // 6
+        if clear_out is None:
+            clear_out = torch.empty(m, dtype=torch.uint8, device=starts.device)
+        assert clear_out.dtype == torch.uint8 and clear_out.is_contiguous() and clear_out.numel() == m
+        for o in (t_out, dist_out):
+            if o is not None:
+                assert o.dtype == torch.float64 and o.is_contiguous() and o.numel() == m
+        st = torch.cuda.current_stream(starts.device).cuda_stream if stream is None else stream
+        check(self._L.sffg_sweep_edges_device(self._h, starts.data_ptr(), ends.data_ptr(), m, rot_mode, float(margin),
+                                              clear_out.data_ptr(), t_out.data_ptr() if t_out is not None else None,
+                                              dist_out.data_ptr() if dist_out is not None else None, st))
+        return clear_out
+
     # ---- Solver<T,R>::isPathFree ---------------------------------------------------------------------------
     def isPathFree(self, starts, ends, sample_dist: float = COLLISION_SAMPLE_SIZE, rot_mode: int = ROT_REFERENCE,
                    want_first_hit: bool = False):
