@@ -14,8 +14,9 @@
 //            - surviving leaf triangles are transformed into the robot frame (as RAPID does) lane-per-triangle,
 //              then lane-per-(obstacle triangle, robot triangle) pair runs the 17-axis separating-axis test in FP32
 //              as a *certificate* test: an axis only counts when its gap exceeds a rigorous rounding bound
-//            - pairs the lane-per-pair stage leaves open get the 9 edge x edge axes and, only if those fail, the 6
-//              contact certificates cooperatively, three pairs per pass on ten lanes each
+//            - pairs the lane-per-pair stage leaves open get the 9 edge x edge axes (three pairs per pass on ten lanes
+//              each) and the 6 contact certificates cooperatively: the certificates first (five pairs per pass on six
+//              lanes each) in the pose verdict kernel, the axes first in every other kernel
 //            - pairs without an FP32 certificate are decided by the exact stage: the same 17 axes in FP64 with the
 //              operation order of the CPU oracle, one axis per lane; __all_sync gives the pair verdict
 //            - __ballot/__any early-out on the first confirmed contact (verdict-equivalent to RAPID's ALL_CONTACTS
@@ -58,7 +59,10 @@ struct XTri {        // obstacle triangle in the robot frame (FP32); 13 words = 
 struct WarpScratch {
   int stack[kStackCap];
   int tri[kTriCap];
-  int cand[kCandCap];
+  union {              // the swept-box candidate list serves only the kernels without the contact probe, and vice versa
+    int cand[kCandCap];
+    int2 wit[32];      // each lane's contact witnesses from phase A ({-1, -1}: none), read by phase B's probe
+  };
   XTri xt[32];
 };
 
@@ -153,9 +157,12 @@ __device__ __forceinline__ bool edge_pierces(const float *a, const float *b, con
   return (v0 > bound && v1 > bound && v2 > bound) || (v0 < -bound && v1 < -bound && v2 < -bound);
 }
 
-// Stage P2, ten lanes per open pair, three pairs per pass (lanes 0..9, 10..19, 20..29; k = lane % 10):
-//   pass a  lanes k < 9 evaluate the nine edge x edge axes e_i x f_j        -> pairs proven disjoint
-//   pass b  (only for pairs pass a left open) lanes k < 6 evaluate the six edge-pierces-triangle contact certificates
+// Stage P2, the pairs the lane-per-pair stage left open, in two kinds of cooperative pass (order: see triangle_stage):
+//   pass c  six lanes per pair, up to five pairs per pass (lane 6g + c): the six edge-pierces-triangle contact certificates
+//                                                                            -> any one proves the pose's contact
+//   pass a  ten lanes per pair, three pairs per pass (lanes 0..9, 10..19, 20..29; k = lane % 10): lanes k < 9 evaluate
+//           the nine edge x edge axes e_i x f_j                              -> pairs proven disjoint
+// what neither decides goes to the FP64 exact stage
 __device__ __forceinline__ bool open_pair_axis(const XTri &x, const RobotTri &rt, int k) {
   const float *p = x.v;
   const float errpos = 2.0f * x.err + kEpsSat * fmaxf(x.mabs, rt.qmax);
@@ -485,14 +492,32 @@ __device__ __forceinline__ bool transform_triangle(const EnvDev &E, const PoseU 
   return keep;
 }
 
+// m without its n lowest set bits
+__device__ __forceinline__ unsigned drop_lowest(unsigned m, int n) {
+#pragma unroll
+  for (int k = 0; k < n; ++k) m &= m - 1;
+  return m;
+}
+// the lane of the n-th lowest set bit of m (n = 0..4), -1 when m has no more than n
+__device__ __forceinline__ int nth_lane(unsigned m, int n) {
+#pragma unroll
+  for (int k = 0; k < 4; ++k)
+    if (k < n) m &= m - 1;
+  return __ffs(m) - 1;
+}
+
 // Triangle stage of one pose over the candidate triangles ws.tri[0, ntri): transform into the robot frame, cull, pair stages
-// P1 (lane-per-pair), P2 (three pairs per cooperative pass) and the FP64 exact stage; stops at the first confirmed contact.
-template <int FMT, bool COUNT>
+// P1 (lane-per-pair), P2 and the FP64 exact stage; stops at the first confirmed contact.  CONTACT_FIRST selects the P2 order:
+// the contact certificates of five pairs before their separating axes (the pose verdict kernel, whose open pairs mostly
+// touch), or the axes of three pairs first and the certificates of what they leave open (every other kernel: edge samples
+// are mostly free, and the distance and sweep kernels keep their registers).  Either order gives every pair that no
+// certificate proves in contact all nine axes, then FP64, so the verdict of every call is the same.
+template <int FMT, bool COUNT, bool CONTACT_FIRST>
 __device__ __forceinline__ void triangle_stage(const EnvDev &E, WarpScratch &ws, const RobotTri *srob, const PoseU &P,
                                                const LanePose<FMT> &lp, int src, int lane, int ntri, bool &hit, bool &have_R2,
                                                PairCtx &pc, Tally &tally) {
   const unsigned lt = (1u << lane) - 1u;
-  const int grp10 = lane / 10, k10 = lane - 10 * grp10;
+  const int grp10 = lane / 10, k10 = lane - 10 * grp10, grp6 = lane / 6, k6 = lane - 6 * grp6;
   const float inv_n_robot = 1.0f / (float)E.n_robot;
   for (int base = 0; base < ntri && !hit; base += 32) {
     const int cnt = (ntri - base) < 32 ? (ntri - base) : 32;
@@ -517,43 +542,98 @@ __device__ __forceinline__ void triangle_stage(const EnvDev &E, WarpScratch &ws,
         tally.pair += np;
         tally.exact += __popc(um);   // pairs the lane-per-pair stage P1 left open
       }
-      while (um && !hit) {
-        const int l0 = __ffs(um) - 1;
-        um &= um - 1;
-        const int l1 = um ? __ffs(um) - 1 : -1;
-        um &= um - 1;   // (0 stays 0)
-        const int l2 = um ? __ffs(um) - 1 : -1;
-        um &= um - 1;
-        const int lmine = grp10 == 0 ? l0 : (grp10 == 1 ? l1 : (grp10 == 2 ? l2 : -1));
-        const int xim = __shfl_sync(kFull, xi_l, lmine & 31), rm = __shfl_sync(kFull, r_l, lmine & 31);
-        bool sep = false;
-        if (lmine >= 0 && k10 < 9) sep = open_pair_axis(ws.xt[xim], srob[rm], k10);
-        const unsigned bs = __ballot_sync(kFull, sep);
-        unsigned open_g = 0;
-        if (!(bs & 0x3ffu)) open_g |= 1u;
-        if (l1 >= 0 && !(bs & (0x3ffu << 10))) open_g |= 2u;
-        if (l2 >= 0 && !(bs & (0x3ffu << 20))) open_g |= 4u;
-        if (open_g == 0) continue;
-        bool con = false;
-        if (lmine >= 0 && k10 < 6 && ((open_g >> grp10) & 1u)) con = open_pair_pierce(ws.xt[xim], srob[rm], k10);
-        if (__any_sync(kFull, con)) {
-          hit = true;
-          break;
-        }
-        while (open_g) {
-          const int g = __ffs(open_g) - 1;
-          open_g &= open_g - 1;
-          const int lg = g == 0 ? l0 : (g == 1 ? l1 : l2);
-          const int xg = __shfl_sync(kFull, xi_l, lg), rg = __shfl_sync(kFull, r_l, lg);
-          if (COUNT) tally.exact_run += 1;
-          if (!have_R2) {
-            lp.exact(src, pc.R2, pc.T2, lane);
-            have_R2 = true;
+      if constexpr (CONTACT_FIRST) {
+        // the pair of lane l, computed again where needed: cheaper in registers than shuffling it from its lane
+        const auto pair_of = [&](int l, int &xi, int &r) {
+          xi = (int)(((float)(pb + l) + 0.5f) * inv_n_robot);
+          r = pb + l - xi * E.n_robot;
+        };
+        while (um && !hit) {
+          const unsigned five = um ^ drop_lowest(um, 5);   // the next five open pairs
+          um ^= five;
+          const int lc = grp6 < 5 ? nth_lane(five, grp6) : -1;   // pass c: lane 6g + c, certificate c of pair g
+          int xi, r;
+          bool con = false;
+          if (lc >= 0) {
+            pair_of(lc, xi, r);
+            con = open_pair_pierce(ws.xt[xi], srob[r], k6);
           }
-          const int t = ws.xt[xg].tri;
-          if (exact_pair_contact(pc.R2, pc.T2, E.tris64 + 9 * (size_t)t, E.robot64 + 9 * (size_t)rg, lane)) {
+          if (__any_sync(kFull, con)) {
             hit = true;
             break;
+          }
+          // none of the five touches provably: pass a, three pairs at a time, and FP64 for what it leaves open
+          unsigned left = five;
+#pragma unroll 1
+          while (left && !hit) {
+            const unsigned three = left ^ drop_lowest(left, 3);
+            left ^= three;
+            const int la = grp10 < 3 ? nth_lane(three, grp10) : -1;
+            bool sep = false;
+            if (la >= 0 && k10 < 9) {
+              pair_of(la, xi, r);
+              sep = open_pair_axis(ws.xt[xi], srob[r], k10);
+            }
+            const unsigned bs = __ballot_sync(kFull, sep);
+#pragma unroll 1
+            for (int g = 0; g < 3; ++g) {
+              const int lg = nth_lane(three, g);
+              if (lg < 0) break;
+              if ((bs >> (10 * g)) & 0x3ffu) continue;
+              if (COUNT) tally.exact_run += 1;
+              if (!have_R2) {
+                lp.exact(src, pc.R2, pc.T2, lane);
+                have_R2 = true;
+              }
+              pair_of(lg, xi, r);
+              const int t = ws.xt[xi].tri;
+              if (exact_pair_contact(pc.R2, pc.T2, E.tris64 + 9 * (size_t)t, E.robot64 + 9 * (size_t)r, lane)) {
+                hit = true;
+                break;
+              }
+            }
+          }
+        }
+      } else {
+        while (um && !hit) {
+          const int l0 = __ffs(um) - 1;
+          um &= um - 1;
+          const int l1 = um ? __ffs(um) - 1 : -1;
+          um &= um - 1;   // (0 stays 0)
+          const int l2 = um ? __ffs(um) - 1 : -1;
+          um &= um - 1;
+          const int lmine = grp10 == 0 ? l0 : (grp10 == 1 ? l1 : (grp10 == 2 ? l2 : -1));
+          const int xim = __shfl_sync(kFull, xi_l, lmine & 31), rm = __shfl_sync(kFull, r_l, lmine & 31);
+          bool sep = false;
+          if (lmine >= 0 && k10 < 9) sep = open_pair_axis(ws.xt[xim], srob[rm], k10);
+          const unsigned bs = __ballot_sync(kFull, sep);
+          unsigned open_g = 0;
+          if (!(bs & 0x3ffu)) open_g |= 1u;
+          if (l1 >= 0 && !(bs & (0x3ffu << 10))) open_g |= 2u;
+          if (l2 >= 0 && !(bs & (0x3ffu << 20))) open_g |= 4u;
+          if (open_g == 0) continue;
+          // pass c on the lanes of the axes, for the pairs no axis separated
+          bool con = false;
+          if (lmine >= 0 && k10 < 6 && ((open_g >> grp10) & 1u)) con = open_pair_pierce(ws.xt[xim], srob[rm], k10);
+          if (__any_sync(kFull, con)) {
+            hit = true;
+            break;
+          }
+          while (open_g) {
+            const int g = __ffs(open_g) - 1;
+            open_g &= open_g - 1;
+            const int lg = g == 0 ? l0 : (g == 1 ? l1 : l2);
+            const int xg = __shfl_sync(kFull, xi_l, lg), rg = __shfl_sync(kFull, r_l, lg);
+            if (COUNT) tally.exact_run += 1;
+            if (!have_R2) {
+              lp.exact(src, pc.R2, pc.T2, lane);
+              have_R2 = true;
+            }
+            const int t = ws.xt[xg].tri;
+            if (exact_pair_contact(pc.R2, pc.T2, E.tris64 + 9 * (size_t)t, E.robot64 + 9 * (size_t)rg, lane)) {
+              hit = true;
+              break;
+            }
           }
         }
       }
@@ -621,7 +701,8 @@ __device__ __forceinline__ StepLeaves walk_step(const EnvDev &E, WarpScratch &ws
   return {m_leaf, ov && child < 0, ~child};
 }
 
-template <int FMT, bool COUNT, bool PROBE>
+// PROBE: the contact probe (every kernel but the edge verdict kernel); CONTACT_FIRST: triangle_stage's P2 order
+template <int FMT, bool COUNT, bool PROBE, bool CONTACT_FIRST>
 __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, const PoseU &P,
                               const LanePose<FMT> &lp, int src, int lane, Tally &tally) {
   const RobotTri *srob = cs.rob;
@@ -637,19 +718,16 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
   // Contact probe: a pose that reaches phase B mostly collides, and mostly with one of its cell's two witnesses (the
   // triangles that mark the cell nearest its centre).  The first pass of the loop below runs the triangle stage over them
   // alone; a confirmed contact ends the pose without a walk, anything else walks from the root as if there were no probe.
-  // (The cell is derived again from the same Thi as in phase A: cheaper than holding it in a register through phase A.)
+  // (Phase A fetched the witnesses of every lane's cell with its plane, into ws.wit.)
   // The edge kernel is built without it (PROBE = false): its samples mostly share the swept-box candidate list, and the
   // probe's code alone cost its per-sample loop 2 % of the edge rate in spills.
   bool probe = false;
-  if (PROBE && E.grid.witness) {
-    const int cell = grid_cell(E.grid, P.Thi[0], P.Thi[1], P.Thi[2]);
-    if (cell >= 0) {
-      const int2 w = __ldg(E.grid.witness + cell);
-      if (lane < 2) ws.tri[lane] = lane ? w.y : w.x;
-      ntri = (w.x >= 0) + (w.y >= 0);   // (w.y >= 0 only with w.x >= 0)
-      probe = ntri > 0;
-      __syncwarp();
-    }
+  if (PROBE) {
+    const int2 w = ws.wit[src];
+    if (lane < 2) ws.tri[lane] = lane ? w.y : w.x;
+    ntri = (w.x >= 0) + (w.y >= 0);   // (w.y >= 0 only with w.x >= 0)
+    probe = ntri > 0;
+    __syncwarp();
   }
 
   bool first = true;
@@ -672,7 +750,7 @@ __device__ bool warp_pose_hit(const EnvDev &E, WarpScratch &ws, const CtaShared 
       continue;
     }
     // ---------------- triangle stage ----------------
-    triangle_stage<FMT, COUNT>(E, ws, srob, P, lp, src, lane, ntri, hit, have_R2, pc, tally);
+    triangle_stage<FMT, COUNT, CONTACT_FIRST>(E, ws, srob, P, lp, src, lane, ntri, hit, have_R2, pc, tally);
     if (hit) break;
     ntri = 0;
     if (probe) {   // no contact with the witnesses: the walk starts (it may deliver them again, which is harmless)
@@ -729,7 +807,7 @@ __device__ bool pose_hits_candidates(const EnvDev &E, WarpScratch &ws, const Cta
     const int cnt = (ncand - base) < 32 ? (ncand - base) : 32;
     if (lane < cnt) ws.tri[lane] = ws.cand[base + lane];
     __syncwarp();
-    triangle_stage<FMT, COUNT>(E, ws, cs.rob, P, lp, src, lane, cnt, hit, have_R2, pc, tally);
+    triangle_stage<FMT, COUNT, false>(E, ws, cs.rob, P, lp, src, lane, cnt, hit, have_R2, pc, tally);
   }
   return hit;
 }
@@ -837,7 +915,9 @@ __device__ __forceinline__ void flush_tally(const EnvDev &E, const Tally &t, uns
 
 // phase A (lane-per-pose cull + rotation) then phase B over the surviving lanes; returns the mask of colliding lanes
 // (stops at the first hit when `first_only`, which is what an edge needs)
-template <int FMT, bool COUNT, bool SWEPT_CAPABLE = false>
+// CONTACT_FIRST: the P2 order of the triangle stage (see triangle_stage); only the pose verdict kernel takes the
+// certificates first
+template <int FMT, bool COUNT, bool SWEPT_CAPABLE = false, bool CONTACT_FIRST = false>
 __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch &ws, const CtaShared &cs, bool valid,
                                                    const LanePose<FMT> &lp, int lane, bool first_only, Tally &tally,
                                                    bool swept = false, bool swept_identity = true) {
@@ -845,14 +925,23 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
   lp.split(thi, tlo);
   const float tlo_mag = fabsf(tlo[0]) + fabsf(tlo[1]) + fabsf(tlo[2]);
   bool alive = valid && E.n_obst > 0 && sphere_hits_root(E, thi[0], thi[1], thi[2], tlo_mag);
+  constexpr bool kProbe = !SWEPT_CAPABLE;   // (warp_pose_hit's PROBE)
   unsigned plane = kNoPlane;   // (loaded before the rotation is built, which hides the load)
+  int2 wit = make_int2(-1, -1);   // the contact witnesses of the cell, loaded with its plane
   if (alive && E.grid.n[0] > 0) {
     const int cell = grid_cell(E.grid, thi[0], thi[1], thi[2]);
     alive = cell < 0 || cell_marked(E, cell);
-    if (alive && cell >= 0) plane = __ldg(E.grid.planes + cell);
+    if (alive && cell >= 0) {
+      plane = __ldg(E.grid.planes + cell);
+      if (kProbe && E.grid.witness) wit = __ldg(E.grid.witness + cell);
+    }
   }
   if (alive) lp.rot32(R);
   if (alive && plane != kNoPlane) alive = !plane_says_free(E, plane, R, thi, tlo_mag);
+  if (kProbe) {
+    ws.wit[lane] = wit;
+    __syncwarp();
+  }
   if (COUNT) tally.past_grid += __popc(__ballot_sync(kFull, alive));
   unsigned todo = __ballot_sync(kFull, alive);
   unsigned hitmask = 0;
@@ -890,7 +979,7 @@ __device__ __forceinline__ unsigned check_32_poses(const EnvDev &E, WarpScratch 
       P.Tlo[k] = FMT == kFmtEulerF32 ? 0.f : __shfl_sync(kFull, tlo[k], src);
     }
     if (SWEPT_CAPABLE && ncand > 0 ? pose_hits_candidates<FMT, COUNT>(E, ws, cs, P, lp, src, lane, ncand, tally)
-                                   : warp_pose_hit<FMT, COUNT, !SWEPT_CAPABLE>(E, ws, cs, P, lp, src, lane, tally)) {
+                                   : warp_pose_hit<FMT, COUNT, kProbe, CONTACT_FIRST>(E, ws, cs, P, lp, src, lane, tally)) {
       hitmask |= 1u << src;
       if (first_only) break;
     }
@@ -944,7 +1033,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocksPerSm) collide_poses_kerne
     if (mine) lp.load(poses, i);
     else lp.clear();
     if (COUNT) nposes += mine ? 1 : 0;
-    const unsigned hitmask = check_32_poses<FMT, COUNT>(E, ws, cs, mine, lp, lane, false, tally);
+    const unsigned hitmask = check_32_poses<FMT, COUNT, false, true>(E, ws, cs, mine, lp, lane, false, tally);
     if (outs.n == 1) {
       if (mine) outs.p[0][i] = (uint8_t)((hitmask >> lane) & 1u);
     } else if (chunk == 32 && (long long)c * 32 + 32 <= n) {
